@@ -2,6 +2,7 @@
 """Benchmark of the streaming GraphSAGE-pool hot path (BASELINE.json metric: train target-vertices/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload reddit|elliptic|arxiv|pubmed]
+                    [--dump-outputs DIR]
 
 A "step" is one training minibatch of the workload: sample the 2-hop neighbourhood of B target vertices from the
 streaming CSR (Philox, with replacement), compact the frontiers, gather the input feature rows, GraphSAGE-pool
@@ -499,6 +500,28 @@ def workload_config(w, name, world):
                                                       2 * w["E"] * 8 * 1.5 / 1e6)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, params, flat, grad, loss_sum):
+    """write what the timed train step hands its caller after its last step, as <out_dir>/<name>.npy in fp32: the updated
+    weights under their state-dict names, that step's gradient as grad.<name>, and its loss sum (over this rank's seeds) as
+    loss_sum, so that two builds run with the same arguments can be compared output for output"""
+    arrays, off = {"loss_sum": loss_sum.reshape(1)}, 0
+    for k in (f"layers.{i}.{n}" for i in range(2) for n in NAMES):
+        n = params[k].numel()
+        arrays[k] = flat[off:off + n].view(params[k].shape)
+        arrays["grad." + k] = grad[off:off + n].view(params[k].shape)
+        off += n
+    assert off == flat.numel(), (off, flat.numel())
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs of %d bytes exceed the dump limit" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 DTYPES = {"fp16": dict(es=2, note="fp16 storage (ten explicit mantissa bits, as TF32) with static loss scaling: activation gradients are stored times a "
                                   "power of two derived from 1 / global batch and every weight / bias gradient is unscaled exactly where it is "
                                   "written in fp32; tcgen05.mma.kind::f16, fp32 accumulation, fp32 master weights and Adam"),
@@ -657,6 +680,8 @@ def measure(dt, headline, args, w, rank, world, dev, dist, g, feats, labels, hos
     ms_dev, wall0, wall1, _ = timed(dev_batches[W:W + K], read_back=False)
     host_enqueue_ms = host_ms[0]
     gs1 = plan.graph_stats()
+    if headline and args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, params, flat, grad, loss_dev)
     out = {"dtype": dt, "arithmetic": DTYPES[dt]["note"], "value": B * world * K / (ms_dev / 1e3), "ms_per_step": ms_dev / K,
            "host_enqueue_ms_per_step": host_enqueue_ms / K, "replicas": replicas,
            "cuda_graph": {"replays_in_timed_region": gs1["replays"] - gs0["replays"], "captures_in_timed_region": gs1["captures"] - gs0["captures"]},
@@ -928,7 +953,12 @@ def main():
                          "(N = 1 prints the other modes too, under `alt`)")
     ap.add_argument("--no-alt", action="store_true", help="N = 1: do not measure the other arithmetic modes")
     ap.add_argument("--no-parity", action="store_true", help="skip the parity leg (one step against the fp64 oracle, untimed)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the headline mode, write what their last step returned (updated weights, gradient, "
+                         "loss sum; rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     EXCHANGE[0] = args.exchange
     IMPL[0] = args.impl
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
