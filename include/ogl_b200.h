@@ -188,9 +188,6 @@ int ogl_plan_step_finish_tail(ogl_plan* p, ogl_features* f, void* stream);
  * weight-gradient GEMM, that one after it.  The plan's gradient buffer must be `peer`'s (ogl_peer_buffer). */
 int ogl_plan_step_finish_dp(ogl_plan* p, ogl_peer* peer, ogl_features* f, float loss_scale, float* per_vertex_loss_dev,
                             float* loss_sum_dev, void* stream);
-/* the same GEMM in n_parts pieces of 256 output rows (piece `part` writes gradient rows [256 part, 256 part + 256) of layer 0's
- * fc_pool.weight): a data-parallel caller exchanges piece i while piece i + 1 is computed */
-int ogl_plan_step_finish_tail_part(ogl_plan* p, ogl_features* f, int part, int n_parts, void* stream);
 /* software pipeline (the job of NodeDataLoader's worker processes, pytorch/model.py:128-131): sample + gather of a FUTURE minibatch,
  * enqueued on the plan's own stream into the plan's second buffer set, ordered after everything enqueued on `stream` so far.  Up to
  * two minibatches may be pending.  The next ogl_plan_train_step / ogl_plan_step_finish[_head] on the plan consumes the oldest pending

@@ -80,7 +80,6 @@ SIGNATURES = {
     "ogl_plan_step_finish_head": (_i, [_vp, _vp, _f, _vp, _vp, _vp]),
     "ogl_plan_step_finish_tail": (_i, [_vp, _vp, _vp]),
     "ogl_plan_step_finish_dp": (_i, [_vp, _vp, _vp, _f, _vp, _vp, _vp]),
-    "ogl_plan_step_finish_tail_part": (_i, [_vp, _vp, _i, _i, _vp]),
     "ogl_plan_prefetch": (_i, [_vp, _vp, _vp, _vp, _i, _i, _vp]),
     "ogl_plan_prefetch_pending": (_i, [_vp]),
     "ogl_graph_row_degrees": (_i, [_vp, _vp, _i64, _vp, _vp]),

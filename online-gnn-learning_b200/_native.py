@@ -321,18 +321,9 @@ class Plan:
         """forward + loss + backward except the last weight-gradient GEMM (layer 0 fc_pool.weight)"""
         check(lib.ogl_plan_step_finish_head(self._h, features._h, float(loss_scale), _ptr(per_vertex_out), _ptr(loss_sum_out), _stream()))
 
-    def step_finish_tail(self, features, part=0, n_parts=1):
-        """the last weight-gradient GEMM (layer 0 fc_pool.weight), whole or piece `part` of `n_parts` (256 gradient rows each)"""
-        if n_parts == 1:
-            check(lib.ogl_plan_step_finish_tail(self._h, features._h, _stream()))
-        else:
-            check(lib.ogl_plan_step_finish_tail_part(self._h, features._h, int(part), int(n_parts), _stream()))
-
-    @property
-    def tail_pieces(self):
-        """[(lo, hi)] flat gradient ranges of the pieces step_finish_tail(part, n_parts) produces"""
-        d = self.dims[0]
-        return [(r0 * d, min(d, r0 + 256) * d) for r0 in range(0, d, 256)]
+    def step_finish_tail(self, features):
+        """the last weight-gradient GEMM (layer 0 fc_pool.weight)"""
+        check(lib.ogl_plan_step_finish_tail(self._h, features._h, _stream()))
 
     @property
     def tail_params(self):

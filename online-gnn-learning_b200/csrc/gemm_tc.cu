@@ -21,7 +21,6 @@
 #include "gemm.cuh"
 #include "sage_kernels.cuh"
 #include <cuda.h>
-#include <stdlib.h>
 
 namespace ogl {
 
@@ -43,10 +42,7 @@ constexpr int SMEM_NT1 = RING_BYTES + STORE_BYTES + BIAS_BYTES + TAIL_BYTES;
 // 16 KB of A + 16 KB of B per CTA.  FIVE stages (160 KB): together with the staging boxes the CTA then leaves ~33 KB of
 // the SM's shared memory free, so the small kernels of the side / prefetch streams (sampling, to_block, scans, column sums;
 // all <= 9 KB) can be resident next to it instead of waiting for the GEMM to leave the SM
-#ifndef OGL_NT_STAGES2
-#define OGL_NT_STAGES2 5
-#endif
-constexpr int STAGES2 = OGL_NT_STAGES2;
+constexpr int STAGES2 = 5;
 constexpr int B2_STAGE_BYTES = (BN_MAX / 2) * BK * 2;    // 16 KB
 constexpr int RING2_BYTES = STAGES2 * (A_STAGE_BYTES + B2_STAGE_BYTES);
 constexpr int SMEM_NT2 = RING2_BYTES + STORE_BYTES + BIAS_BYTES + TAIL_BYTES;
@@ -105,12 +101,6 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void prefetch_tensormap(const CUtensorMap* map) {     // descriptor fetch off the first load's critical path
   asm volatile("prefetch.tensormap [%0];" ::"l"(map) : "memory");
-}
-// L2 prefetch of a tensor box (no shared memory involved): the producers run these a few stages AHEAD of the loads.  The ring
-// holds 160-192 KB per SM, which at the 2-3 us a DRAM miss costs under load covers less than the tensor pipe consumes; a box that
-// is already in L2 when its load is issued comes back in ~0.7 us
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* map, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(map), "r"(c0), "r"(c1) : "memory");
 }
 __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N>
@@ -342,11 +332,6 @@ struct NtParams {
   int out_f32_tma;              // TF kernels: fp32 output through TMA stores (activations), rounded to TF32 if round_out
   int round_out;
   int zero_tail;
-  int prefetch;                 // k-blocks the A operand is prefetched into L2 ahead of its load (0: off)
-  int loader;                   // 3: two TMA producers (warp 0: A boxes, warp 10: B boxes), 0: one
-  int order;                    // tile order of a unit: 0 = round robin over all (row block, column tile) pairs, 1 = row-block major
-                                //   (the column tiles of one row block back to back on the same unit: its A block is re-read from L2)
-  int debug;                    // perf experiments (OGL_GEMM_DBG): 1 = epilogue drains the accumulator without storing
 };
 
 // CG = 1: one CTA per 128-row tile.  CG = 2: a CTA pair (cluster of 2, tcgen05 cta_group::2) computes a 256-row super
@@ -370,16 +355,13 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
   const int m_pad = p.zero_tail ? min((m_dyn + 127) / 128 * 128, p.m_max) : m_dyn;
   const int m_tiles = ((m_pad + BM - 1) / BM + CG - 1) / CG;      // row blocks of CG * 128 rows
   const int total_tiles = m_tiles * p.n_tiles;
-  // i-th tile of this unit -> (row block mt, column tile nb); false past the unit's last tile
+  // i-th tile of this unit -> (row block mt, column tile nb), round robin over all (row block, column tile) pairs; false past the
+  // unit's last tile
   auto tile_at = [&](int i, int& mt, int& nb) -> bool {
-    if (p.order == 0) {
-      const int t = unit + i * n_units;
-      if (t >= total_tiles) return false;
-      mt = t / p.n_tiles; nb = t % p.n_tiles;
-      return true;
-    }
-    mt = unit + (i / p.n_tiles) * n_units; nb = i % p.n_tiles;
-    return mt < m_tiles;
+    const int t = unit + i * n_units;
+    if (t >= total_tiles) return false;
+    mt = t / p.n_tiles; nb = t % p.n_tiles;
+    return true;
   };
   int rows_valid[2];
   rows_valid[0] = uniform(p.a_rows_dev[0] ? min(*p.a_rows_dev[0], m_dyn) : m_dyn);
@@ -390,9 +372,8 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
     if (p.out_bf16 || p.out_f32_tma) prefetch_tensormap(&p.tc);
   }
   if (threadIdx.x == 0) {
-    s.tmem_slot[2] = 0;                            // the A producer's progress counter (read by the L2 prefetcher)
-    // full[]: loader 0: one TMA producer; 3: two TMA producers (A | B), one expect_tx arrival each
-    for (int i = 0; i < NST; ++i) { mbar_init(&s.full[i], p.loader == 3 ? 2 : 1); mbar_init(&s.empty[i], 1); }
+    // full[]: two TMA producers (A | B), one expect_tx arrival each
+    for (int i = 0; i < NST; ++i) { mbar_init(&s.full[i], 2); mbar_init(&s.empty[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&s.acc_full[i], 1); mbar_init(&s.acc_empty[i], 8 * CG); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -411,47 +392,15 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
 
   // ===== TMA producers (in pair mode: in both CTAs, each for its own shared memory) =====
   // The A and the B boxes of a stage are issued by two producer warps (0 and 10), each with its own expect_tx arrival on the stage's
-  // full barrier (loader 3; loader 0 = one producer for both).  That split dates from the thread-divergent issue path, where every
-  // TMA instruction cost ~500 clocks of waterfall (the "30 B/clk per issuing thread" of tools/exp/ingest_probe.cu); with elect_one()
-  // one producer does as well (tools/nt_exp.py), the second is kept because it costs nothing.  which: 0 = A and B, 1 = A only,
-  // 2 = B only.  Warp 11 can run L2 PREFETCHES of the A boxes p.prefetch k-blocks ahead (OGL_GEMM_PF_NT; off: measured slower before
-  // and after the issue fix -- the kernel is bound by L2 -> SM bytes, not by the latency of its misses).  The prefetcher paces itself
-  // on a progress counter in shared memory that the A producer advances once per stage.
-  // (run by ONE lane of warp 11) the L2 prefetcher of the A boxes: paces itself on the A producer's progress counter
-  auto l2_prefetcher = [&]() {
-    // prefetch cursor: (tile, segment, k-block) of the position p.prefetch k-blocks ahead, across segment and tile boundaries
-    int pt = unit, pseg = 0, pkb = 0;
-    auto pf_issue = [&]() {
-      while (pt < total_tiles) {                    // settle on the first live position at or after the cursor
-        bool found = false;
-        while (pseg < p.n_seg) {
-          if ((pt / p.n_tiles) * CG * BM < rows_valid[pseg] && pkb < (p.k[pseg] + BKE - 1) / BKE) { found = true; break; }
-          ++pseg; pkb = 0;
-        }
-        if (found) break;
-        pseg = 0; pkb = 0; pt += n_units;
-      }
-      if (pt < total_tiles) {
-        tma_prefetch_2d(&p.ta[pseg], pkb * BKE, ((pt / p.n_tiles) * CG + rank) * BM);
-        ++pkb;
-      }
-    };
-    volatile int* prog = (volatile int*)(s.tmem_slot + 2);          // k-blocks the A producer has issued so far
-    for (int n_pf = 0; pt < total_tiles; ++n_pf) {
-      while (n_pf - *prog >= p.prefetch) __nanosleep(64);
-      pf_issue();
-    }
-  };
+  // full barrier.  That split dates from the thread-divergent issue path, where every TMA instruction cost ~500 clocks of waterfall
+  // (the "30 B/clk per issuing thread" of tools/exp/ingest_probe.cu); with elect_one() one producer does as well, the second is kept
+  // because it costs nothing.  Warp 11 is idle.
   // (run by ALL lanes of a producer warp, converged; the copies themselves are issued by the elected lane)
-  auto tma_producer = [&](int which) {
+  auto tma_producer = [&](bool a_boxes) {
     int stage = 0;
     uint32_t phase = 0;
-    volatile int* prog = (volatile int*)(s.tmem_slot + 2);
-    int n_issued = 0;
     // bytes this producer lands per stage on the barrier the MMA issuer waits on (pair mode: both CTAs' boxes, on the leader's)
-    const uint32_t tx_a = (uint32_t)(CG * A_STAGE_BYTES);
-    const uint32_t tx_b = CG == 2 ? (uint32_t)(2 * (p.bn / 2) * 128) : (uint32_t)(p.bn * 128);
-    const uint32_t tx = which == 0 ? tx_a + tx_b : (which == 1 ? tx_a : tx_b);
+    const uint32_t tx = a_boxes ? (uint32_t)(CG * A_STAGE_BYTES) : (CG == 2 ? (uint32_t)(2 * (p.bn / 2) * 128) : (uint32_t)(p.bn * 128));
     int mt, nb;
     for (int it = 0; tile_at(it, mt, nb); ++it) {
       const int mb = mt * CG + rank;
@@ -461,17 +410,15 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
         const int nkb = (p.k[seg] + BKE - 1) / BKE;
         for (int kb = 0; kb < nkb; ++kb) {
           mbar_wait(&s.empty[stage], phase ^ 1);
-          ++n_issued;
           if (elect_one()) {
-            if (which != 2 && p.prefetch > 0) *prog = n_issued;
             if (CG == 2) {
               if (rank == 0) mbar_expect_tx(&s.full[stage], tx);
-              if (which != 2) tma_load_2d_pair(s.a(stage), &p.ta[seg], &s.full[stage], kb * BKE, mb * BM);
-              if (which != 1) tma_load_2d_pair(s.b(stage), &p.tb[seg], &s.full[stage], kb * BKE, nb * BN_MAX + rank * (bn_tile / 2));
+              if (a_boxes) tma_load_2d_pair(s.a(stage), &p.ta[seg], &s.full[stage], kb * BKE, mb * BM);
+              else tma_load_2d_pair(s.b(stage), &p.tb[seg], &s.full[stage], kb * BKE, nb * BN_MAX + rank * (bn_tile / 2));
             } else {
               mbar_expect_tx(&s.full[stage], tx);
-              if (which != 2) tma_load_2d(s.a(stage), &p.ta[seg], &s.full[stage], kb * BKE, mb * BM);
-              if (which != 1) tma_load_2d(s.b(stage), &p.tb[seg], &s.full[stage], kb * BKE, nb * BN_MAX);
+              if (a_boxes) tma_load_2d(s.a(stage), &p.ta[seg], &s.full[stage], kb * BKE, mb * BM);
+              else tma_load_2d(s.b(stage), &p.tb[seg], &s.full[stage], kb * BKE, nb * BN_MAX);
             }
           }
           __syncwarp();
@@ -481,7 +428,7 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
     }
   };
   if (warp == 0) {
-    if (!(p.debug & 2)) tma_producer(p.loader == 3 ? 1 : 0);
+    tma_producer(true);
     __syncwarp();
   } else if (warp == 1) {
     // ===== MMA issuer (pair mode: the leader CTA only): the whole warp runs the loop, the elected lane issues =====
@@ -505,7 +452,7 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
           const int K = p.k[seg];
           const int nkb = (K + BKE - 1) / BKE;
           for (int kb = 0; kb < nkb; ++kb) {
-            if (!(p.debug & 2)) mbar_wait(&s.full[stage], phase);      // (debug 2: MMA issue rate alone, operands = stale smem)
+            mbar_wait(&s.full[stage], phase);
             tc_fence_after();
             // descriptors of this stage: the 14-bit address field advances by 2 (= 32 bytes) per k step of one MMA (16 bf16 /
             // 8 tf32 elements); the issue loop is kept branch-free for full k-blocks so that the tensor pipe never waits on this thread
@@ -522,10 +469,8 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
                 const int n_ki = (k_left + KI - 1) / KI;
                 for (int ki = 0; ki < n_ki; ++ki) tc_mma<CG, TF>(d_tmem, ad + 2 * ki, bd + 2 * ki, idesc, ki ? 1u : accumulate);
               }
-              if (!(p.debug & 2)) {
-                if (CG == 2) tc_commit_pair(&s.empty[stage]);
-                else tc_commit(&s.empty[stage]);
-              }
+              if (CG == 2) tc_commit_pair(&s.empty[stage]);
+              else tc_commit(&s.empty[stage]);
             }
             __syncwarp();
             accumulate = 1;
@@ -542,12 +487,9 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
     }
     __syncwarp();
   } else if (warp >= 10) {
-    // ===== second TMA producer (warp 10) =====
-    if (p.loader == 3) {
-      if (warp == 10 && !(p.debug & 2)) tma_producer(2);      // the second TMA producer: the B boxes
-      if (warp == 11 && lane == 0 && !(p.debug & 2) && p.prefetch > 0) l2_prefetcher();      // the L2 prefetcher of the A boxes
-      __syncwarp();
-    }
+    // ===== second TMA producer (warp 10): the B boxes =====
+    if (warp == 10) tma_producer(false);
+    __syncwarp();
   } else {
     // ===== epilogue: TMEM -> registers -> bias / ReLU / mask -> swizzled smem box -> TMA store =====
     const int quarter = warp & 3;                 // TMEM lanes [32*quarter, +32) are this warp's
@@ -581,9 +523,7 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
       epi_barrier();
       mbar_wait(&s.acc_full[acc], acc_phase);
       tc_fence_after();
-      if (p.debug & 1) {
-        // nothing: measures the load + MMA pipeline alone
-      } else if (TF && p.out_f32_tma) {
+      if (TF && p.out_f32_tma) {
         // fp32 activations of the tf32 mode: one 32 x 32 fp32 box (32 rows of 128 bytes) per step, TF32-rounded, TMA store
         for (int c0 = parity * 32; c0 < bn_tile; c0 += 64) {
           if (boxes_issued >= 1) {
@@ -794,7 +734,6 @@ struct TnParams {
   int n_prob;
   int total_tiles, splits;
   int use_tma_store;
-  int prefetch;                  // contraction blocks both operands are prefetched into L2 ahead of their loads (0: off)
   float alpha_direct;            // output scale of the un-staged single-split store (staged partials are scaled by the reduce)
   const int32_t* m_dev;
   int m_max;
@@ -1078,13 +1017,8 @@ int make_map_f32_3d(CUtensorMap* map, const void* ptr, int64_t d0, int64_t d1, i
 
 bool gemm_tc_available() { return tc_init() == 1; }
 
-// programmatic dependent launch on every tcgen05 GEMM (OGL_PDL=0 turns it off): the row counts the kernels read before their
-// griddepcontrol.wait are written by the sampling kernels of an earlier launch sequence, never by the immediate predecessor
-static bool use_pdl() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("OGL_PDL"); v = e ? (atoi(e) != 0) : 1; }
-  return v == 1;
-}
+// programmatic dependent launch on every tcgen05 GEMM: the row counts the kernels read before their griddepcontrol.wait are
+// written by the sampling kernels of an earlier launch sequence, never by the immediate predecessor
 template <typename Kernel, typename Params>
 static int launch_gemm(Kernel kernel, int grid, int block, int smem, int cluster, const Params& p, cudaStream_t s) {
   cudaLaunchConfig_t cfg = {};
@@ -1099,11 +1033,9 @@ static int launch_gemm(Kernel kernel, int grid, int block, int smem, int cluster
     attrs[n].val.clusterDim.x = (unsigned)cluster; attrs[n].val.clusterDim.y = 1; attrs[n].val.clusterDim.z = 1;
     ++n;
   }
-  if (use_pdl()) {
-    attrs[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attrs[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
+  attrs[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attrs[n].val.programmaticStreamSerializationAllowed = 1;
+  ++n;
   cfg.attrs = attrs;
   cfg.numAttrs = (unsigned)n;
   OGL_CUDA(cudaLaunchKernelEx(&cfg, kernel, p));
@@ -1152,27 +1084,13 @@ int gemm_nt_tc(const GemmNT& g, cudaStream_t s) {
   p.out_f32_tma = (tf && (g.out_tf32 || g.mask)) ? 1 : 0;
   p.round_out = g.out_tf32;
   p.zero_tail = g.zero_tail;
-  {
-    static int dbg = -1, pfd = -1, ldr = -1, ord = -1;
-    if (ord < 0) { const char* e = getenv("OGL_NT_ORDER"); ord = e ? atoi(e) : 0; }
-    p.order = ord;
-    if (dbg < 0) { const char* e = getenv("OGL_GEMM_DBG"); dbg = e ? atoi(e) : 0; }
-    if (ldr < 0) { const char* e = getenv("OGL_GEMM_LOADER"); ldr = e ? atoi(e) : 3; }
-    if (ldr != 0) ldr = 3;
-    p.loader = ldr;
-    // (measured, tf32 fc_pool GEMM: 140 us without the prefetcher, 150 us with it 12 k-blocks ahead -- off by default)
-    if (pfd < 0) { const char* e = getenv("OGL_GEMM_PF_NT"); pfd = e ? atoi(e) : 0; }
-    p.debug = dbg;
-    p.prefetch = ord == 0 ? pfd : 0;      // (the prefetcher's cursor follows the round-robin order)
-  }
   OGL_ARG(!(g.mask && !(g.out_bf16 || p.out_f32_tma)), "gemm_nt_tc: the mask epilogue is implemented for the TMA-store outputs only");
   if (g.out_bf16) OGL_TRY(make_map(&p.tc, g.c, g.m_max, g.ldc, g.ldc, 64, 32, 2, CU_TENSOR_MAP_SWIZZLE_128B, g.f16));
   if (p.out_f32_tma) OGL_TRY(make_map(&p.tc, g.c, g.m_max, g.ldc, g.ldc, 32, 32, 4));
   OGL_ARG(g.ldc % 8 == 0 && ((uintptr_t)g.c & 15) == 0, "gemm_nt_tc: output pitch must be a multiple of 8 elements");
   OGL_ARG(!g.mask || (g.ldmask % 8 == 0 && ((uintptr_t)g.mask & 15) == 0), "gemm_nt_tc: mask pitch must be a multiple of 8 elements");
   if (cg == 2) {
-    int pairs = (int)(super_tiles < sm_count() / 2 ? super_tiles : sm_count() / 2);
-    if (const char* e = getenv("OGL_NT_MAXPAIRS")) pairs = pairs < atoi(e) ? pairs : atoi(e);      // experiments: is the kernel bound per SM or chip-wide?
+    const int pairs = (int)(super_tiles < sm_count() / 2 ? super_tiles : sm_count() / 2);
     if (tf) OGL_TRY(launch_gemm(k_gemm_nt_tc<2, 1>, 2 * pairs, THREADS_NT, SMEM_NT2, 2, p, s));
     else if (g.f16) OGL_TRY(launch_gemm(k_gemm_nt_tc<2, 2>, 2 * pairs, THREADS_NT, SMEM_NT2, 2, p, s));
     else OGL_TRY(launch_gemm(k_gemm_nt_tc<2, 0>, 2 * pairs, THREADS_NT, SMEM_NT2, 2, p, s));
@@ -1218,7 +1136,6 @@ int gemm_tn_tc_group(const GemmTN* g, int count, cudaStream_t s) {
   p.total_tiles = tiles;
   // one CTA per SM and exactly one wave: tiles * splits <= #SMs (150 CTAs on 148 SMs would run as two waves)
   int splits = sm_count() / tiles;
-  if (const char* e = getenv("OGL_TN_MAXCTAS")) splits = atoi(e) / tiles > 0 ? (splits < atoi(e) / tiles ? splits : atoi(e) / tiles) : 1;
   const int by_rows = (int)ceil_div(g[0].m_max, 4 * cw);          // at least 4 contraction blocks per split
   if (splits > by_rows) splits = by_rows;
   float* ws = g[0].partial;
@@ -1251,11 +1168,6 @@ int gemm_tn_tc_group(const GemmTN* g, int count, cudaStream_t s) {
   }
   p.use_tma_store = staged ? 1 : 0;
   p.alpha_direct = g[0].alpha;
-  {
-    static int pfd = -1;
-    if (pfd < 0) { const char* e = getenv("OGL_GEMM_PF_TN"); pfd = e ? atoi(e) : 0; }
-    p.prefetch = pfd;
-  }
   if (tf) OGL_TRY(launch_gemm(k_gemm_tn_tc<1>, tiles * splits, THREADS, SMEM_TN, 1, p, s));
   else if (g[0].f16) OGL_TRY(launch_gemm(k_gemm_tn_tc<2>, tiles * splits, THREADS, SMEM_TN, 1, p, s));
   else OGL_TRY(launch_gemm(k_gemm_tn_tc<0>, tiles * splits, THREADS, SMEM_TN, 1, p, s));
@@ -1276,7 +1188,6 @@ extern "C" int ogl_gemm_bf16_nt(const void* a_dev, int lda, const void* b_dev, i
   GemmNT g;
   g.a[0] = a_dev; g.lda[0] = lda; g.b[0] = b_dev; g.ldb[0] = ldb; g.k[0] = k; g.n_seg = 1;
   g.c = c_dev; g.ldc = ldc; g.m_max = m; g.n = n; g.in_bf16 = 1; g.out_bf16 = 0; g.zero_tail = 0;
-  if (const char* e = getenv("OGL_GEMM_CG")) g.force_cg = atoi(e);          // tests: force the 1-CTA / CTA-pair kernel
   return gemm_nt_tc(g, (cudaStream_t)stream);
 }
 

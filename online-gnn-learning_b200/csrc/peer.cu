@@ -17,7 +17,6 @@
 #include "common.cuh"
 #include "sage_kernels.cuh"
 #include "peer.cuh"
-#include <stdlib.h>
 
 namespace ogl {
 
@@ -25,14 +24,13 @@ namespace {
 
 constexpr int kMaxWorld = 8;
 constexpr int kFlagWords = 64;                    // per rank: arrive[8] | pad | done[8] | pad | cta counter
-constexpr int kArrive = 0, kDone = 16, kCounter = 32, kCounter2 = 33, kEpoch = 34, kGathered = 40;
+constexpr int kArrive = 0, kDone = 16, kCounter = 32, kEpoch = 34;
 // kEpoch: exchanges this rank has completed.  The kernels take their epoch from this word (every CTA of a launch reads it before the
 // launch's last CTA advances it), not from a kernel argument: an exchange can then sit inside a captured CUDA graph that is
 // replayed every step
 constexpr long long kSpinLimit = 20000000000ll;   // ~10 s of SM clocks: a missing peer traps instead of hanging the box
 
 struct PeerView {
-  float* gsum[kMaxWorld];          // two-shot mode: every rank's buffer of reduced gradients (written by the slice owners)
   const float* grads[kMaxWorld];
   uint32_t* flags[kMaxWorld];
   int rank, world;
@@ -56,9 +54,6 @@ __device__ __forceinline__ float4 ld_peer4(const float* p) {
   asm volatile("ld.relaxed.sys.global.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p) : "memory");
   return v;
 }
-__device__ __forceinline__ void st_peer4(float* p, float4 v) {
-  asm volatile("st.relaxed.sys.global.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
 __device__ __forceinline__ void spin_until(const uint32_t* flag, uint32_t epoch) {
   const long long t0 = clock64();
   while ((int32_t)(ld_acquire_sys(flag) - epoch) < 0) {
@@ -79,13 +74,9 @@ __device__ __forceinline__ void shadow_one(int64_t i, float pi, const ShadowSeg*
     ((T*)q.wt)[(int64_t)c * q.pitch_out + o] = from_f32<T>(pi);
   }
 }
-// grads of [lo, hi): summed over the ranks in rank order, Adam (same arithmetic as k_adam_shadow) on the local replica.
-// TWO_SHOT = false: every rank loads every peer's gradients itself (W - 1 remote loads per element: fewest synchronisations, best
-// for 2-3 ranks).  TWO_SHOT = true (reduce-scatter + all-gather inside the kernel): rank r sums only its 1/W slice of the range and
-// stores the sums into the `gsum` buffer of EVERY rank (P2P stores), a second flag barrier follows, then every rank runs Adam over
-// the whole range from its local gsum -- (W - 1) / W remote loads + stores per element instead of W - 1 loads.  All CTAs of the
-// grid are resident (<= 1 per SM): the second barrier is grid-wide.
-template <typename T, bool TWO_SHOT>
+// grads of [lo, hi): summed over the ranks in rank order, Adam (same arithmetic as k_adam_shadow) on the local replica.  Every rank
+// loads every peer's gradients itself (W - 1 remote loads per element, one flag barrier).
+template <typename T>
 __global__ void __launch_bounds__(256) k_peer_sum_adam(const PeerView pv, int64_t lo, int64_t hi, float* __restrict__ p,
                                                        float* __restrict__ m, float* __restrict__ v, float lr, float b1, float b2, float eps,
                                                        const uint32_t* __restrict__ t_dev, const ShadowSeg* __restrict__ segs, int n_segs,
@@ -108,11 +99,8 @@ __global__ void __launch_bounds__(256) k_peer_sum_adam(const PeerView pv, int64_
   // together: an NVLink round trip is paid once per quad, not once per rank
   const int64_t lo4 = (lo + 3) & ~(int64_t)3, hi4 = hi & ~(int64_t)3;
   const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, nth = (int64_t)gridDim.x * blockDim.x;
-  if (TWO_SHOT && lo4 < hi4) {
-    // ---- reduce-scatter: my slice of the quads, summed over the ranks, stored to every rank's gsum
-    const int64_t q0 = lo4 / 4, nq = hi4 / 4 - q0, per = (nq + W - 1) / W;
-    const int64_t s0 = q0 + per * pv.rank, s1 = (s0 + per < q0 + nq) ? s0 + per : q0 + nq;
-    for (int64_t q = s0 + tid; q < s1; q += nth) {
+  if (lo4 < hi4) {
+    for (int64_t q = lo4 / 4 + tid; q < hi4 / 4; q += nth) {
       float4 gr[kMaxWorld];
 #pragma unroll
       for (int r = 0; r < kMaxWorld; ++r)
@@ -121,40 +109,6 @@ __global__ void __launch_bounds__(256) k_peer_sum_adam(const PeerView pv, int64_
 #pragma unroll
       for (int r = 1; r < kMaxWorld; ++r)
         if (r < W) { g.x += gr[r].x; g.y += gr[r].y; g.z += gr[r].z; g.w += gr[r].w; }
-#pragma unroll
-      for (int r = 0; r < kMaxWorld; ++r)
-        if (r < W) st_peer4(pv.gsum[r] + q * 4, g);
-    }
-    // ---- all ranks' slices have landed everywhere: grid-wide (CTA counter) then box-wide (flags) barrier
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      uint32_t* counter = pv.flags[pv.rank] + kCounter2;
-      __threadfence_system();
-      const uint32_t old = atomicAdd(counter, 1u);
-      if (old == gridDim.x - 1) {
-        *counter = 0;
-        __threadfence_system();
-        for (int r = 0; r < W; ++r) st_release_sys(pv.flags[r] + kGathered + pv.rank, epoch);
-      }
-    }
-    if (threadIdx.x < W) spin_until(pv.flags[pv.rank] + kGathered + threadIdx.x, epoch);
-    __syncthreads();
-  }
-  if (lo4 < hi4) {
-    for (int64_t q = lo4 / 4 + tid; q < hi4 / 4; q += nth) {
-      float4 g;
-      if (TWO_SHOT) {
-        g = ld_peer4(pv.gsum[pv.rank] + q * 4);
-      } else {
-        float4 gr[kMaxWorld];
-#pragma unroll
-        for (int r = 0; r < kMaxWorld; ++r)
-          if (r < W) gr[r] = ld_peer4(pv.grads[r] + q * 4);
-        g = gr[0];
-#pragma unroll
-        for (int r = 1; r < kMaxWorld; ++r)
-          if (r < W) { g.x += gr[r].x; g.y += gr[r].y; g.z += gr[r].z; g.w += gr[r].w; }
-      }
       float4 m4 = *reinterpret_cast<const float4*>(m + q * 4);
       float4 v4 = *reinterpret_cast<const float4*>(v + q * 4);
       float4 p4 = *reinterpret_cast<const float4*>(p + q * 4);
@@ -214,9 +168,8 @@ using namespace ogl;
 struct ogl_peer {
   int rank = 0, world = 1;
   int64_t n_floats = 0;
-  void* base = nullptr;                 // local allocation: [n_floats fp32 gradients | n_floats reduced gradients | kFlagWords uint32 flags]
-  size_t gsum_off = 0, flags_off = 0;
-  int two_shot = 0;                     // exchange algorithm (same on every rank): 0 = one-shot, 1 = reduce-scatter + all-gather
+  void* base = nullptr;                 // local allocation: [n_floats fp32 gradients | kFlagWords uint32 flags]
+  size_t flags_off = 0;
   void* peer_base[kMaxWorld] = {};      // mapped peers (own slot = base)
   int opened[kMaxWorld] = {};
   int connected = 0;
@@ -229,10 +182,7 @@ extern "C" int ogl_peer_create(ogl_peer** out, int rank, int world, int64_t n_fl
           "ogl_peer_create: need 0 <= rank < world <= %d and n_floats > 0", kMaxWorld);
   ogl_peer* p = new ogl_peer();
   p->rank = rank; p->world = world; p->n_floats = n_floats;
-  p->gsum_off = ((size_t)n_floats * 4 + 255) / 256 * 256;
-  p->flags_off = 2 * p->gsum_off;
-  p->two_shot = 0;      // measured on 8 B200: one-shot 0.708 ms / step, two-shot 0.737 (the second barrier costs more than the bytes save)
-  if (const char* e = getenv("OGL_PEER_TWO_SHOT")) p->two_shot = atoi(e) != 0;     // experiments / tests (must agree on all ranks)
+  p->flags_off = ((size_t)n_floats * 4 + 255) / 256 * 256;
   OGL_CUDA(cudaMalloc(&p->base, p->flags_off + kFlagWords * 4));
   OGL_CUDA(cudaMemset(p->base, 0, p->flags_off + kFlagWords * 4));
   OGL_CUDA(cudaDeviceSynchronize());
@@ -241,7 +191,6 @@ extern "C" int ogl_peer_create(ogl_peer** out, int rank, int world, int64_t n_fl
     p->connected = 1;
     p->view.rank = 0; p->view.world = 1;
     p->view.grads[0] = (const float*)p->base;
-    p->view.gsum[0] = (float*)((char*)p->base + p->gsum_off);
     p->view.flags[0] = (uint32_t*)((char*)p->base + p->flags_off);
   }
   *out = p;
@@ -271,7 +220,6 @@ static void finish_connect(ogl_peer* p) {
   p->view.rank = p->rank; p->view.world = p->world;
   for (int r = 0; r < p->world; ++r) {
     p->view.grads[r] = (const float*)p->peer_base[r];
-    p->view.gsum[r] = (float*)((char*)p->peer_base[r] + p->gsum_off);
     p->view.flags[r] = (uint32_t*)((char*)p->peer_base[r] + p->flags_off);
   }
   p->connected = 1;
@@ -332,24 +280,13 @@ int peer_sum_adam(ogl_peer* p, const PeerAdamArgs& a, int64_t lo, int64_t hi, cu
   int grid = (int)ceil_div(quads, 256);
   if (grid > 2 * sm_count()) grid = 2 * sm_count();
   if (grid < 1) grid = 1;
-  const bool two = p->two_shot && p->world > 1;
-  if (two && grid > sm_count()) grid = sm_count();          // grid-wide barrier inside: every CTA resident
-#define OGL_PEER_LAUNCH(T, TWO)                                                                                                          \
-  OGL_LAUNCH((k_peer_sum_adam<T, TWO>), grid, 256, 0, s, p->view, lo, hi, a.params, a.m, a.v, a.lr, a.b1, a.b2, a.eps, a.t_dev, \
+#define OGL_PEER_LAUNCH(T)                                                                                                          \
+  OGL_LAUNCH((k_peer_sum_adam<T>), grid, 256, 0, s, p->view, lo, hi, a.params, a.m, a.v, a.lr, a.b1, a.b2, a.eps, a.t_dev, \
              a.segs, a.n_segs, a.reduced_out)
-  if (a.mode == OGL_BF16) {
-    if (two) OGL_PEER_LAUNCH(__nv_bfloat16, true);
-    else OGL_PEER_LAUNCH(__nv_bfloat16, false);
-  } else if (a.mode == OGL_FP16) {
-    if (two) OGL_PEER_LAUNCH(__half, true);
-    else OGL_PEER_LAUNCH(__half, false);
-  } else if (a.mode == OGL_TF32) {
-    if (two) OGL_PEER_LAUNCH(tf32_t, true);
-    else OGL_PEER_LAUNCH(tf32_t, false);
-  } else {
-    if (two) OGL_PEER_LAUNCH(float, true);
-    else OGL_PEER_LAUNCH(float, false);
-  }
+  if (a.mode == OGL_BF16) OGL_PEER_LAUNCH(__nv_bfloat16);
+  else if (a.mode == OGL_FP16) OGL_PEER_LAUNCH(__half);
+  else if (a.mode == OGL_TF32) OGL_PEER_LAUNCH(tf32_t);
+  else OGL_PEER_LAUNCH(float);
 #undef OGL_PEER_LAUNCH
   return OGL_OK;
 }

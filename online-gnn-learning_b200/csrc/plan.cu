@@ -163,12 +163,6 @@ struct ogl_plan {
   int use_side = 1;
   cudaStream_t side = nullptr;
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  int fuse_head = 0;                     // train steps run the last layer's segmax + output GEMM + loss + dneigh GEMM as ONE kernel
-                                         // (k_head_fused; option "fuse_head" / OGL_FUSE_HEAD=1).  OFF by default: 36 us against 58 us for
-                                         // the five launches it replaces when timed alone, but the graph-replayed, overlapped step does
-                                         // not get shorter (0.535 vs 0.534 ms) and the end-to-end loop gets slower -- DESIGN.md section 3
-  int head_active = 0;                   // ... set by step_body around forward / loss / backward of a step
-  uint32_t* head_counter = nullptr;      // the fused head's "CTAs done" word (zero between launches)
   float head_loss_scale = 0.f;           // loss scale of the last ogl_plan_step_finish_head (its tail must unscale by the same)
   float grad_scale = 1.f;                // mode OGL_FP16: the loss scale the stored activation gradients of the current backward pass carry
   int skip_gather = 0;                   // step_finish: the input rows were already gathered by step_begin
@@ -176,7 +170,6 @@ struct ogl_plan {
   int adam_in_backward = 0;              // fused step with do_step: the backward pass runs Adam on all but the last gradient itself
   int64_t adam_done_from = 0;            // ... and leaves [0, adam_done_from) to ogl_plan_adam_step
   ogl_peer* dp_peer = nullptr;           // step kind 5: the peer group of the data-parallel finish being enqueued / captured
-  int tail_part = 0, tail_parts = 1;     // tail_mode 2: the last weight-gradient GEMM in `tail_parts` pieces of 256 output rows each
   int tail_mode = 0;                     // backward: 0 = all, 1 = everything but the last weight-gradient GEMM (layer 0 fc_pool),
                                          // 2 = only that GEMM (data-parallel: its predecessors' gradients are already on the wire)
   int in_train_step = 0;                 // set by the fused train step: sampling may defer the reverse edge lists to the side stream
@@ -191,12 +184,11 @@ struct ogl_plan {
     int n_seeds, do_step;
     float loss_scale;
     int kind;            // 0 = whole step, 1 = step_begin (sample + gather), 2 = step_finish (forward .. Adam),
-                         // 3 = step_finish minus the last weight-gradient GEMM, 4 = that GEMM
+                         // 3 = step_finish minus the last weight-gradient GEMM, 4 = that GEMM, 5 = data-parallel finish
     int parity;          // which of the two minibatch buffer sets the captured pointers belong to
-    int part, parts;     // kind 4: piece of the last weight-gradient GEMM
     bool operator==(const StepKey& o) const {
       return g == o.g && f == o.f && per == o.per && loss == o.loss && g_gen == o.g_gen && n_seeds == o.n_seeds && do_step == o.do_step &&
-             loss_scale == o.loss_scale && kind == o.kind && parity == o.parity && part == o.part && parts == o.parts;
+             loss_scale == o.loss_scale && kind == o.kind && parity == o.parity;
     }
   };
   struct StepGraph { StepKey key; cudaGraphExec_t exec; uint64_t last_use; };
@@ -237,6 +229,14 @@ static void prof_end(ogl_plan* p, cudaStream_t s) {
   ogl_plan::ProfRec& r = p->prof_recs[p->prof_used++];
   r.launches = g_launches.load() - r.launches;
   cudaEventRecord(r.e1, s);
+}
+// stage profiling: the level row counts of the step just enqueued, for the per-step averages of ogl_plan_profile_read
+static int record_level_counts(ogl_plan* p, cudaStream_t s) {
+  if (p->prof_on && p->prof_steps < kProfSteps) {
+    OGL_CUDA(cudaMemcpyAsync(p->prof_counts_host + 8 * p->prof_steps, p->counts, sizeof(int32_t) * (p->L + 1), cudaMemcpyDeviceToHost, s));
+    p->prof_steps++;
+  }
+  return OGL_OK;
 }
 #define STAGE(name, call)            \
   do {                               \
@@ -386,8 +386,6 @@ extern "C" int ogl_plan_create(ogl_plan** out, const ogl_plan_config* cfg) {
   OGL_CUDA(cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming));
   DM0(p->per_loss, sizeof(float) * cfg->max_seeds);
   DM0(p->loss_sum, sizeof(float) * 4);
-  DM0(p->head_counter, sizeof(uint32_t) * 4);
-  if (const char* e = getenv("OGL_FUSE_HEAD")) p->fuse_head = atoi(e) != 0;
   DM0(p->adam_m, sizeof(float) * p->n_params);
   DM0(p->adam_v, sizeof(float) * p->n_params);
   *out = p;
@@ -413,7 +411,7 @@ extern "C" int ogl_plan_destroy(ogl_plan* p) {
     for (auto x : *v) cudaFree(x);
   cudaFree(p->alt.counts); cudaFree(p->alt.x); cudaFree(p->alt.seeds_stage);
   void* ptrs[] = {p->counts, p->ctl, p->seeds_stage, p->tn_partial, p->colsum_partial, p->per_loss,
-                  p->loss_sum, p->adam_m, p->adam_v, p->shadow_segs, p->head_counter};
+                  p->loss_sum, p->adam_m, p->adam_v, p->shadow_segs};
   for (void* q : ptrs) cudaFree(q);
   for (auto& r : p->prof_recs) { cudaEventDestroy(r.e0); cudaEventDestroy(r.e1); }
   cudaDeviceSynchronize();
@@ -535,7 +533,6 @@ extern "C" int ogl_plan_forward(ogl_plan* p, ogl_features* f, float* logits_dev,
     g1.c = lb.hp; g1.ldc = lb.pin; g1.m_max = p->nmax[sl]; g1.m_dev = p->counts + sl; g1.n = lb.in;
     g1.in_bf16 = p->bf16; g1.out_bf16 = p->bf16; g1.f16 = p->fp16; g1.tf32 = p->tf32; g1.out_tf32 = p->tf32;
     STAGE(nm("l%d.pool_gemm", l).c_str(), gemm_nt(p, g1, s));
-    if (p->head_active && l == L - 1) break;       // the fused head (plan_loss) does the rest of the last layer
     STAGE(nm("l%d.segmax", l).c_str(),
           segmax_fwd(p->mode, lb.hp, lb.pin, p->edge_lid[h], p->cfg.fanouts[h], p->counts + dl, p->nmax[dl], lb.neigh, lb.arg, s));
     GemmNT g2;
@@ -571,15 +568,6 @@ static int plan_loss(ogl_plan* p, ogl_features* f, float scale, int want_grad, f
   LayerBuf& last = p->layer[L - 1];
   p->grad_scale = want_grad ? grad_scale_for(p, scale) : 1.f;
   scale *= p->grad_scale;
-  if (p->head_active) {
-    // last layer on the seed rows: segment max + [x_self | neigh] x [W_self | W_neigh]^T + cross entropy + loss sum + dneigh GEMM
-    float* per_h = per_vertex_loss_dev ? per_vertex_loss_dev : p->per_loss;
-    STAGE(nm("l%d.head", L - 1).c_str(),
-          head_fused(p->mode, last.hp, p->act[1], last.pin, last.in, p->edge_lid[0], p->cfg.fanouts[0], last.ws, last.wn, p->params + last.o_bs,
-                     p->params + last.o_bn, last.out, f->labels, p->nodes[0], p->counts, p->nmax[0], round_up(p->nmax[0], 128), scale, want_grad,
-                     last.neigh, last.arg, (float*)p->act[0], last.pout, per_h, last.dpre, last.pout, last.dng, loss_sum_dev, p->head_counter, s));
-    return OGL_OK;
-  }
   float* per = per_vertex_loss_dev ? per_vertex_loss_dev : p->per_loss;
   STAGE("xent", xent(p->mode, (const float*)p->act[0], last.pout, p->cfg.dims[L], f->labels, p->nodes[0], p->counts, p->nmax[0],
                      round_up(p->nmax[0], 128), scale, per, last.dpre, last.pout, want_grad, s));
@@ -615,17 +603,7 @@ static int plan_backward_layers(ogl_plan* p, cudaStream_t s) {
     return tp;
   };
   if (p->tail_mode == 2) {                        // only dWp of layer 0 (its dhp was left in place by the tail_mode 1 pass)
-    GemmTN tp = dw_pool(0);
-    if (p->tail_parts > 1) {
-      // one piece of 256 output rows: data-parallel runs exchange piece i over NVLink while piece i + 1 is computed, so that only
-      // the last (smallest) piece's exchange is exposed at the end of the step
-      const int r0 = p->tail_part * 256, r1 = std::min(tp.n, r0 + 256);
-      OGL_ARG(r0 < tp.n, "ogl_plan_step_finish_tail: part %d of %d is empty", p->tail_part, p->tail_parts);
-      tp.a = (const char*)tp.a + (size_t)r0 * p->es;
-      tp.c = tp.c + (int64_t)r0 * tp.ldc;
-      tp.n = r1 - r0;
-    }
-    STAGE("l0.dW_pool", gemm_tn(p, tp, s));
+    STAGE("l0.dW_pool", gemm_tn(p, dw_pool(0), s));
     return OGL_OK;
   }
   OGL_TRY(join_side(p, s));                      // reverse edge lists built on the side stream during sampling
@@ -663,7 +641,7 @@ static int plan_backward_layers(ogl_plan* p, cudaStream_t s) {
     n1.c = lb.dng; n1.ldc = lb.pin; n1.m_max = p->nmax[dl]; n1.m_dev = p->counts + dl; n1.n = lb.in;
     n1.in_bf16 = p->bf16; n1.out_bf16 = p->bf16; n1.f16 = p->fp16; n1.tf32 = p->tf32; n1.out_tf32 = p->tf32; n1.zero_tail = 0;
     n1.mask = lb.neigh; n1.ldmask = lb.pin;        // relu'(hp) at the argmax: neigh[d, f] == hp[src(arg), f]
-    if (!(p->head_active && l == L - 1)) STAGE(nm("l%d.dneigh_gemm", l).c_str(), gemm_nt(p, n1, s));      // (else: done by the fused head)
+    STAGE(nm("l%d.dneigh_gemm", l).c_str(), gemm_nt(p, n1, s));
     // fc_pool bias gradient: every dng[d, f] lands in exactly one source row, so colsum(dhp) == colsum(dng).  Side stream too (behind the
     // weight-gradient group): only Adam reads it
     if (ov) {
@@ -788,11 +766,6 @@ static int join_side(ogl_plan* p, cudaStream_t s) {
   return OGL_OK;
 }
 
-static int head_usable(const ogl_plan* p) {
-  const LayerBuf& last = p->layer[p->L - 1];
-  return p->fuse_head && head_fused_supported(p->mode, last.pin, last.out) ? 1 : 0;
-}
-
 static int step_body(ogl_plan* p, int kind, ogl_graph* g, ogl_features* f, int n_seeds, float loss_scale, int do_step,
                      float* per_vertex_loss_dev, float* loss_sum_dev, cudaStream_t s) {
   if (kind == 0 || kind == 1) {
@@ -826,7 +799,6 @@ static int step_body(ogl_plan* p, int kind, ogl_graph* g, ogl_features* f, int n
     p->skip_gather = 1;
     const int keep_mode = p->train_mode;
     p->train_mode = 1;
-    p->head_active = head_usable(p);
     int r = ogl_plan_forward(p, f, nullptr, s);
     p->skip_gather = 0;
     // the peers must have finished reading my previous gradients before this step's backward pass overwrites them: checked HERE,
@@ -838,7 +810,6 @@ static int step_body(ogl_plan* p, int kind, ogl_graph* g, ogl_features* f, int n
       r = ogl_plan_loss_backward(p, f, loss_scale, per_vertex_loss_dev, loss_sum_dev, s);
       p->tail_mode = 0;
     }
-    p->head_active = 0;
     p->train_mode = keep_mode;
     OGL_TRY(r);
     const int64_t n0 = p->layer[0].o_bp;            // = in * in: layer 0's fc_pool.weight leads the flat buffers
@@ -857,14 +828,12 @@ static int step_body(ogl_plan* p, int kind, ogl_graph* g, ogl_features* f, int n
   p->skip_gather = (kind == 2 || kind == 3);
   const int keep_mode = p->train_mode;
   p->train_mode = 1;                             // a train step: feat_drop on (the reference calls model.train() first, pytorch/model.py:120)
-  p->head_active = head_usable(p);
   const int rf = ogl_plan_forward(p, f, nullptr, s);
   p->skip_gather = 0;
-  if (rf != OGL_OK) { p->train_mode = keep_mode; p->head_active = 0; return rf; }
+  if (rf != OGL_OK) { p->train_mode = keep_mode; return rf; }
   p->tail_mode = (kind == 3) ? 1 : 0;
   p->adam_in_backward = (do_step && kind != 3) ? 1 : 0;
   const int rl = ogl_plan_loss_backward(p, f, loss_scale, per_vertex_loss_dev, loss_sum_dev, s);
-  p->head_active = 0;
   p->train_mode = keep_mode;
   p->tail_mode = 0;
   p->adam_in_backward = 0;
@@ -878,8 +847,7 @@ static int step_body(ogl_plan* p, int kind, ogl_graph* g, ogl_features* f, int n
 static int run_step(ogl_plan* p, int kind, ogl_graph* g, ogl_features* f, int n_seeds, float loss_scale, int do_step,
                     float* per_vertex_loss_dev, float* loss_sum_dev, cudaStream_t s) {
   if (!p->use_graph || p->prof_on) return step_body(p, kind, g, f, n_seeds, loss_scale, do_step, per_vertex_loss_dev, loss_sum_dev, s);
-  const ogl_plan::StepKey key{kind == 5 ? (const void*)p->dp_peer : (const void*)g, f, per_vertex_loss_dev, loss_sum_dev, g ? graph_generation(g) : 0, n_seeds, do_step, loss_scale, kind, p->parity,
-                              kind == 4 ? p->tail_part : 0, kind == 4 ? p->tail_parts : 1};
+  const ogl_plan::StepKey key{kind == 5 ? (const void*)p->dp_peer : (const void*)g, f, per_vertex_loss_dev, loss_sum_dev, g ? graph_generation(g) : 0, n_seeds, do_step, loss_scale, kind, p->parity};
   ogl_plan::StepGraph* hit = nullptr;
   for (auto& sg : p->step_graphs)
     if (sg.key == key) { hit = &sg; break; }
@@ -942,13 +910,7 @@ static int ensure_pipeline(ogl_plan* p) {
     DM0(a.rev_edge[h], sizeof(int32_t) * ne);
   }
   DM0(a.x, p->es * (size_t)round_up(p->nmax[L], 128) * pitch_of(p->cfg.dims[0]));
-  {
-    // OGL_PRE_PRIO (experiments): 1 = highest stream priority for the prefetch stream, -1 = lowest, 0 / unset = default
-    int least = 0, greatest = 0, prio = 0;
-    OGL_CUDA(cudaDeviceGetStreamPriorityRange(&least, &greatest));
-    if (const char* e = getenv("OGL_PRE_PRIO")) prio = atoi(e) > 0 ? greatest : (atoi(e) < 0 ? least : 0);
-    OGL_CUDA(cudaStreamCreateWithPriority(&p->pre, cudaStreamNonBlocking, prio));
-  }
+  OGL_CUDA(cudaStreamCreateWithFlags(&p->pre, cudaStreamNonBlocking));
   OGL_CUDA(cudaEventCreateWithFlags(&p->ev_tail, cudaEventDisableTiming));
   for (int i = 0; i < 2; ++i) OGL_CUDA(cudaEventCreateWithFlags(&p->ev_ready[i], cudaEventDisableTiming));
   OGL_CUDA(cudaMallocHost(&p->seed_ring, sizeof(int64_t) * ogl_plan::kSeedRing * p->cfg.max_seeds));
@@ -1053,11 +1015,7 @@ extern "C" int ogl_plan_train_step(ogl_plan* p, ogl_graph* g, ogl_features* f, c
     OGL_TRY(run_step(p, 0, g, f, n_seeds, loss_scale, do_step, per_vertex_loss_dev, loss_sum_dev, s));
     p->cur_open = 0;
   }
-  if (p->prof_on && p->prof_steps < kProfSteps) {
-    OGL_CUDA(cudaMemcpyAsync(p->prof_counts_host + 8 * p->prof_steps, p->counts, sizeof(int32_t) * (p->L + 1), cudaMemcpyDeviceToHost, s));
-    p->prof_steps++;
-  }
-  return OGL_OK;
+  return record_level_counts(p, s);
 }
 
 // `n_batches` consecutive train steps of `batch` seeds each in ONE call (the reference runs batch_timestep minibatches per
@@ -1121,35 +1079,13 @@ extern "C" int ogl_plan_step_finish_head(ogl_plan* p, ogl_features* f, float los
   return run_step(p, 3, nullptr, f, p->n_seeds, loss_scale, 0, per_vertex_loss_dev, loss_sum_dev, (cudaStream_t)stream);
 }
 
-extern "C" int ogl_plan_step_finish_tail_part(ogl_plan* p, ogl_features* f, int part, int n_parts, void* stream) {
-  OGL_ARG(p && f && p->params && p->n_seeds > 0, "ogl_plan_step_finish_tail: no step begun / parameters not bound");
-  OGL_ARG(n_parts >= 1 && part >= 0 && part < n_parts && (n_parts - 1) * 256 < p->cfg.dims[0],
-          "ogl_plan_step_finish_tail_part: part %d of %d (pieces are 256 rows of the %d x %d gradient)", part, n_parts, p->cfg.dims[0], p->cfg.dims[0]);
-  cudaStream_t s = (cudaStream_t)stream;
-  p->tail_part = part; p->tail_parts = n_parts;
-  const int r4 = run_step(p, 4, nullptr, f, p->n_seeds, p->head_loss_scale, 0, nullptr, nullptr, s);
-  p->tail_part = 0; p->tail_parts = 1;
-  if (part + 1 < n_parts) return r4;              // (the minibatch is released by the last piece)
-  advance_prefetched(p);
-  OGL_TRY(r4);
-  if (p->prof_on && p->prof_steps < kProfSteps) {
-    OGL_CUDA(cudaMemcpyAsync(p->prof_counts_host + 8 * p->prof_steps, p->counts, sizeof(int32_t) * (p->L + 1), cudaMemcpyDeviceToHost, s));
-    p->prof_steps++;
-  }
-  return OGL_OK;
-}
-
 extern "C" int ogl_plan_step_finish_tail(ogl_plan* p, ogl_features* f, void* stream) {
   OGL_ARG(p && f && p->params && p->n_seeds > 0, "ogl_plan_step_finish_tail: no step begun / parameters not bound");
   cudaStream_t s = (cudaStream_t)stream;
   const int r4 = run_step(p, 4, nullptr, f, p->n_seeds, p->head_loss_scale, 0, nullptr, nullptr, s);
   advance_prefetched(p);
   OGL_TRY(r4);
-  if (p->prof_on && p->prof_steps < kProfSteps) {
-    OGL_CUDA(cudaMemcpyAsync(p->prof_counts_host + 8 * p->prof_steps, p->counts, sizeof(int32_t) * (p->L + 1), cudaMemcpyDeviceToHost, s));
-    p->prof_steps++;
-  }
-  return OGL_OK;
+  return record_level_counts(p, s);
 }
 
 // data-parallel finish: forward .. backward with the gradient exchange over NVLink peer memory and Adam inside the same launch
@@ -1164,11 +1100,7 @@ extern "C" int ogl_plan_step_finish_dp(ogl_plan* p, ogl_peer* peer, ogl_features
   p->dp_peer = nullptr;
   advance_prefetched(p);
   OGL_TRY(r5);
-  if (p->prof_on && p->prof_steps < kProfSteps) {
-    OGL_CUDA(cudaMemcpyAsync(p->prof_counts_host + 8 * p->prof_steps, p->counts, sizeof(int32_t) * (p->L + 1), cudaMemcpyDeviceToHost, s));
-    p->prof_steps++;
-  }
-  return OGL_OK;
+  return record_level_counts(p, s);
 }
 
 extern "C" int ogl_plan_step_finish(ogl_plan* p, ogl_features* f, float loss_scale, int do_step, float* per_vertex_loss_dev,
@@ -1180,11 +1112,7 @@ extern "C" int ogl_plan_step_finish(ogl_plan* p, ogl_features* f, float loss_sca
   const int r2 = run_step(p, 2, nullptr, f, p->n_seeds, loss_scale, do_step, per_vertex_loss_dev, loss_sum_dev, s);
   advance_prefetched(p);
   OGL_TRY(r2);
-  if (p->prof_on && p->prof_steps < kProfSteps) {
-    OGL_CUDA(cudaMemcpyAsync(p->prof_counts_host + 8 * p->prof_steps, p->counts, sizeof(int32_t) * (p->L + 1), cudaMemcpyDeviceToHost, s));
-    p->prof_steps++;
-  }
-  return OGL_OK;
+  return record_level_counts(p, s);
 }
 
 extern "C" int ogl_plan_set_option(ogl_plan* p, const char* name, int value) {
@@ -1193,15 +1121,6 @@ extern "C" int ogl_plan_set_option(ogl_plan* p, const char* name, int value) {
   if (strcmp(name, "side_stream") == 0) { p->use_side = value ? 1 : 0; return OGL_OK; }
   if (strcmp(name, "pipeline") == 0) { p->use_pipeline = value ? 1 : 0; return OGL_OK; }
   if (strcmp(name, "train_mode") == 0) { p->train_mode = value ? 1 : 0; return OGL_OK; }
-  if (strcmp(name, "fuse_head") == 0) {            // (captured step graphs hold the old launch sequence)
-    if ((value ? 1 : 0) != p->fuse_head) {
-      OGL_CUDA(cudaDeviceSynchronize());
-      for (auto& sg : p->step_graphs) cudaGraphExecDestroy(sg.exec);
-      p->step_graphs.clear();
-    }
-    p->fuse_head = value ? 1 : 0;
-    return OGL_OK;
-  }
   set_error("ogl_plan_set_option: unknown option '%s'", name);
   return OGL_ERR_ARG;
 }

@@ -364,215 +364,6 @@ __global__ void __launch_bounds__(kBlock) k_xent(const float* __restrict__ logit
   }
 }
 
-// ---- fused head of the train step: the LAST layer's segment max, output GEMM, cross entropy, loss sum and dneigh GEMM ------------
-// On the seed rows (B = 1024 in the benchmarked configuration) these five launches do ~0.3 GFLOP and ~30 MB of work but cost
-// ~58 us of GPU time (two tcgen05 launches whose 8 CTAs walk a 19-block contraction one after the other, three latency-bound
-// kernels) plus the gaps between them.  Every one of them is ROW-LOCAL on the seed rows:
-//     neigh[d]   = max over d's sampled neighbours of hp[.]                       (first-slot-wins argmax, as k_segmax_fwd)
-//     logits[d]  = [x_self[d] | neigh[d]] . [W_self | W_neigh]^T + b_self + b_neigh
-//     loss[d], dlogits[d] = cross entropy(logits[d], label) * scale                (dlogits stored in the arithmetic type)
-//     dneigh[d]  = (dlogits[d] . W_neigh) masked by neigh[d] > 0
-// so ONE CTA per seed row does all of it: thread t owns the row's 16-byte column strip t (blockDim = strips rounded up to a warp), the
-// row's operands never leave registers, the 41-odd class sums meet in shared memory.  Products of two stored values are exact in
-// fp32 (fp16 / bf16 / TF32 operands), accumulation is fp32 in a fixed order (inside a strip, xor-shuffle tree over a warp's strips,
-// warps ascending): the arithmetic of the tensor-core kernels up to the summation order.  The last CTA to finish sums the
-// per-vertex losses in a fixed order (deterministic, as k_sum_f32).
-constexpr int kHeadMaxStrips = 256;  // pitch <= 256 * Vec<T>::N (2048 16-bit / 1024 32-bit elements)
-constexpr int kHeadMaxC = 64;        // classes: two per lane of the softmax warp
-template <typename T>
-__global__ void __launch_bounds__(kHeadMaxStrips) k_head_fused(const T* __restrict__ hp, const T* __restrict__ x, int pitch, int in,
-                                                               const int32_t* __restrict__ edge_lid, int fanout, const T* __restrict__ ws,
-                                                               const T* __restrict__ wn, const float* __restrict__ bs,
-                                                               const float* __restrict__ bn, int C, const int32_t* __restrict__ labels,
-                                                               const int32_t* __restrict__ nodes, const int32_t* __restrict__ n_dev, int n_max,
-                                                               int rows_buf, float scale, int want_grad, T* __restrict__ neigh,
-                                                               uint8_t* __restrict__ arg, float* __restrict__ logits, int ldl,
-                                                               float* __restrict__ per_loss, T* __restrict__ dlogits, int ldd,
-                                                               T* __restrict__ dng, float* __restrict__ loss_sum,
-                                                               uint32_t* __restrict__ done_counter) {
-  constexpr int NV = Vec<T>::N;
-  __shared__ float part[kHeadMaxStrips / 32][kHeadMaxC];     // per-warp partial class sums
-  __shared__ float dls[kHeadMaxC];                           // dlogits of the row, as stored
-  __shared__ float red[32];
-  __shared__ int is_last;
-  const int n = dyn_count(n_dev, n_max);
-  const int nz = pad128(n, rows_buf);
-  const int vpr = pitch / NV;
-  const int strip = threadIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
-  const bool live = strip < vpr;
-  const int r = blockIdx.x;
-  const int64_t at = (int64_t)r * pitch + strip * NV;
-  if (r >= n && r < nz) {                          // zero-tail rule: later contractions over the rows read up to the padded count
-    if (live) *reinterpret_cast<uint4*>(neigh + at) = make_uint4(0u, 0u, 0u, 0u);
-    if (want_grad)
-      for (int c = threadIdx.x; c < ldd; c += blockDim.x) dlogits[(int64_t)r * ldd + c] = from_f32<T>(0.f);
-  }
-  if (r < n) {
-    // ---- segment max over the row's sampled neighbours (slots compared in ascending order, five rows in flight)
-    float best[NV];
-    uint8_t slot[NV];
-#pragma unroll
-    for (int k = 0; k < NV; ++k) { best[k] = 0.f; slot[k] = 255; }
-    bool any = false;
-    const int32_t* el = edge_lid + (int64_t)r * fanout;
-    constexpr int kSlots = 5;
-    for (int j0 = 0; j0 < fanout; j0 += kSlots) {
-      int lid[kSlots];
-      uint4 raw[kSlots];
-#pragma unroll
-      for (int u = 0; u < kSlots; ++u) lid[u] = (j0 + u < fanout) ? __ldg(el + j0 + u) : -1;
-#pragma unroll
-      for (int u = 0; u < kSlots; ++u)
-        if (lid[u] >= 0 && live) raw[u] = __ldg(reinterpret_cast<const uint4*>(hp + (int64_t)lid[u] * pitch) + strip);
-#pragma unroll
-      for (int u = 0; u < kSlots; ++u) {
-        if (lid[u] < 0) continue;
-        if (live) {
-          const T* v = reinterpret_cast<const T*>(&raw[u]);
-#pragma unroll
-          for (int k = 0; k < NV; ++k) {
-            const float xv = to_f32<T>(v[k]);
-            if (!any || xv > best[k]) { best[k] = xv; slot[k] = (uint8_t)(j0 + u); }
-          }
-        }
-        any = true;
-      }
-    }
-    // neigh / arg rows leave for the backward pass (weight gradient, mask, max-pool backward); best[] holds exactly the stored values
-    if (live) {
-      T o[NV];
-#pragma unroll
-      for (int k = 0; k < NV; ++k) o[k] = from_f32<T>(best[k]);
-      *reinterpret_cast<uint4*>(neigh + at) = *reinterpret_cast<const uint4*>(o);
-      if (NV == 8) *reinterpret_cast<uint2*>(arg + at) = *reinterpret_cast<const uint2*>(slot);
-      else *reinterpret_cast<uint32_t*>(arg + at) = *reinterpret_cast<const uint32_t*>(slot);
-    }
-    // ---- logits: the row's own features and its neighbourhood maximum against the two weight matrices, four classes at a time
-    float xs[NV];
-    {
-      uint4 raw = make_uint4(0u, 0u, 0u, 0u);
-      if (live) raw = __ldg(reinterpret_cast<const uint4*>(x + at));
-      const T* v = reinterpret_cast<const T*>(&raw);
-#pragma unroll
-      for (int k = 0; k < NV; ++k) {
-        const bool col = live && strip * NV + k < in;      // (pad columns contribute nothing, whatever they hold)
-        xs[k] = col ? to_f32<T>(v[k]) : 0.f;
-        if (!col) best[k] = 0.f;
-      }
-    }
-    for (int c0 = 0; c0 < C; c0 += 4) {
-      float acc[4] = {0.f, 0.f, 0.f, 0.f};
-      uint4 w1[4], w2[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        w1[u] = make_uint4(0u, 0u, 0u, 0u);
-        w2[u] = make_uint4(0u, 0u, 0u, 0u);
-        if (c0 + u < C && live) {
-          w1[u] = __ldg(reinterpret_cast<const uint4*>(ws + (int64_t)(c0 + u) * pitch) + strip);
-          w2[u] = __ldg(reinterpret_cast<const uint4*>(wn + (int64_t)(c0 + u) * pitch) + strip);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const T* a1 = reinterpret_cast<const T*>(&w1[u]);
-        const T* a2 = reinterpret_cast<const T*>(&w2[u]);
-#pragma unroll
-        for (int k = 0; k < NV; ++k) {
-          acc[u] = fmaf(xs[k], to_f32<T>(a1[k]), acc[u]);
-          acc[u] = fmaf(best[k], to_f32<T>(a2[k]), acc[u]);
-        }
-      }
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) acc[u] += __shfl_xor_sync(0xffffffffu, acc[u], o);
-        if (lane == 0 && c0 + u < C) part[warp][c0 + u] = acc[u];
-      }
-    }
-    __syncthreads();
-    // ---- warp 0: the row's logits, cross entropy (log-softmax + NLL), dlogits = (softmax - onehot) * scale in the arithmetic type
-    if (warp == 0) {
-      float lg[2];
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const int c = lane + 32 * h;
-        float v = -INFINITY;
-        if (c < C) {
-          v = 0.f;
-          for (int w = 0; w < n_warps; ++w) v += part[w][c];
-          v += __ldg(bs + c) + __ldg(bn + c);
-          logits[(int64_t)r * ldl + c] = v;
-        }
-        lg[h] = v;
-      }
-      float mx = fmaxf(lg[0], lg[1]);
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-      float se = (lane < C ? expf(lg[0] - mx) : 0.f) + (lane + 32 < C ? expf(lg[1] - mx) : 0.f);
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) se += __shfl_xor_sync(0xffffffffu, se, o);
-      const float lse = mx + logf(se);
-      const int y = labels[nodes[r]];
-      const float l0 = __shfl_sync(0xffffffffu, lg[0], y & 31), l1 = __shfl_sync(0xffffffffu, lg[1], y & 31);
-      if (per_loss && lane == 0) per_loss[r] = lse - ((y >> 5) ? l1 : l0);
-      if (want_grad) {
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int c = lane + 32 * h;
-          float g = 0.f;
-          if (c < C) g = (expf(lg[h] - lse) - (c == y ? 1.f : 0.f)) * scale;
-          const T gt = from_f32<T>(g);
-          dls[c] = to_f32<T>(gt);                    // as stored (rounded): what the gradient GEMMs consume
-          if (c < ldd) dlogits[(int64_t)r * ldd + c] = gt;
-        }
-      }
-    }
-    // ---- dneigh = dlogits . W_neigh, masked by relu'(hp) at the argmax (neigh > 0), classes in ascending order
-    if (want_grad) {
-      __syncthreads();
-      if (live) {
-        float dacc[NV];
-#pragma unroll
-        for (int k = 0; k < NV; ++k) dacc[k] = 0.f;
-#pragma unroll 4
-        for (int c = 0; c < C; ++c) {
-          const float dc = dls[c];
-          const uint4 raw = __ldg(reinterpret_cast<const uint4*>(wn + (int64_t)c * pitch) + strip);
-          const T* a2 = reinterpret_cast<const T*>(&raw);
-#pragma unroll
-          for (int k = 0; k < NV; ++k) dacc[k] = fmaf(dc, to_f32<T>(a2[k]), dacc[k]);
-        }
-        T o[NV];
-#pragma unroll
-        for (int k = 0; k < NV; ++k) o[k] = from_f32<T>(best[k] > 0.f ? dacc[k] : 0.f);
-        *reinterpret_cast<uint4*>(dng + at) = *reinterpret_cast<const uint4*>(o);
-      }
-    }
-  }
-  // ---- the last CTA to get here sums the per-vertex losses, in a fixed order
-  if (loss_sum) {
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      __threadfence();
-      is_last = atomicAdd(done_counter, 1u) == gridDim.x - 1;
-    }
-    __syncthreads();
-    if (is_last) {
-      __threadfence();
-      float a = 0.f;
-      for (int i = threadIdx.x; i < n; i += blockDim.x) a += __ldcg(per_loss + i);
-      for (int o = 16; o > 0; o >>= 1) a += __shfl_down_sync(0xffffffffu, a, o);
-      if (lane == 0) red[warp] = a;
-      __syncthreads();
-      if (threadIdx.x < 32) {
-        a = threadIdx.x < n_warps ? red[threadIdx.x] : 0.f;
-        for (int o = 16; o > 0; o >>= 1) a += __shfl_down_sync(0xffffffffu, a, o);
-        if (threadIdx.x == 0) { *loss_sum = a; *done_counter = 0; }
-      }
-    }
-  }
-}
-
 // single CTA, fixed order: deterministic sum of the per-vertex losses
 __global__ void __launch_bounds__(1024) k_sum_f32(const float* __restrict__ x, const int32_t* __restrict__ n_dev, int n_max, float* __restrict__ out) {
   __shared__ float s[32];
@@ -731,26 +522,6 @@ int xent(int mode, const float* logits, int ldl, int C, const int32_t* labels, c
          int rows_buf, float scale, float* per_loss, void* dlogits, int ldd, int want_grad, cudaStream_t s) {
   const int grid = grid_for((int64_t)(rows_buf > n_max ? rows_buf : n_max) * 32, kBlock);
   L2T(k_xent, grid, s, ARGS(logits, ldl, C, labels, nodes, n_dev, n_max, rows_buf, scale, per_loss, (T*)dlogits, ldd, want_grad));
-  return OGL_OK;
-}
-bool head_fused_supported(int mode, int pitch, int n_classes) {
-  return n_classes <= kHeadMaxC && pitch / mode_vec(mode) <= kHeadMaxStrips;
-}
-int head_fused(int mode, const void* hp, const void* x, int pitch, int in, const int32_t* edge_lid, int fanout, const void* ws, const void* wn,
-               const float* bs, const float* bn, int C, const int32_t* labels, const int32_t* nodes, const int32_t* n_dev, int n_max,
-               int rows_buf, float scale, int want_grad, void* neigh, uint8_t* arg, float* logits, int ldl, float* per_loss, void* dlogits,
-               int ldd, void* dng, float* loss_sum, uint32_t* done_counter, cudaStream_t s) {
-  OGL_ARG(head_fused_supported(mode, pitch, C), "head_fused: %d classes / pitch %d not supported", C, pitch);
-  const int rows = rows_buf > n_max ? rows_buf : n_max;               // one CTA per seed row (+ the zero-filled pad rows)
-  const int block = round_up(pitch / mode_vec(mode), 32);              // one thread per 16-byte column strip
-#define HEAD_ARGS                                                                                                                       \
-  (const T*)hp, (const T*)x, pitch, in, edge_lid, fanout, (const T*)ws, (const T*)wn, bs, bn, C, labels, nodes, n_dev, n_max, rows_buf,    \
-      scale, want_grad, (T*)neigh, arg, logits, ldl, per_loss, (T*)dlogits, ldd, (T*)dng, loss_sum, done_counter
-  if (mode == OGL_BF16) { using T = __nv_bfloat16; OGL_LAUNCH((k_head_fused<T>), rows, block, 0, s, HEAD_ARGS); }
-  else if (mode == OGL_FP16) { using T = __half; OGL_LAUNCH((k_head_fused<T>), rows, block, 0, s, HEAD_ARGS); }
-  else if (mode == OGL_TF32) { using T = tf32_t; OGL_LAUNCH((k_head_fused<T>), rows, block, 0, s, HEAD_ARGS); }
-  else { using T = float; OGL_LAUNCH((k_head_fused<T>), rows, block, 0, s, HEAD_ARGS); }
-#undef HEAD_ARGS
   return OGL_OK;
 }
 int sum_f32(const float* x, const int32_t* n_dev, int n_max, float* out, cudaStream_t s) {

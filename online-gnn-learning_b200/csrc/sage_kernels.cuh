@@ -39,13 +39,6 @@ int colsum(int mode, const void* x, int pitch, int cols, const int32_t* n_dev, i
            float alpha = 1.f);
 int xent(int mode, const float* logits, int ldl, int C, const int32_t* labels, const int32_t* nodes, const int32_t* n_dev, int n_max,
          int rows_buf, float scale, float* per_loss, void* dlogits, int ldd, int want_grad, cudaStream_t s);
-// fused head of a train step on the seed rows (last layer): segment max + output GEMM + cross entropy + loss sum + dneigh GEMM in one
-// launch, one warp per row (see k_head_fused); done_counter: a zeroed device word the kernel leaves zeroed
-bool head_fused_supported(int mode, int pitch, int n_classes);
-int head_fused(int mode, const void* hp, const void* x, int pitch, int in, const int32_t* edge_lid, int fanout, const void* ws, const void* wn,
-               const float* bs, const float* bn, int C, const int32_t* labels, const int32_t* nodes, const int32_t* n_dev, int n_max,
-               int rows_buf, float scale, int want_grad, void* neigh, uint8_t* arg, float* logits, int ldl, float* per_loss, void* dlogits,
-               int ldd, void* dng, float* loss_sum, uint32_t* done_counter, cudaStream_t s);
 int sum_f32(const float* x, const int32_t* n_dev, int n_max, float* out, cudaStream_t s);
 int adam(float* p, const float* g, float* m, float* v, int64_t n, float lr, float b1, float b2, float eps, uint32_t* t_dev, cudaStream_t s);
 // Adam over the parameter range [lo, hi) (the step counter *t_dev is read, not advanced)

@@ -6,8 +6,6 @@ them over PCIe and runs DGL/cuBLAS kernels (:77-107), every minibatch here is ON
 feature gather, the GraphSAGE-pool forward/backward, CE loss, Adam -- stays on the GPU with no host
 synchronisation.  Per-vertex losses for PBR come back only in faithful mode.
 """
-import os
-
 import numpy as np
 import torch
 
@@ -126,10 +124,6 @@ class PytorchSupervisedGraphSage(SupervisedGraphSage):
         plan = self._train_plan(graph)
         if parallel.world() > 1:
             return self._dp_steps(graph, plan, seeds, batch, per_vertex_out)
-        if os.environ.get("OGL_NO_MULTISTEP"):                     # A/B switch: one C call per minibatch
-            for i in range(0, n, batch):
-                self._fused_step(graph, seeds[i:i + batch], per_vertex_out=None if per_vertex_out is None else per_vertex_out[i:i + batch])
-            return
         if n_full:
             plan.train_steps(graph.native, graph.features, seeds[:n_full * batch], batch, loss_scale=1.0 / batch, do_step=True,
                              per_vertex_out=None if per_vertex_out is None else per_vertex_out[:n_full * batch])

@@ -88,9 +88,10 @@ class Pipeline:
     feature store only), `finish` = forward .. backward (.. Adam).  `begin` of step t+1 is a prefetch (Plan.prefetch: the
     plan's own stream and second buffer set), so it overlaps forward / backward of step t -- the job NodeDataLoader's worker
     processes do in the reference (pytorch/model.py:128-131).  With more than one rank the gradient exchange is bucketed:
-    the all-reduce of everything but layer 0's fc_pool.weight overlaps the last weight-gradient GEMM, the small second
-    bucket + Adam run on a communication stream; forward(t+1) waits for Adam(t).  Same arithmetic as the unpipelined loop
-    (no stale gradients, same Philox step per minibatch)."""
+    the exchange of everything but layer 0's fc_pool.weight overlaps the last weight-gradient GEMM.  With a peer group both
+    exchanges and Adam are nodes of the step's own launch sequence (Plan.step_finish_dp); with NCCL the all-reduces, the small
+    second bucket and Adam run on a communication stream and forward(t+1) waits for Adam(t).  Same arithmetic as the
+    unpipelined loop (no stale gradients, same Philox step per minibatch)."""
 
     def __init__(self, plan, graph, features, flat_grad, global_batch, peer=None, force_split=False):
         """peer: a native.Peer from make_peer_exchange -> the gradient exchange + Adam is ONE kernel per bucket over NVLink peer
@@ -100,17 +101,10 @@ class Pipeline:
         if peer is not None:
             assert flat_grad.data_ptr() == peer.grads.data_ptr(), "the plan must be bound to the peer group's gradient buffer"
         self.scale = 1.0 / float(global_batch)
-        # force_split (experiments): run the data-parallel launch structure (head | bucket exchange | tail | bucket exchange) on ONE
-        # rank with a one-rank peer group -- what the structure itself costs, without NVLink traffic or waiting for other ranks
+        # force_split (experiments; needs `peer`): run the one-graph data-parallel finish (Plan.step_finish_dp) on ONE rank with a
+        # one-rank peer group -- what its launch structure costs, without NVLink traffic or waiting for other ranks
         self.w = max(world(), 2) if force_split else world()
         self.comm = torch.cuda.Stream() if self.w > 1 else None
-        import os
-        self.split_launch = bool(int(os.environ.get("OGL_DP_SPLIT_LAUNCH", "0")))      # the older form: head | exchange | tail | exchange
-        pieces = getattr(plan, "tail_pieces", [None])
-        # measured on 2 and 8 B200 (tf32, Reddit shape): exchanging the last gradient in 256-row pieces is SLOWER (1.135 vs 1.014 ms
-        # at 8 GPUs: three GEMM prologues, three reduces and three box-wide barriers cost more than the exposed exchange they hide)
-        self.tail_pieces = len(pieces) if int(os.environ.get("OGL_DP_TAIL_PIECES", "0")) else 1
-        self.ev_piece = [torch.cuda.Event() for _ in range(len(pieces))] if self.w > 1 else []
         self.ev_bwd = torch.cuda.Event()
         self.ev_head = torch.cuda.Event()
         self.ev_adam = torch.cuda.Event()
@@ -140,7 +134,7 @@ class Pipeline:
         if self.w == 1:
             self.plan.step_finish(self.features, self.scale, do_step=True, per_vertex_out=per_vertex_out, loss_sum_out=loss_sum_out)
             return
-        if self.peer is not None and not self.split_launch and hasattr(self.plan, "step_finish_dp"):
+        if self.peer is not None:
             # one launch sequence (one CUDA graph) per step, the exchanges inside it (ogl_plan_step_finish_dp)
             self.plan.step_finish_dp(self.peer, self.features, self.scale, per_vertex_out=per_vertex_out, loss_sum_out=loss_sum_out)
             return
@@ -148,39 +142,18 @@ class Pipeline:
             main.wait_event(self.ev_adam)                # weights (and the gradient buffer) of the previous step are settled
         # two gradient buckets: everything except layer 0's fc_pool.weight is final before the last weight-gradient GEMM
         # runs, so its all-reduce overlaps that GEMM; the small second bucket + Adam overlap the next step's start
-        n0, n = self.plan.tail_params, self.plan.n_params
-        if self.peer is not None:
-            self.peer.wait_readers()                     # every peer has read this rank's gradients of the previous step
+        n0 = self.plan.tail_params
         self.plan.step_finish_head(self.features, self.scale, per_vertex_out=per_vertex_out, loss_sum_out=loss_sum_out)
         self.ev_head.record(main)
         with torch.cuda.stream(self.comm):
             self.comm.wait_event(self.ev_head)
-            if self.peer is not None:
-                self.plan.peer_adam(self.peer, n0, n, last=False)     # P2P sum + Adam of bucket 1, beside the tail GEMM
-            else:
-                allreduce_grads(self.flat_grad[n0:])
-        if self.peer is not None and self.tail_pieces > 1:
-            # the last weight-gradient GEMM in pieces of 256 gradient rows: piece i is exchanged (and its Adam done) while piece
-            # i + 1 is computed, so only the last, smallest piece's exchange is exposed before the next step's forward pass
-            pieces = self.plan.tail_pieces
-            for i, (lo, hi) in enumerate(pieces):
-                self.plan.step_finish_tail(self.features, part=i, n_parts=len(pieces))
-                self.ev_piece[i].record(main)
-                with torch.cuda.stream(self.comm):
-                    self.comm.wait_event(self.ev_piece[i])
-                    self.plan.peer_adam(self.peer, lo, hi, last=(i + 1 == len(pieces)))
-            self.ev_adam.record(self.comm)
-            self._adam_pending = True
-            return
+            allreduce_grads(self.flat_grad[n0:])
         self.plan.step_finish_tail(self.features)
         self.ev_bwd.record(main)
         with torch.cuda.stream(self.comm):
             self.comm.wait_event(self.ev_bwd)
-            if self.peer is not None:
-                self.plan.peer_adam(self.peer, 0, n0, last=True)
-            else:
-                allreduce_grads(self.flat_grad[:n0])
-                self.plan.adam_step()
+            allreduce_grads(self.flat_grad[:n0])
+            self.plan.adam_step()
             self.ev_adam.record(self.comm)
         self._adam_pending = True
 

@@ -10,12 +10,13 @@ pytestmark = pytest.mark.gpu
 from test_gpu_sage import Case  # noqa: E402
 
 
-@pytest.mark.parametrize("two_shot", [0, 1])
+@pytest.mark.parametrize("offset", [0, 1])
 @pytest.mark.parametrize("mode", ["bf16", "fp32"])
-def test_peer_adam_two_ranks_equals_summed_gradient_adam(mode, two_shot, monkeypatch):
-    """two_shot = 0: every rank loads every peer's gradients; 1: reduce-scatter + all-gather inside the kernel (default for >= 4 ranks)"""
+def test_peer_adam_two_ranks_equals_summed_gradient_adam(mode, offset):
+    """every rank loads every peer's gradients and sums them in rank order: the sum equals the summed gradient bit for bit, and the
+    weights equal Adam on it.  offset = 0: the data-parallel pipeline's two buckets; 1: the bucket boundary moved one float off the
+    16-byte grid, so that both buckets also run the kernel's scalar head / tail loops"""
     from ogl_b200 import native
-    monkeypatch.setenv("OGL_PEER_TWO_SHOT", str(two_shot))
     W, B = 2, 64
     kw = dict(dims=(64, 32, 5), fanouts=(6, 4), n_seeds=B, mode=mode, gemm_impl=0 if mode == "bf16" else 1)
     ranks = [Case(**kw) for _ in range(W)]
@@ -27,7 +28,7 @@ def test_peer_adam_two_ranks_equals_summed_gradient_adam(mode, two_shot, monkeyp
         c.plan.bind_params(c.flat, p.grads)
     rng = np.random.default_rng(9)
     streams = [torch.cuda.Stream() for _ in range(W)]
-    n0 = ref.plan.tail_params
+    n0 = ref.plan.tail_params + offset
     reduced = [torch.zeros(n, device="cuda") for _ in range(W)]
     for step in range(3):
         for r, c in enumerate(ranks):
@@ -40,7 +41,7 @@ def test_peer_adam_two_ranks_equals_summed_gradient_adam(mode, two_shot, monkeyp
             want += peers[r].grads
         ref.grad.copy_(want)
         ref.plan.adam_step()
-        # two buckets, like the data-parallel pipeline; every rank on its own stream (the kernels wait for each other)
+        # two buckets; every rank on its own stream (the kernels wait for each other)
         for lo, hi, last in ((n0, n, False), (0, n0, True)):
             for r, c in enumerate(ranks):
                 with torch.cuda.stream(streams[r]):
