@@ -240,6 +240,25 @@ int ogl_plan_graph_stats(ogl_plan* p, int64_t out[2]);
 /* eval: sample + forward + per-vertex CE loss (PBR recompute_priorities, pytorch/model.py:210-254) */
 int ogl_plan_eval_step(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds, int n_seeds,
                        int seeds_on_host, float* logits_dev, float* per_vertex_loss_dev, void* stream);
+/* ---- full-neighbourhood inference (DGL's model.inference(g, x)): every in-edge, no sampling -------------------------------
+ * ogl_plan_infer_full: logits [n, classes] fp32 of the plan's model for the vertices seeds_dev[0..n) (device int64; seeds_dev == NULL:
+ *   n = the number of vertices of g, all of them, in id order).  Layer by layer over every vertex: relu(fc_pool) over all rows, the
+ *   segment max over the whole in-edge row of each vertex, fc_self + fc_neigh; with seeds the last layer runs on the seed rows only.
+ *   Evaluation semantics (no feat_drop).  Max-pooling is exact, so the result is bit-reproducible and independent of the order in which
+ *   the edges were inserted.  Ordered on `stream`; changes no plan state (Philox / Adam counters, minibatch buffers, pending
+ *   prefetches, captured step graphs).  The plan keeps the activations of every layer for all vertices ([V, pitch] tables, allocated
+ *   on first use, grown with the graph, freed with the plan): a graph whose activations do not fit in device memory fails with
+ *   OGL_ERR_CAPACITY.  A seed id outside [0, n_vertices) is replaced by vertex 0 and raises bit 0 of ogl_plan_error_flags.
+ *   Destination shards (ogl_graph_set_source_bound) are rejected.
+ * ogl_graph_segment_max: the segment max on its own: out[r, :cols] = max over the in-edges (u -> v_r) of x[u, :cols], 0 for a vertex
+ *   without in-edges, v_r = rows_dev[r] (rows_dev == NULL: v_r = r and n_rows must be the vertex count).  x [*, ld] holds a row for
+ *   every vertex of g in the storage type of `mode` (OGL_F32 / OGL_TF32: fp32, OGL_BF16: bf16, OGL_FP16: fp16); x and out 16-byte
+ *   aligned, ld and ldo multiples of 16 bytes; columns are written in 16-byte strips up to round_up(cols, 16 bytes) <= ldo.  A listed
+ *   id outside [0, n_vertices) gives a zero row.  Synchronises `stream` (it frees its scratch before returning). */
+int ogl_plan_infer_full(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds_dev, int64_t n, float* logits_dev,
+                        void* stream);
+int ogl_graph_segment_max(ogl_graph* g, int mode, const void* x_dev, int ld, int cols, const int64_t* rows_dev, int64_t n_rows,
+                          void* out_dev, int ldo, void* stream);
 
 /* stage profiling for bench.py's roofline: CUDA events recorded around every stage of the plan's calls on the
  * caller's stream (off by default).  enable=1 (re)starts a collection.  _read synchronises the device and returns,

@@ -141,6 +141,20 @@ class Graph:
             check(lib.ogl_graph_gather_rows(self._h, _ptr(v), v.numel(), _ptr(offsets), _ptr(src), _stream()))
         return offsets, src
 
+    def segment_max(self, x, rows=None, cols=None):
+        """out[r] = max over the in-edges (u -> v_r) of x[u, :cols] (0 for a vertex without in-edges), v_r = rows[r] or r for every
+        vertex; x: CUDA fp32 / bf16 / fp16 [*, ld] with a row per vertex and unit column stride.  -> [n_rows, cols] of x's dtype"""
+        mode = {torch.float32: OGL_F32, torch.bfloat16: OGL_BF16, torch.float16: OGL_FP16}[x.dtype]
+        assert x.is_cuda and x.dim() == 2 and x.stride(1) == 1
+        cols = x.shape[1] if cols is None else int(cols)
+        nv = 4 if x.dtype == torch.float32 else 8
+        r = None if rows is None else _dev(rows, torch.int64)
+        n = self.num_vertices if r is None else r.numel()
+        out = torch.empty(n, (cols + nv - 1) // nv * nv, dtype=x.dtype, device="cuda")
+        check(lib.ogl_graph_segment_max(self._h, mode, C.c_void_p(x.data_ptr()), x.stride(0), cols, _ptr(r), n, _ptr(out), out.shape[1],
+                                        _stream()))
+        return out[:, :cols]
+
     def stats(self):
         a = (C.c_int64 * 4)()
         check(lib.ogl_graph_stats(self._h, C.byref(a)))
@@ -338,6 +352,19 @@ class Plan:
                                      _ptr(logits_out), _ptr(per_vertex_out), _stream()))
         self.n_seeds = n
         self._stamp += 1
+
+    def infer_full(self, graph, features, seeds=None, logits_out=None):
+        """logits [n, C] fp32 of every listed vertex (seeds: int64 ids; None: every vertex of `graph`, in id order) from its WHOLE
+        in-neighbourhood, layer by layer over all vertices, no sampling; changes no plan state.  Out-of-range ids raise bit 0 of
+        error_flags()."""
+        s = None if seeds is None else _dev(seeds, torch.int64)
+        n = graph.num_vertices if s is None else s.numel()
+        out = logits_out
+        if out is None:
+            out = torch.empty(n, self.dims[-1], dtype=torch.float32, device="cuda")
+        assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and tuple(out.shape) == (n, self.dims[-1])
+        check(lib.ogl_plan_infer_full(self._h, graph._h, features._h, _ptr(s), n, _ptr(out), _stream()))
+        return out
 
     def reset_optimizer(self, philox_step=0):
         """zero Adam's moments / step counter and set the Philox step (a fresh optimiser; replays of a run from its start)"""

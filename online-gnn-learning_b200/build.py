@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "csrc", "_obj")
 LIB = os.path.join(HERE, "libogl_b200.so")
-SOURCES = ["common.cu", "graph.cu", "sample.cu", "replay.cu", "gemm_simt.cu", "gemm_tc.cu", "sage_kernels.cu", "peer.cu", "infer.cu", "plan.cu"]
+SOURCES = ["common.cu", "graph.cu", "sample.cu", "replay.cu", "gemm_simt.cu", "gemm_tc.cu", "sage_kernels.cu", "peer.cu", "infer.cu", "full_infer.cu", "plan.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
          "-Xcompiler", "-fvisibility=hidden", "-Xptxas", "-v"]

@@ -1,0 +1,35 @@
+// Segment max over the in-edge rows of the streaming CSR (full-neighbourhood inference, see full_infer.cu).
+#pragma once
+#include "graph.cuh"
+
+namespace ogl {
+
+// a row with more in-edges than this is a hub: its edges are cut into chunks of this many, one warp per chunk
+constexpr int kSegmaxChunk = 2048;
+
+struct SegmaxHub {
+  int64_t r;       // output row
+  int32_t v;       // vertex
+  int32_t base;    // first chunk slot
+  int32_t n;       // chunk slots (0: the row was reduced in place by the row pass)
+  int32_t pad;
+};
+
+// device scratch of csr_segmax, sized from the graph's edge count and the row width in bytes
+struct SegmaxWs {
+  unsigned long long* ctl = nullptr;   // [0] row cursor, [1] hubs, [2] chunk slots, [3] chunk cursor
+  SegmaxHub* hubs = nullptr;
+  int32_t* chunk_hub = nullptr;
+  void* partial = nullptr;             // [chunk_cap, row bytes]
+  int64_t hub_cap = 0, chunk_cap = 0, row_bytes = 0;
+};
+int segmax_ws_reserve(SegmaxWs* ws, int64_t n_edges, int64_t row_bytes);
+void segmax_ws_free(SegmaxWs* ws);
+
+// out[r, :cols] = max over the in-edges (u -> v_r) of x[u, :cols], 0 for a row without in-edges; v_r = rows32[r] | rows64[r] | r
+// (at most one list).  A listed id outside [0, n_vertices) gives a zero row.  Columns are processed in 16-byte strips, so out
+// columns up to round_up(cols, 16 / element bytes) are written.  Exact: the result does not depend on edge order or on the split.
+int csr_segmax(int mode, const GraphView& gv, int64_t n_edges, const void* x, int ld, int cols, const int32_t* rows32,
+               const int64_t* rows64, int64_t n_rows, void* out, int ldo, SegmaxWs* ws, cudaStream_t s);
+
+}  // namespace ogl

@@ -936,6 +936,8 @@ extern "C" int ogl_graph_set_active_prefix(ogl_graph* g, int64_t n_active, void*
 
 namespace ogl {
 uint64_t graph_generation(const ogl_graph* g) { return g->generation; }
+int64_t graph_num_edges(const ogl_graph* g) { return g->n_edges; }
+int64_t graph_source_bound(const ogl_graph* g) { return g->src_bound; }
 GraphView graph_view(const ogl_graph* g) {
   GraphView v;
   v.row_start = g->row_start; v.deg = g->deg; v.adj = g->adj; v.n_vertices = g->n_vertices;

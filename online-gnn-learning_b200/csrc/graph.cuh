@@ -33,4 +33,8 @@ namespace ogl {
 GraphView graph_view(const ogl_graph* g);
 // changes whenever a device pointer of the view changes (pool rebuild): invalidates captured CUDA graphs
 uint64_t graph_generation(const ogl_graph* g);
+// directed edges stored (the sum of the row degrees)
+int64_t graph_num_edges(const ogl_graph* g);
+// 0, or the source id bound of a destination shard (ogl_graph_set_source_bound)
+int64_t graph_source_bound(const ogl_graph* g);
 }

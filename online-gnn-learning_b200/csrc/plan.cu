@@ -9,6 +9,7 @@
 #include "gemm.cuh"
 #include "sage_kernels.cuh"
 #include "peer.cuh"
+#include "full_infer.cuh"
 #include <cmath>
 #include <vector>
 #include <string>
@@ -204,6 +205,15 @@ struct ogl_plan {
   size_t prof_used = 0;
   int32_t* prof_counts_host = nullptr;   // pinned [kProfSteps][8]
   int prof_steps = 0;
+  // full-neighbourhood inference (ogl_plan_infer_full): its own activations over every vertex, allocated on first use and grown
+  // geometrically with the graph; nothing of the train / eval state above is read or written by it except the weights
+  struct FullWs {
+    int64_t rows = 0;                    // row capacity (a multiple of 128)
+    void *hp = nullptr, *neigh = nullptr, *hs = nullptr, *h[2] = {nullptr, nullptr};
+    float* logits = nullptr;
+    int32_t* seeds = nullptr;
+    SegmaxWs sm;
+  } full;
 };
 constexpr int kProfSteps = 4096;
 
@@ -426,6 +436,8 @@ extern "C" int ogl_plan_destroy(ogl_plan* p) {
   for (auto& sg : p->step_graphs) cudaGraphExecDestroy(sg.exec);
   if (p->cap_stream) cudaStreamDestroy(p->cap_stream);
   if (p->prof_counts_host) cudaFreeHost(p->prof_counts_host);
+  for (void* q : {p->full.hp, p->full.neigh, p->full.hs, p->full.h[0], p->full.h[1], (void*)p->full.logits, (void*)p->full.seeds}) cudaFree(q);
+  segmax_ws_free(&p->full.sm);
   delete p;
   return OGL_OK;
 }
@@ -1157,6 +1169,99 @@ extern "C" int ogl_plan_eval_step(ogl_plan* p, ogl_graph* g, ogl_features* f, co
   if (per_vertex_loss_dev) OGL_TRY(plan_loss(p, f, 1.f, 0, per_vertex_loss_dev, nullptr, s));
   OGL_TRY(bump(p->ctl, nullptr, s));
   return OGL_OK;
+}
+
+// ------------------------------------------------------------------ full-neighbourhood inference ----
+// DGL's model.inference(g, x): layer by layer over EVERY vertex and EVERY in-edge, no sampling.  Per layer: hp = relu(h Wp^T + bp) over
+// all rows (layer 0 reads the feature table itself), the CSR segment max, then [h | neigh] [Ws | Wn]^T + b (ReLU except on the
+// last layer).  With seeds, the last layer's segment max and output GEMM run on the seed rows only.  Reads the weights and shadows;
+// leaves the Philox / Adam counters, the minibatch buffers, pending prefetches and captured step graphs alone.
+static int full_ws_reserve(ogl_plan* p, int64_t rows_needed) {
+  ogl_plan::FullWs& w = p->full;
+  if (rows_needed <= w.rows) return OGL_OK;
+  const int64_t rows = round_up((int)std::max<int64_t>(rows_needed, w.rows + w.rows / 2), 128);
+  int max_pin = 0, max_hid = 8;
+  for (int l = 0; l < p->L; ++l) {
+    max_pin = std::max(max_pin, p->layer[l].pin);
+    if (l < p->L - 1) max_hid = std::max(max_hid, p->layer[l].pout);
+  }
+  for (void* q : {w.hp, w.neigh, w.hs, w.h[0], w.h[1], (void*)w.logits, (void*)w.seeds}) cudaFree(q);
+  w.hp = w.neigh = w.hs = w.h[0] = w.h[1] = nullptr;
+  w.logits = nullptr;
+  w.seeds = nullptr;
+  w.rows = 0;
+  const size_t r = (size_t)rows;
+  const size_t bytes[7] = {p->es * r * max_pin, p->es * r * max_pin, p->es * r * max_pin, p->es * r * max_hid, p->es * r * max_hid,
+                           sizeof(float) * r * p->layer[p->L - 1].pout, sizeof(int32_t) * r};
+  void** ptrs[7] = {&w.hp, &w.neigh, &w.hs, &w.h[0], &w.h[1], (void**)&w.logits, (void**)&w.seeds};
+  for (int i = 0; i < 7; ++i)
+    if (dmalloc0(ptrs[i], bytes[i]) != OGL_OK) {
+      cudaGetLastError();
+      for (int j = 0; j < 7; ++j) { cudaFree(*ptrs[j]); *ptrs[j] = nullptr; }
+      set_error("ogl_plan_infer_full: cannot allocate the activations of %lld rows (full-graph inference keeps every layer's [V, pitch] "
+                "tables in device memory; graphs that do not fit are not supported)", (long long)rows);
+      return OGL_ERR_CAPACITY;
+    }
+  w.rows = rows;
+  return OGL_OK;
+}
+
+extern "C" int ogl_plan_infer_full(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds_dev, int64_t n, float* logits_dev,
+                                   void* stream) {
+  OGL_ARG(p && g && f, "ogl_plan_infer_full: null");
+  OGL_ARG(p->params, "ogl_plan_infer_full: parameters not bound");
+  OGL_ARG(f->mode == p->cfg.mode && f->F == p->cfg.dims[0], "ogl_plan_infer_full: feature store does not match the plan (mode/F)");
+  OGL_ARG(graph_source_bound(g) == 0, "ogl_plan_infer_full: the graph is a destination shard (ogl_graph_set_source_bound); full inference "
+          "needs every source row");
+  cudaStream_t s = (cudaStream_t)stream;
+  const GraphView gv = graph_view(g);
+  const int64_t V = gv.n_vertices;
+  OGL_ARG(V <= f->v_cap, "ogl_plan_infer_full: graph has more vertices than the feature store");
+  OGL_ARG(V < (1LL << 31), "ogl_plan_infer_full: too many vertices");
+  if (!seeds_dev) n = V;
+  OGL_ARG(n >= 0 && n < (1LL << 31), "ogl_plan_infer_full: n out of range");
+  if (n == 0) return OGL_OK;
+  OGL_ARG(logits_dev, "ogl_plan_infer_full: null logits");
+  OGL_ARG(V > 0, "ogl_plan_infer_full: the graph has no vertices");
+  OGL_TRY(full_ws_reserve(p, std::max(V, n)));
+  ogl_plan::FullWs& w = p->full;
+  const int L = p->L;
+  const int64_t E = graph_num_edges(g);
+  // out-of-range seed ids are replaced by vertex 0 and raise error bit 0, as in ogl_plan_eval_step
+  if (seeds_dev) OGL_TRY(cast_nodes(seeds_dev, w.seeds, n, V, p->ctl + 2, s));
+  const void* h = f->table;
+  int ldh = f->pitch;
+  for (int l = 0; l < L; ++l) {
+    LayerBuf& lb = p->layer[l];
+    const bool last = l == L - 1, on_seeds = last && seeds_dev;
+    const int m = (int)(on_seeds ? n : V);
+    GemmNT g1;
+    g1.a[0] = h; g1.lda[0] = ldh; g1.b[0] = lb.wp; g1.ldb[0] = lb.pin; g1.k[0] = lb.in; g1.n_seg = 1;
+    g1.bias = p->params + lb.o_bp; g1.relu = 1;
+    g1.c = w.hp; g1.ldc = lb.pin; g1.m_max = (int)V; g1.n = lb.in;
+    g1.in_bf16 = p->bf16; g1.out_bf16 = p->bf16; g1.f16 = p->fp16; g1.tf32 = p->tf32; g1.out_tf32 = p->tf32;
+    STAGE(nm("full.l%d.pool_gemm", l).c_str(), gemm_nt(p, g1, s));
+    STAGE(nm("full.l%d.segmax", l).c_str(), csr_segmax(p->mode, gv, E, w.hp, lb.pin, lb.in, on_seeds ? w.seeds : nullptr, nullptr, m,
+                                                       w.neigh, lb.pin, &w.sm, s));
+    const int mp = round_up(m, 128);
+    if (mp > m) OGL_CUDA(cudaMemsetAsync((char*)w.neigh + p->es * (size_t)m * lb.pin, 0, p->es * (size_t)(mp - m) * lb.pin, s));
+    const void* self = h;
+    if (on_seeds) {
+      OGL_TRY(gather_rows(p->mode, h, ldh, w.seeds, nullptr, m, w.hs, s));
+      self = w.hs;
+    }
+    GemmNT g2;
+    g2.a[0] = self; g2.lda[0] = ldh; g2.b[0] = lb.ws; g2.ldb[0] = lb.pin; g2.k[0] = lb.in;
+    g2.a[1] = w.neigh; g2.lda[1] = lb.pin; g2.b[1] = lb.wn; g2.ldb[1] = lb.pin; g2.k[1] = lb.in; g2.n_seg = 2;
+    g2.bias = p->params + lb.o_bs; g2.bias2 = p->params + lb.o_bn; g2.relu = !last;
+    void* out = last ? (void*)w.logits : w.h[l & 1];
+    g2.c = out; g2.ldc = lb.pout; g2.m_max = m; g2.n = lb.out;
+    g2.in_bf16 = p->bf16; g2.out_bf16 = last ? 0 : p->bf16; g2.f16 = p->fp16; g2.tf32 = p->tf32; g2.out_tf32 = last ? 0 : p->tf32;
+    STAGE(nm("full.l%d.out_gemm", l).c_str(), gemm_nt(p, g2, s));
+    h = out;
+    ldh = lb.pout;
+  }
+  return unpad_copy(w.logits, p->layer[L - 1].pout, (int)n, nullptr, p->cfg.dims[L], logits_dev, s);
 }
 
 // ------------------------------------------------------------------ stage profiling -----------------

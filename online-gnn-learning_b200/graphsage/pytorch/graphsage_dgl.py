@@ -154,6 +154,19 @@ class GraphSAGE(nn.Module):
             plan._version = self._version
         return plan
 
+    def inference(self, graph, vertices=None):
+        """DGL's `model.inference(g, x)`: fp32 logits [n, C] on the device for `vertices` (int64 ids; None: every vertex of `graph`, a
+        DeviceGraph) from their WHOLE in-neighbourhoods -- layer by layer over every vertex and every in-edge, no sampling, no
+        feat_drop.  Exact max-pooling makes the result bit-reproducible and independent of edge-insertion order.  Runs on a plan of
+        this model kept for `graph` (one full-inference workspace per model and graph); no training or sampled-evaluation state
+        changes.  Ids outside the graph raise bit 0 of that plan's error_flags() (see inference_plan)."""
+        plan = self.inference_plan(graph)
+        return plan.infer_full(graph.native, graph.features, seeds=vertices)
+
+    def inference_plan(self, graph):
+        """the plan `inference` runs on for `graph` (fan-out 1, one seed: only its weights and full-inference workspace are used)"""
+        return self.plan_for(graph, [1] * len(self.layers), 1)
+
     def mark_updated(self, plan):
         """`plan` just ran its fused Adam step: its own shadows are fresh, the other plans' are stale"""
         self._version += 1

@@ -31,9 +31,14 @@ class _FusedAdam:
 
 class PytorchSupervisedGraphSage(SupervisedGraphSage):
     def __init__(self, graphsage_model, batch_per_timestep, batch_size, labels, samples, reduction="mean", n_workers=1,
-                 cuda=False, batch_full=512, fanouts=None):
+                 cuda=False, batch_full=512, fanouts=None, eval_neighbourhood="sampled"):
         if not cuda:
             raise RuntimeError("ogl_b200 trainers are the `--cuda` path; there is no CPU fallback")
+        if eval_neighbourhood not in ("sampled", "full"):
+            raise ValueError("eval_neighbourhood must be 'sampled' or 'full', got %r" % (eval_neighbourhood,))
+        # "full": evaluate / evaluate_next_snapshots score every vertex from its whole in-neighbourhood (GraphSAGE.inference), which makes
+        # the F1 columns independent of the sampler; "sampled" (the reference's behaviour): fan-out-sampled neighbourhoods
+        self.eval_neighbourhood = eval_neighbourhood
         super().__init__(graphsage_model, batch_per_timestep, batch_size, labels, samples, n_workers, cuda, batch_full)
         self.reduction = reduction
         n_layers = len(graphsage_model.layers)
@@ -72,8 +77,17 @@ class PytorchSupervisedGraphSage(SupervisedGraphSage):
 
     # ---- evaluation (reference :39-71) -------------------------------------------------------------
     def _eval_logits_device(self, graph, test_vertices):
-        """eval-mode forward over `test_vertices` in batch_full chunks; logits [n, C] stay on the device"""
+        """eval-mode forward over `test_vertices` in batch_full chunks (or, with eval_neighbourhood="full", over their whole
+        neighbourhoods); logits [n, C] stay on the device"""
         self.graphsage_model.eval()
+        if self.eval_neighbourhood == "full":
+            v = torch.as_tensor(np.asarray(test_vertices, dtype=np.int64)).cuda()
+            if v.numel() == 0:
+                return None
+            out = self.graphsage_model.inference(graph, v)
+            if self.graphsage_model.inference_plan(graph).error_flags() & 1:
+                raise IndexError("a vertex id outside the graph was evaluated (DGL's NodeDataLoader raises on such ids)")
+            return out
         seeds = self._host_seeds(test_vertices)
         n = seeds.numel()
         if n == 0:
@@ -203,9 +217,10 @@ class PytorchSupervisedGraphSage(SupervisedGraphSage):
 class RandomPytorchSupervisedGraphSage(PytorchSupervisedGraphSage):
     """RBR: rehearsal on uniformly drawn train vertices (reference :110-138)."""
 
-    def __init__(self, model, batch_per_timestep, batch_size, labels, samples, cuda=False, batch_full=512, n_workers=0, fanouts=None):
+    def __init__(self, model, batch_per_timestep, batch_size, labels, samples, cuda=False, batch_full=512, n_workers=0, fanouts=None,
+                 eval_neighbourhood="sampled"):
         super().__init__(model, batch_per_timestep, batch_size, labels, samples, n_workers=n_workers, cuda=cuda,
-                         batch_full=batch_full, fanouts=fanouts)
+                         batch_full=batch_full, fanouts=fanouts, eval_neighbourhood=eval_neighbourhood)
 
     def choose_vertices(self, graph_util):
         draws = [graph_util.draw_random_train_nodes(self.batch_size) for _ in range(self.batch_per_timestep)]
@@ -228,9 +243,10 @@ class PrioritizedPytorchSupervisedGraphSage(PytorchSupervisedGraphSage):
     """PBR: loss-prioritised rehearsal (reference :141-257)."""
 
     def __init__(self, model, batch_per_timestep, batch_size, labels, samples, priority_strategy, full_pass=2, cuda=False,
-                 batch_full=512, n_workers=0, fanouts=None):
+                 batch_full=512, n_workers=0, fanouts=None, eval_neighbourhood="sampled"):
+        # (recompute_priorities stays on sampled neighbourhoods whatever eval_neighbourhood says)
         super().__init__(model, batch_per_timestep, batch_size, labels, samples, reduction="none", n_workers=n_workers,
-                         cuda=cuda, batch_full=batch_full, fanouts=fanouts)
+                         cuda=cuda, batch_full=batch_full, fanouts=fanouts, eval_neighbourhood=eval_neighbourhood)
         self.time_step = 0
         self._per_buf = None
         self.pass_var = 0
@@ -312,9 +328,10 @@ class PrioritizedPytorchSupervisedGraphSage(PytorchSupervisedGraphSage):
 class FullPytorchSupervisedGraphSage(PytorchSupervisedGraphSage):
     """offline baseline: `batch_per_timestep` epochs over the whole train set (reference :260-290)."""
 
-    def __init__(self, model, batch_per_timestep, batch_size, labels, samples, cuda=False, batch_full=512, n_workers=0, fanouts=None):
+    def __init__(self, model, batch_per_timestep, batch_size, labels, samples, cuda=False, batch_full=512, n_workers=0, fanouts=None,
+                 eval_neighbourhood="sampled"):
         super().__init__(model, batch_per_timestep, batch_size, labels, samples, n_workers=n_workers, cuda=cuda,
-                         batch_full=batch_full, fanouts=fanouts)
+                         batch_full=batch_full, fanouts=fanouts, eval_neighbourhood=eval_neighbourhood)
 
     def choose_vertices(self, graph_util):
         return list(graph_util.get_train_set())
@@ -333,9 +350,10 @@ class FullPytorchSupervisedGraphSage(PytorchSupervisedGraphSage):
 class NoRehPytorchSupervisedGraphSage(PytorchSupervisedGraphSage):
     """no rehearsal: train on the newest vertices only (reference :293-323)."""
 
-    def __init__(self, model, batch_per_timestep, batch_size, labels, samples, cuda=False, batch_full=512, n_workers=0, fanouts=None):
+    def __init__(self, model, batch_per_timestep, batch_size, labels, samples, cuda=False, batch_full=512, n_workers=0, fanouts=None,
+                 eval_neighbourhood="sampled"):
         super().__init__(model, batch_per_timestep, batch_size, labels, samples, n_workers=n_workers, cuda=cuda,
-                         batch_full=batch_full, fanouts=fanouts)
+                         batch_full=batch_full, fanouts=fanouts, eval_neighbourhood=eval_neighbourhood)
 
     def choose_vertices(self, graph_util):
         return []

@@ -45,6 +45,9 @@ def parse(argv=None):
                     help="arithmetic of the dense path: tf32 (default: tensor cores, rtol 1e-3 vs the reference's fp32, fp32 range), bf16 (fastest, ~5e-3), "
                          "fp16 (tf32's error at bf16's speed; loss-scaled, standardised features), fp32 (exact, SIMT)")
     ap.add_argument("--fast_choosers", action="store_true", help="on-GPU counter-RNG draws / proportional PBR instead of the literal reference choosers")
+    ap.add_argument("--eval_neighbourhood", choices=["sampled", "full"], default="sampled",
+                    help="neighbourhoods the F1 evaluation scores vertices from: sampled (the reference's fan-outs) or full (every in-edge, "
+                         "GraphSAGE.inference: exact and independent of the sampler)")
     args = ap.parse_args(argv)
     custom = {k: v for k, v in vars(args).items() if v is not None}
     with open(os.path.join(ROOT, "settings", args.dataset + ".json")) as f:
@@ -89,7 +92,8 @@ def run(args, data):
     print("create graphsage")
     mk = lambda: GraphSAGE(feat_size, data["embedding_size"], n_classes, data["depth"] - 1, activation, data["dropout"], "pool",
                            edge_feats=data["edge_feats"], pool_feats=data["latent_dim"]).cuda()
-    kw = dict(cuda=data["cuda"], batch_full=data["batch_full"], n_workers=data["n_sampling_workers"])
+    kw = dict(cuda=data["cuda"], batch_full=data["batch_full"], n_workers=data["n_sampling_workers"],
+              eval_neighbourhood=data["eval_neighbourhood"])
     t_random = RandomT(mk(), data["batch_timestep"], data["batch_size"], labels, data["samples"], **kw)
     t_priority = PrioritizedT(mk(), data["batch_timestep"], data["batch_size"], labels, data["samples"], ogl_b200.LossPriority(),
                               full_pass=data["priority_forward"], **kw)
