@@ -249,7 +249,14 @@ int ogl_plan_eval_step(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t
  *   prefetches, captured step graphs).  The plan keeps the activations of every layer for all vertices ([V, pitch] tables, allocated
  *   on first use, grown with the graph, freed with the plan): a graph whose activations do not fit in device memory fails with
  *   OGL_ERR_CAPACITY.  A seed id outside [0, n_vertices) is replaced by vertex 0 and raises bit 0 of ogl_plan_error_flags.
- *   Destination shards (ogl_graph_set_source_bound) are rejected.
+ *   Destination shards (ogl_graph_set_source_bound) are rejected.  It is a loop of ogl_plan_infer_full_layer over the layers.
+ * ogl_plan_infer_full_layer: layer `layer` of ogl_plan_infer_full for the destination rows rows_dev[0..n) (device int64) or, with
+ *   rows_dev == NULL, [row0, row0 + n) (within [0, n_vertices)): hp = relu(h Wp^T + bp) over ALL vertices of g (h = f's table for
+ *   layer 0, h_dev is then unused; else h_dev [n_vertices, ldh] in the storage type, ldh = round_up(layer's input width, 8), 16-byte
+ *   aligned), the segment max over the listed rows, out[0..n) = [h_r | neigh_r] [Ws | Wn]^T + b: ReLU and the storage type with
+ *   ldo = round_up(layer's output width, 8) for a hidden layer, fp32 logits with ldo >= classes for the last.  Every row is computed on
+ *   its own, so any split of the rows gives the bits of the one call over all of them (data-parallel inference: each rank runs its
+ *   rows, then the ranks exchange them).  n == 0 is a no-op.  Same state guarantees, workspace and errors as ogl_plan_infer_full.
  * ogl_graph_segment_max: the segment max on its own: out[r, :cols] = max over the in-edges (u -> v_r) of x[u, :cols], 0 for a vertex
  *   without in-edges, v_r = rows_dev[r] (rows_dev == NULL: v_r = r and n_rows must be the vertex count).  x [*, ld] holds a row for
  *   every vertex of g in the storage type of `mode` (OGL_F32 / OGL_TF32: fp32, OGL_BF16: bf16, OGL_FP16: fp16); x and out 16-byte
@@ -257,6 +264,8 @@ int ogl_plan_eval_step(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t
  *   id outside [0, n_vertices) gives a zero row.  Synchronises `stream` (it frees its scratch before returning). */
 int ogl_plan_infer_full(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds_dev, int64_t n, float* logits_dev,
                         void* stream);
+int ogl_plan_infer_full_layer(ogl_plan* p, ogl_graph* g, ogl_features* f, int layer, const void* h_dev, int ldh,
+                              const int64_t* rows_dev, int64_t row0, int64_t n, void* out_dev, int ldo, void* stream);
 int ogl_graph_segment_max(ogl_graph* g, int mode, const void* x_dev, int ld, int cols, const int64_t* rows_dev, int64_t n_rows,
                           void* out_dev, int ldo, void* stream);
 

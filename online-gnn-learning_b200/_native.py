@@ -366,6 +366,37 @@ class Plan:
         check(lib.ogl_plan_infer_full(self._h, graph._h, features._h, _ptr(s), n, _ptr(out), _stream()))
         return out
 
+    def hidden_table(self, layer, rows):
+        """a [round_up(rows, 128), pitch] table in the plan's storage dtype for the output of hidden `layer` (the input `h` of layer
+        + 1 of infer_full_layer); pitch = round_up(width, 8)"""
+        assert 0 <= layer < self.L - 1, "layer %d has no hidden output (the model has %d layers)" % (layer, self.L)
+        return torch.empty((int(rows) + 127) // 128 * 128, (self.dims[layer + 1] + 7) // 8 * 8, dtype=self.dtype, device="cuda")
+
+    def infer_full_layer(self, graph, features, layer, h, rows=None, row0=0, n=None, out=None):
+        """layer `layer` of infer_full for the destination rows `rows` (int64 ids) or [row0, row0 + n) (n None: to the last vertex):
+        the pool GEMM over every vertex of h (a hidden_table(layer - 1, V) holding the previous layer's output for every vertex;
+        unused for layer 0, which reads `features`), the segment max and the output GEMM over the listed rows.  -> out[:n]: the
+        hidden rows (a hidden_table(layer, n) or a row slice of one) or, for the last layer, fp32 logits [n, C].  Every row is
+        computed on its own, so a split of the rows gives the bits of the one call over all of them."""
+        r = None if rows is None else _dev(rows, torch.int64)
+        if r is not None:
+            n = r.numel()
+        elif n is None:
+            n = graph.num_vertices - int(row0)
+        last = layer == self.L - 1
+        if out is None:
+            out = (torch.empty(n, self.dims[-1], dtype=torch.float32, device="cuda") if last
+                   else self.hidden_table(layer, n))
+        assert out.is_cuda and out.dim() == 2 and out.stride(1) == 1 and out.shape[0] >= n
+        assert out.dtype == (torch.float32 if last else self.dtype)
+        hp, ldh = None, 0
+        if h is not None:
+            assert h.is_cuda and h.dim() == 2 and h.stride(1) == 1 and h.dtype == self.dtype
+            hp, ldh = C.c_void_p(h.data_ptr()), h.stride(0)
+        check(lib.ogl_plan_infer_full_layer(self._h, graph._h, features._h, int(layer), hp, ldh, _ptr(r), int(row0), int(n),
+                                            C.c_void_p(out.data_ptr()), out.stride(0), _stream()))
+        return out[:n]
+
     def reset_optimizer(self, philox_step=0):
         """zero Adam's moments / step counter and set the Philox step (a fresh optimiser; replays of a run from its start)"""
         check(lib.ogl_plan_reset_optimizer(self._h, int(philox_step) & 0xFFFFFFFF, _stream()))

@@ -95,14 +95,14 @@ __device__ __forceinline__ int64_t warp_next(unsigned long long* cursor, int lan
 
 template <typename T, typename Idx>
 __global__ void __launch_bounds__(kBlock) k_csr_segmax_rows(GraphView gv, const T* __restrict__ x, int ld, int strips,
-                                                            const Idx* __restrict__ rows, int64_t n_rows, T* __restrict__ out, int ldo,
+                                                            const Idx* __restrict__ rows, int64_t row0, int64_t n_rows, T* __restrict__ out, int ldo,
                                                             unsigned long long* __restrict__ ctl, SegmaxHub* __restrict__ hubs, int64_t hub_cap,
                                                             int32_t* __restrict__ chunk_hub, int64_t chunk_cap) {
   const int lane = threadIdx.x & 31;
   for (;;) {
     const int64_t r = warp_next(ctl + 0, lane);
     if (r >= n_rows) break;
-    const int64_t v = rows ? (int64_t)rows[r] : r;
+    const int64_t v = rows ? (int64_t)rows[r] : row0 + r;
     T* o = out + r * (int64_t)ldo;
     if (v < 0 || v >= gv.n_vertices) { warp_zero_row(o, strips, lane); continue; }
     const int deg = gv.deg[v];
@@ -176,17 +176,17 @@ __global__ void __launch_bounds__(kBlock) k_csr_segmax_combine(const unsigned lo
 }
 
 template <typename T>
-int launch_segmax(const GraphView& gv, const void* x, int ld, int strips, const int32_t* rows32, const int64_t* rows64, int64_t n_rows,
-                  void* out, int ldo, SegmaxWs* ws, cudaStream_t s) {
+int launch_segmax(const GraphView& gv, const void* x, int ld, int strips, const int32_t* rows32, const int64_t* rows64, int64_t row0,
+                  int64_t n_rows, void* out, int ldo, SegmaxWs* ws, cudaStream_t s) {
   const int ldp = strips * Strip<T>::N;
   const int persistent = sm_count() * 8;
   const int rgrid = (int)std::min<int64_t>(persistent, ceil_div(n_rows, kBlock / 32));
   OGL_CUDA(cudaMemsetAsync(ws->ctl, 0, 4 * sizeof(unsigned long long), s));
   if (rows64)
-    OGL_LAUNCH((k_csr_segmax_rows<T, int64_t>), rgrid, kBlock, 0, s, gv, (const T*)x, ld, strips, rows64, n_rows, (T*)out, ldo, ws->ctl,
+    OGL_LAUNCH((k_csr_segmax_rows<T, int64_t>), rgrid, kBlock, 0, s, gv, (const T*)x, ld, strips, rows64, row0, n_rows, (T*)out, ldo, ws->ctl,
                ws->hubs, ws->hub_cap, ws->chunk_hub, ws->chunk_cap);
   else
-    OGL_LAUNCH((k_csr_segmax_rows<T, int32_t>), rgrid, kBlock, 0, s, gv, (const T*)x, ld, strips, rows32, n_rows, (T*)out, ldo, ws->ctl,
+    OGL_LAUNCH((k_csr_segmax_rows<T, int32_t>), rgrid, kBlock, 0, s, gv, (const T*)x, ld, strips, rows32, row0, n_rows, (T*)out, ldo, ws->ctl,
                ws->hubs, ws->hub_cap, ws->chunk_hub, ws->chunk_cap);
   OGL_LAUNCH((k_csr_segmax_chunks<T>), persistent, kBlock, 0, s, gv, (const T*)x, ld, strips, ws->ctl, ws->hubs, ws->chunk_hub,
              ws->chunk_cap, (T*)ws->partial, ldp);
@@ -220,16 +220,16 @@ int segmax_ws_reserve(SegmaxWs* ws, int64_t n_edges, int64_t row_bytes) {
 }
 
 int csr_segmax(int mode, const GraphView& gv, int64_t n_edges, const void* x, int ld, int cols, const int32_t* rows32,
-               const int64_t* rows64, int64_t n_rows, void* out, int ldo, SegmaxWs* ws, cudaStream_t s) {
+               const int64_t* rows64, int64_t row0, int64_t n_rows, void* out, int ldo, SegmaxWs* ws, cudaStream_t s) {
   if (n_rows <= 0) return OGL_OK;
   const int nv = mode_vec(mode);
   const int strips = (cols + nv - 1) / nv;
   OGL_TRY(segmax_ws_reserve(ws, n_edges, (int64_t)strips * 16));
   switch (mode) {
-    case OGL_BF16: return launch_segmax<__nv_bfloat16>(gv, x, ld, strips, rows32, rows64, n_rows, out, ldo, ws, s);
-    case OGL_FP16: return launch_segmax<__half>(gv, x, ld, strips, rows32, rows64, n_rows, out, ldo, ws, s);
-    case OGL_TF32: return launch_segmax<tf32_t>(gv, x, ld, strips, rows32, rows64, n_rows, out, ldo, ws, s);
-    default: return launch_segmax<float>(gv, x, ld, strips, rows32, rows64, n_rows, out, ldo, ws, s);
+    case OGL_BF16: return launch_segmax<__nv_bfloat16>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s);
+    case OGL_FP16: return launch_segmax<__half>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s);
+    case OGL_TF32: return launch_segmax<tf32_t>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s);
+    default: return launch_segmax<float>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s);
   }
 }
 
@@ -255,7 +255,7 @@ extern "C" int ogl_graph_segment_max(ogl_graph* g, int mode, const void* x_dev, 
           nv, nv);
   cudaStream_t s = (cudaStream_t)stream;
   SegmaxWs ws;
-  int r = csr_segmax(mode, gv, graph_num_edges(g), x_dev, ld, cols, nullptr, rows_dev, n_rows, out_dev, ldo, &ws, s);
+  int r = csr_segmax(mode, gv, graph_num_edges(g), x_dev, ld, cols, nullptr, rows_dev, 0, n_rows, out_dev, ldo, &ws, s);
   if (r == OGL_OK && cudaStreamSynchronize(s) != cudaSuccess) {          // (the workspace is freed below)
     set_error("ogl_graph_segment_max: %s", cudaGetErrorString(cudaGetLastError()));
     r = OGL_ERR_CUDA;

@@ -26,10 +26,10 @@ struct SegmaxWs {
 int segmax_ws_reserve(SegmaxWs* ws, int64_t n_edges, int64_t row_bytes);
 void segmax_ws_free(SegmaxWs* ws);
 
-// out[r, :cols] = max over the in-edges (u -> v_r) of x[u, :cols], 0 for a row without in-edges; v_r = rows32[r] | rows64[r] | r
-// (at most one list).  A listed id outside [0, n_vertices) gives a zero row.  Columns are processed in 16-byte strips, so out
-// columns up to round_up(cols, 16 / element bytes) are written.  Exact: the result does not depend on edge order or on the split.
+// out[r, :cols] = max over the in-edges (u -> v_r) of x[u, :cols], 0 for a row without in-edges; v_r = rows32[r] | rows64[r] |
+// row0 + r (at most one list; row0 is ignored with a list).  A listed id outside [0, n_vertices) gives a zero row.  Columns are
+// processed in 16-byte strips, so out columns up to round_up(cols, 16 / element bytes) are written.  Exact: the result does not depend on edge order or on the split.
 int csr_segmax(int mode, const GraphView& gv, int64_t n_edges, const void* x, int ld, int cols, const int32_t* rows32,
-               const int64_t* rows64, int64_t n_rows, void* out, int ldo, SegmaxWs* ws, cudaStream_t s);
+               const int64_t* rows64, int64_t row0, int64_t n_rows, void* out, int ldo, SegmaxWs* ws, cudaStream_t s);
 
 }  // namespace ogl

@@ -1206,18 +1206,69 @@ static int full_ws_reserve(ogl_plan* p, int64_t rows_needed) {
   return OGL_OK;
 }
 
+// the argument checks both entry points share; *V = the graph's vertex count
+static int full_check(const ogl_plan* p, ogl_graph* g, const ogl_features* f, const char* who, int64_t* V) {
+  OGL_ARG(p && g && f, "%s: null", who);
+  OGL_ARG(p->params, "%s: parameters not bound", who);
+  OGL_ARG(f->mode == p->cfg.mode && f->F == p->cfg.dims[0], "%s: feature store does not match the plan (mode/F)", who);
+  OGL_ARG(graph_source_bound(g) == 0, "%s: the graph is a destination shard (ogl_graph_set_source_bound); full inference needs every "
+          "source row", who);
+  *V = graph_view(g).n_vertices;
+  OGL_ARG(*V <= f->v_cap, "%s: graph has more vertices than the feature store", who);
+  OGL_ARG(*V < (1LL << 31), "%s: too many vertices", who);
+  return OGL_OK;
+}
+
+// layer l for the destination rows rows32[0..n) (device, ids already in [0, V)) or, with rows32 == nullptr, [row0, row0 + n):
+// hp = relu(h Wp^T + bp) over every vertex (layer 0 reads the feature table itself), the segment max over the n rows, then
+// [h_r | neigh_r] [Ws | Wn]^T + b into out [n, ldo]: ReLU and the storage type for a hidden layer, fp32 logits for the last.
+// The GEMMs compute every row on its own, so any split of the rows gives the same bits.
+static int full_layer(ogl_plan* p, const GraphView& gv, int64_t E, const ogl_features* f, int l, const void* h, int ldh,
+                      const int32_t* rows32, int64_t row0, int64_t n, void* out, int ldo, cudaStream_t s) {
+  ogl_plan::FullWs& w = p->full;
+  LayerBuf& lb = p->layer[l];
+  const bool last = l == p->L - 1;
+  const int m = (int)n;
+  if (l == 0) {
+    h = f->table;
+    ldh = f->pitch;
+  }
+  GemmNT g1;
+  g1.a[0] = h; g1.lda[0] = ldh; g1.b[0] = lb.wp; g1.ldb[0] = lb.pin; g1.k[0] = lb.in; g1.n_seg = 1;
+  g1.bias = p->params + lb.o_bp; g1.relu = 1;
+  g1.c = w.hp; g1.ldc = lb.pin; g1.m_max = (int)gv.n_vertices; g1.n = lb.in;
+  g1.in_bf16 = p->bf16; g1.out_bf16 = p->bf16; g1.f16 = p->fp16; g1.tf32 = p->tf32; g1.out_tf32 = p->tf32;
+  STAGE(nm("full.l%d.pool_gemm", l).c_str(), gemm_nt(p, g1, s));
+  STAGE(nm("full.l%d.segmax", l).c_str(), csr_segmax(p->mode, gv, E, w.hp, lb.pin, lb.in, rows32, nullptr, row0, m, w.neigh, lb.pin,
+                                                     &w.sm, s));
+  const int mp = round_up(m, 128);
+  if (mp > m) OGL_CUDA(cudaMemsetAsync((char*)w.neigh + p->es * (size_t)m * lb.pin, 0, p->es * (size_t)(mp - m) * lb.pin, s));
+  // the self term: the listed rows gathered, or the range read in place (the TMA base of the GEMM must be 16-byte aligned)
+  const void* self = (const char*)h + p->es * (size_t)row0 * ldh;
+  if (rows32) {
+    OGL_TRY(gather_rows(p->mode, h, ldh, rows32, nullptr, m, w.hs, s));
+    self = w.hs;
+  }
+  OGL_ARG(((uintptr_t)self & 15) == 0, "full inference: the self rows of layer %d start off the 16-byte grid", l);
+  GemmNT g2;
+  g2.a[0] = self; g2.lda[0] = ldh; g2.b[0] = lb.ws; g2.ldb[0] = lb.pin; g2.k[0] = lb.in;
+  g2.a[1] = w.neigh; g2.lda[1] = lb.pin; g2.b[1] = lb.wn; g2.ldb[1] = lb.pin; g2.k[1] = lb.in; g2.n_seg = 2;
+  g2.bias = p->params + lb.o_bs; g2.bias2 = p->params + lb.o_bn; g2.relu = !last;
+  // (the logits go through the plan's padded buffer: the GEMM writes rows of a multiple of 8 columns)
+  g2.c = last ? (void*)w.logits : out; g2.ldc = last ? lb.pout : ldo; g2.m_max = m; g2.n = lb.out;
+  g2.in_bf16 = p->bf16; g2.out_bf16 = last ? 0 : p->bf16; g2.f16 = p->fp16; g2.tf32 = p->tf32; g2.out_tf32 = last ? 0 : p->tf32;
+  STAGE(nm("full.l%d.out_gemm", l).c_str(), gemm_nt(p, g2, s));
+  if (last)
+    OGL_CUDA(cudaMemcpy2DAsync(out, sizeof(float) * ldo, w.logits, sizeof(float) * lb.pout, sizeof(float) * lb.out, n,
+                               cudaMemcpyDeviceToDevice, s));
+  return OGL_OK;
+}
+
 extern "C" int ogl_plan_infer_full(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds_dev, int64_t n, float* logits_dev,
                                    void* stream) {
-  OGL_ARG(p && g && f, "ogl_plan_infer_full: null");
-  OGL_ARG(p->params, "ogl_plan_infer_full: parameters not bound");
-  OGL_ARG(f->mode == p->cfg.mode && f->F == p->cfg.dims[0], "ogl_plan_infer_full: feature store does not match the plan (mode/F)");
-  OGL_ARG(graph_source_bound(g) == 0, "ogl_plan_infer_full: the graph is a destination shard (ogl_graph_set_source_bound); full inference "
-          "needs every source row");
+  int64_t V = 0;
+  OGL_TRY(full_check(p, g, f, "ogl_plan_infer_full", &V));
   cudaStream_t s = (cudaStream_t)stream;
-  const GraphView gv = graph_view(g);
-  const int64_t V = gv.n_vertices;
-  OGL_ARG(V <= f->v_cap, "ogl_plan_infer_full: graph has more vertices than the feature store");
-  OGL_ARG(V < (1LL << 31), "ogl_plan_infer_full: too many vertices");
   if (!seeds_dev) n = V;
   OGL_ARG(n >= 0 && n < (1LL << 31), "ogl_plan_infer_full: n out of range");
   if (n == 0) return OGL_OK;
@@ -1226,42 +1277,45 @@ extern "C" int ogl_plan_infer_full(ogl_plan* p, ogl_graph* g, ogl_features* f, c
   OGL_TRY(full_ws_reserve(p, std::max(V, n)));
   ogl_plan::FullWs& w = p->full;
   const int L = p->L;
+  const GraphView gv = graph_view(g);
   const int64_t E = graph_num_edges(g);
   // out-of-range seed ids are replaced by vertex 0 and raise error bit 0, as in ogl_plan_eval_step
   if (seeds_dev) OGL_TRY(cast_nodes(seeds_dev, w.seeds, n, V, p->ctl + 2, s));
-  const void* h = f->table;
-  int ldh = f->pitch;
+  const void* h = nullptr;
   for (int l = 0; l < L; ++l) {
-    LayerBuf& lb = p->layer[l];
     const bool last = l == L - 1, on_seeds = last && seeds_dev;
-    const int m = (int)(on_seeds ? n : V);
-    GemmNT g1;
-    g1.a[0] = h; g1.lda[0] = ldh; g1.b[0] = lb.wp; g1.ldb[0] = lb.pin; g1.k[0] = lb.in; g1.n_seg = 1;
-    g1.bias = p->params + lb.o_bp; g1.relu = 1;
-    g1.c = w.hp; g1.ldc = lb.pin; g1.m_max = (int)V; g1.n = lb.in;
-    g1.in_bf16 = p->bf16; g1.out_bf16 = p->bf16; g1.f16 = p->fp16; g1.tf32 = p->tf32; g1.out_tf32 = p->tf32;
-    STAGE(nm("full.l%d.pool_gemm", l).c_str(), gemm_nt(p, g1, s));
-    STAGE(nm("full.l%d.segmax", l).c_str(), csr_segmax(p->mode, gv, E, w.hp, lb.pin, lb.in, on_seeds ? w.seeds : nullptr, nullptr, m,
-                                                       w.neigh, lb.pin, &w.sm, s));
-    const int mp = round_up(m, 128);
-    if (mp > m) OGL_CUDA(cudaMemsetAsync((char*)w.neigh + p->es * (size_t)m * lb.pin, 0, p->es * (size_t)(mp - m) * lb.pin, s));
-    const void* self = h;
-    if (on_seeds) {
-      OGL_TRY(gather_rows(p->mode, h, ldh, w.seeds, nullptr, m, w.hs, s));
-      self = w.hs;
-    }
-    GemmNT g2;
-    g2.a[0] = self; g2.lda[0] = ldh; g2.b[0] = lb.ws; g2.ldb[0] = lb.pin; g2.k[0] = lb.in;
-    g2.a[1] = w.neigh; g2.lda[1] = lb.pin; g2.b[1] = lb.wn; g2.ldb[1] = lb.pin; g2.k[1] = lb.in; g2.n_seg = 2;
-    g2.bias = p->params + lb.o_bs; g2.bias2 = p->params + lb.o_bn; g2.relu = !last;
-    void* out = last ? (void*)w.logits : w.h[l & 1];
-    g2.c = out; g2.ldc = lb.pout; g2.m_max = m; g2.n = lb.out;
-    g2.in_bf16 = p->bf16; g2.out_bf16 = last ? 0 : p->bf16; g2.f16 = p->fp16; g2.tf32 = p->tf32; g2.out_tf32 = last ? 0 : p->tf32;
-    STAGE(nm("full.l%d.out_gemm", l).c_str(), gemm_nt(p, g2, s));
+    void* out = last ? (void*)logits_dev : w.h[l & 1];
+    OGL_TRY(full_layer(p, gv, E, f, l, h, p->layer[l].pin, on_seeds ? w.seeds : nullptr, 0, on_seeds ? n : V, out,
+                       last ? p->cfg.dims[L] : p->layer[l].pout, s));
     h = out;
-    ldh = lb.pout;
   }
-  return unpad_copy(w.logits, p->layer[L - 1].pout, (int)n, nullptr, p->cfg.dims[L], logits_dev, s);
+  return OGL_OK;
+}
+
+extern "C" int ogl_plan_infer_full_layer(ogl_plan* p, ogl_graph* g, ogl_features* f, int layer, const void* h_dev, int ldh,
+                                         const int64_t* rows_dev, int64_t row0, int64_t n, void* out_dev, int ldo, void* stream) {
+  int64_t V = 0;
+  OGL_TRY(full_check(p, g, f, "ogl_plan_infer_full_layer", &V));
+  OGL_ARG(layer >= 0 && layer < p->L, "ogl_plan_infer_full_layer: layer %d out of range [0, %d)", layer, p->L);
+  OGL_ARG(n >= 0 && n < (1LL << 31), "ogl_plan_infer_full_layer: n out of range");
+  OGL_ARG(rows_dev || (row0 >= 0 && row0 + n <= V), "ogl_plan_infer_full_layer: rows [%lld, %lld) are not vertices of the graph (%lld)",
+          (long long)row0, (long long)(row0 + n), (long long)V);
+  if (n == 0) return OGL_OK;
+  OGL_ARG(V > 0, "ogl_plan_infer_full_layer: the graph has no vertices");
+  const LayerBuf& lb = p->layer[layer];
+  const bool last = layer == p->L - 1;
+  OGL_ARG(layer == 0 || (h_dev && ldh == lb.pin && ((uintptr_t)h_dev & 15) == 0),
+          "ogl_plan_infer_full_layer: h must be a 16-byte aligned [n_vertices, %d] table of layer %d's input", lb.pin, layer);
+  if (last)
+    OGL_ARG(out_dev && ldo >= lb.out && ((uintptr_t)out_dev & 3) == 0, "ogl_plan_infer_full_layer: the logits need ldo >= %d", lb.out);
+  else
+    OGL_ARG(out_dev && ldo == lb.pout && ((uintptr_t)out_dev & 15) == 0,
+            "ogl_plan_infer_full_layer: out must be a 16-byte aligned [n, %d] table of layer %d's output", lb.pout, layer);
+  cudaStream_t s = (cudaStream_t)stream;
+  OGL_TRY(full_ws_reserve(p, std::max(V, n)));
+  if (rows_dev) OGL_TRY(cast_nodes(rows_dev, p->full.seeds, n, V, p->ctl + 2, s));
+  return full_layer(p, graph_view(g), graph_num_edges(g), f, layer, h_dev, ldh, rows_dev ? p->full.seeds : nullptr, rows_dev ? 0 : row0, n,
+                    out_dev, ldo, s);
 }
 
 // ------------------------------------------------------------------ stage profiling -----------------

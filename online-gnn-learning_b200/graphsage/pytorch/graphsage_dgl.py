@@ -11,7 +11,7 @@ import math
 import torch
 import torch.nn as nn
 
-from ... import config
+from ... import config, parallel
 from ..._native import Plan
 
 
@@ -154,13 +154,18 @@ class GraphSAGE(nn.Module):
             plan._version = self._version
         return plan
 
-    def inference(self, graph, vertices=None):
+    def inference(self, graph, vertices=None, distributed=False):
         """DGL's `model.inference(g, x)`: fp32 logits [n, C] on the device for `vertices` (int64 ids; None: every vertex of `graph`, a
         DeviceGraph) from their WHOLE in-neighbourhoods -- layer by layer over every vertex and every in-edge, no sampling, no
         feat_drop.  Exact max-pooling makes the result bit-reproducible and independent of edge-insertion order.  Runs on a plan of
         this model kept for `graph` (one full-inference workspace per model and graph); no training or sampled-evaluation state
-        changes.  Ids outside the graph raise bit 0 of that plan's error_flags() (see inference_plan)."""
+        changes.  Ids outside the graph raise bit 0 of that plan's error_flags() (see inference_plan).
+        distributed=True (data-parallel runs, torchrun): every rank computes its share of the rows (parallel.infer_full) and
+        receives the others', so each rank returns the same, bit-identical logits.  It is a collective: every rank of the process
+        group must make the call, which is why it is never switched on implicitly."""
         plan = self.inference_plan(graph)
+        if distributed:
+            return parallel.infer_full(plan, graph.native, graph.features, vertices)
         return plan.infer_full(graph.native, graph.features, seeds=vertices)
 
     def inference_plan(self, graph):

@@ -84,7 +84,8 @@ class PytorchSupervisedGraphSage(SupervisedGraphSage):
             v = torch.as_tensor(np.asarray(test_vertices, dtype=np.int64)).cuda()
             if v.numel() == 0:
                 return None
-            out = self.graphsage_model.inference(graph, v)
+            # under torchrun every rank evaluates in lock-step on the same graph and weights: the ranks share the rows
+            out = self.graphsage_model.inference(graph, v, distributed=parallel.world() > 1)
             if self.graphsage_model.inference_plan(graph).error_flags() & 1:
                 raise IndexError("a vertex id outside the graph was evaluated (DGL's NodeDataLoader raises on such ids)")
             return out

@@ -18,11 +18,76 @@ def rank():
 def shard(seeds, r=None, w=None):
     """rank r's contiguous slice of a global seed list (equal sizes up to the remainder, order preserved)"""
     r = rank() if r is None else r
+    b = shard_bounds(len(seeds), w)
+    return seeds[b[r]:b[r + 1]]
+
+
+def shard_bounds(n, w=None):
+    """the w + 1 boundaries of shard()'s slices of an n-element list"""
     w = world() if w is None else w
-    n = len(seeds)
     base, rem = divmod(n, w)
-    lo = r * base + min(r, rem)
-    return seeds[lo:lo + base + (1 if r < rem else 0)]
+    return [r * base + min(r, rem) for r in range(w + 1)]
+
+
+def edge_balanced_bounds(degrees, w=None):
+    """w + 1 row boundaries 0 = b_0 <= ... <= b_w = V that split the cost sum(deg + 1) of full inference's segment max (one source row
+    read per in-edge, one output row per vertex) evenly: b_r is the first row whose cost prefix reaches r / w of the total, so a
+    shard's cost is off the even share by less than one row's.  degrees: the [V] in-degrees (Graph.degrees()); the graph is
+    replicated, so every rank computes the same bounds."""
+    w = world() if w is None else w
+    cost = degrees.to(torch.int64) + 1
+    prefix = torch.cat([torch.zeros(1, dtype=torch.int64, device=cost.device), torch.cumsum(cost, 0)])
+    total = int(prefix[-1])
+    targets = torch.tensor([(r * total + w - 1) // w for r in range(w + 1)], dtype=torch.int64, device=cost.device)
+    return torch.searchsorted(prefix, targets).tolist()
+
+
+def allgather_rows(table, bounds, group=None):
+    """rank r's rows table[bounds[r]:bounds[r + 1]] go to every rank, in place: one broadcast per non-empty slice from its owner (rows
+    are contiguous, nothing is staged); no-op on one rank"""
+    if world() == 1:
+        return table
+    for r in range(len(bounds) - 1):
+        if bounds[r + 1] > bounds[r]:
+            src = r if group is None else dist.get_global_rank(group, r)
+            dist.broadcast(table[bounds[r]:bounds[r + 1]], src=src, group=group)
+    return table
+
+
+def infer_full(plan, graph, features, vertices=None, exchange=allgather_rows, r=None, w=None):
+    """Plan.infer_full split over the ranks: fp32 logits [n, C] of `vertices` (int64 ids; None: every vertex), the full result on
+    every rank and bit-identical to the one-rank call.  Every hidden layer runs on this rank's edge_balanced_bounds range of rows,
+    then exchange(table, bounds) fills in the other ranks' rows of its [V, pitch] output table; the last layer runs on this rank's
+    shard() of `vertices` (or its range of rows) and its logits are exchanged the same way.  Every rank must call it (the exchange
+    is collective).  r, w: this rank and the number of ranks (default: the process group's; a test runs every rank of a world in
+    one process with them and an exchange of its own)."""
+    r = rank() if r is None else r
+    w = world() if w is None else w
+    V = graph.num_vertices
+    bounds = edge_balanced_bounds(graph.degrees(), w)
+    lo, hi = bounds[r], bounds[r + 1]
+    h = None
+    tables = [None, None]
+    for l in range(plan.L - 1):
+        if tables[l & 1] is None:
+            tables[l & 1] = plan.hidden_table(l, V)
+        out = tables[l & 1]
+        plan.infer_full_layer(graph, features, l, h, row0=lo, n=hi - lo, out=out[lo:hi])
+        exchange(out, bounds)
+        h = out
+    C = plan.dims[-1]
+    if vertices is None:
+        logits = torch.empty(V, C, dtype=torch.float32, device="cuda")
+        plan.infer_full_layer(graph, features, plan.L - 1, h, row0=lo, n=hi - lo, out=logits[lo:hi])
+    else:
+        v = vertices.to(device="cuda", dtype=torch.int64) if isinstance(vertices, torch.Tensor) else \
+            torch.as_tensor(vertices, dtype=torch.int64, device="cuda")
+        logits = torch.empty(v.numel(), C, dtype=torch.float32, device="cuda")
+        bounds = shard_bounds(v.numel(), w)
+        lo, hi = bounds[r], bounds[r + 1]
+        plan.infer_full_layer(graph, features, plan.L - 1, h, rows=v[lo:hi], out=logits[lo:hi])
+    exchange(logits, bounds)
+    return logits
 
 
 def allreduce_grads(flat_grad, group=None):
