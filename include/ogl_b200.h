@@ -141,7 +141,8 @@ int ogl_plan_set_step(ogl_plan* p, uint32_t step, void* stream);
 int ogl_plan_reset_optimizer(ogl_plan* p, uint32_t philox_step, void* stream);
 /* sticky device-side error flags since the last call (synchronises; clears them).  bit 0: a seed id outside [0, n_vertices) was
  * passed to a sampling / train / eval call -- it was replaced by vertex 0 so that no row metadata is read out of bounds (DGL's
- * NodeDataLoader raises on such ids, pytorch/model.py:128-131) */
+ * NodeDataLoader raises on such ids, pytorch/model.py:128-131).  bit 1: ogl_plan_infer_full_loss / ogl_plan_full_xent met a label
+ * outside [0, classes) -- that vertex's loss is NaN (torch's cross_entropy raises on such labels) */
 int ogl_plan_error_flags(ogl_plan* p, uint32_t* out);
 
 /* sample the L-hop minibatch for `seeds` (device int64, n_seeds <= max_seeds) */
@@ -261,11 +262,28 @@ int ogl_plan_eval_step(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t
  *   without in-edges, v_r = rows_dev[r] (rows_dev == NULL: v_r = r and n_rows must be the vertex count).  x [*, ld] holds a row for
  *   every vertex of g in the storage type of `mode` (OGL_F32 / OGL_TF32: fp32, OGL_BF16: bf16, OGL_FP16: fp16); x and out 16-byte
  *   aligned, ld and ldo multiples of 16 bytes; columns are written in 16-byte strips up to round_up(cols, 16 bytes) <= ldo.  A listed
- *   id outside [0, n_vertices) gives a zero row.  Synchronises `stream` (it frees its scratch before returning). */
+ *   id outside [0, n_vertices) gives a zero row.  Synchronises `stream` (it frees its scratch before returning).
+ * ogl_plan_infer_full_loss: ogl_plan_infer_full followed by the per-vertex cross entropy on its logits (PBR priorities from exact
+ *   neighbourhoods, pytorch/model.py:210-254): per_vertex_loss_dev[r] = logsumexp(logits[r, :classes]) - logits[r, y] (fp32 [n]),
+ *   y = f's label of seed r (of vertex r without seeds).  logits_dev (fp32 [n, classes]) may be NULL; when given it receives the
+ *   logits, bit-identical to ogl_plan_infer_full's.  The loss is the training loss's arithmetic (ogl_plan_loss_backward,
+ *   ogl_plan_eval_step): equal logits give bit-equal losses.  Same state guarantees, workspace and rejections as
+ *   ogl_plan_infer_full; an out-of-range seed id uses vertex 0 (logits and label) and raises bit 0, a label outside [0, classes)
+ *   gives NaN and raises bit 1 of ogl_plan_error_flags.
+ * ogl_plan_full_xent: that loss on its own over a caller's fp32 logits block [n, ld] (ld >= classes, the plan's class count): row r
+ *   belongs to vertex rows_dev[r] (device int64) or, with rows_dev == NULL, row0 + r (within the feature store's rows).  A listed id
+ *   outside [0, the feature store's vertex capacity) uses vertex 0's label and raises bit 0; a label outside [0, classes) gives NaN
+ *   and raises bit 1.  n == 0 is a no-op.  Ordered on `stream`, no host synchronisation; changes no plan state but the error flags.
+ *   Data-parallel priorities run the last layer on a rank's rows (ogl_plan_infer_full_layer), this loss on them, and exchange
+ *   only the losses. */
 int ogl_plan_infer_full(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds_dev, int64_t n, float* logits_dev,
                         void* stream);
 int ogl_plan_infer_full_layer(ogl_plan* p, ogl_graph* g, ogl_features* f, int layer, const void* h_dev, int ldh,
                               const int64_t* rows_dev, int64_t row0, int64_t n, void* out_dev, int ldo, void* stream);
+int ogl_plan_infer_full_loss(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds_dev, int64_t n,
+                             float* logits_dev /* may be NULL */, float* per_vertex_loss_dev, void* stream);
+int ogl_plan_full_xent(ogl_plan* p, ogl_features* f, const float* logits_dev, int ld, const int64_t* rows_dev, int64_t row0,
+                       int64_t n, float* per_vertex_loss_dev, void* stream);
 int ogl_graph_segment_max(ogl_graph* g, int mode, const void* x_dev, int ld, int cols, const int64_t* rows_dev, int64_t n_rows,
                           void* out_dev, int ldo, void* stream);
 

@@ -366,6 +366,37 @@ class Plan:
         check(lib.ogl_plan_infer_full(self._h, graph._h, features._h, _ptr(s), n, _ptr(out), _stream()))
         return out
 
+    def infer_full_loss(self, graph, features, seeds=None, logits_out=None, loss_out=None):
+        """infer_full followed by the per-vertex cross entropy on its logits: fp32 losses [n] (logsumexp(logits) - logits[label]), the
+        training loss's arithmetic, so equal logits give bit-equal losses.  logits_out [n, C] (optional) receives the logits, bit-equal
+        to infer_full's.  Changes no plan state; an out-of-range id raises bit 0 of error_flags() (vertex 0 is scored instead), a
+        label outside [0, C) gives NaN and raises bit 1."""
+        s = None if seeds is None else _dev(seeds, torch.int64)
+        n = graph.num_vertices if s is None else s.numel()
+        if logits_out is not None:
+            assert logits_out.is_cuda and logits_out.dtype == torch.float32 and logits_out.is_contiguous() and \
+                tuple(logits_out.shape) == (n, self.dims[-1])
+        out = loss_out if loss_out is not None else torch.empty(n, dtype=torch.float32, device="cuda")
+        assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and tuple(out.shape) == (n,)
+        if n:                                  # (an empty id list has no device pointer: NULL would mean "every vertex")
+            check(lib.ogl_plan_infer_full_loss(self._h, graph._h, features._h, _ptr(s), n, _ptr(logits_out), _ptr(out), _stream()))
+        return out
+
+    def full_xent(self, features, logits, rows=None, row0=0, out=None):
+        """the loss of infer_full_loss on its own: fp32 losses [n] of the fp32 logits [n, >= C] (unit column stride, any row pitch)
+        whose row r belongs to vertex rows[r] (int64 ids) or row0 + r.  Ordered on the stream, no synchronisation."""
+        assert logits.is_cuda and logits.dtype == torch.float32 and logits.dim() == 2 and logits.stride(1) == 1 and \
+            logits.shape[1] >= self.dims[-1], "full_xent: logits must be fp32 [n, >= %d] with unit column stride" % self.dims[-1]
+        n = logits.shape[0]
+        r = None if rows is None else _dev(rows, torch.int64)
+        assert r is None or tuple(r.shape) == (n,), "full_xent: one vertex id per logits row"
+        if out is None:
+            out = torch.empty(n, dtype=torch.float32, device="cuda")
+        assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and tuple(out.shape) == (n,)
+        check(lib.ogl_plan_full_xent(self._h, features._h, C.c_void_p(logits.data_ptr()) if n else None, logits.stride(0),
+                                     _ptr(r), int(row0), n, _ptr(out), _stream()))
+        return out
+
     def hidden_table(self, layer, rows):
         """a [round_up(rows, 128), pitch] table in the plan's storage dtype for the output of hidden `layer` (the input `h` of layer
         + 1 of infer_full_layer); pitch = round_up(width, 8)"""
@@ -402,7 +433,8 @@ class Plan:
         check(lib.ogl_plan_reset_optimizer(self._h, int(philox_step) & 0xFFFFFFFF, _stream()))
 
     def error_flags(self):
-        """sticky device error bits since the last call (bit 0: out-of-range seed id); synchronises"""
+        """sticky device error bits since the last call (bit 0: out-of-range seed id; bit 1: a full-inference loss met a label outside
+        [0, C)); synchronises"""
         v = C.c_uint32()
         check(lib.ogl_plan_error_flags(self._h, C.byref(v)))
         return int(v.value)

@@ -10,7 +10,11 @@
 //   combine: one warp per hub takes the max over its partial rows.
 // Max is exact and order-free, so every split gives the same bits; the only races are on the work cursors.  The reduction uses the
 // float max (fmaxf / __hmax2), not an integer compare of the bit patterns: no sign or NaN assumption on x.
+//
+// The per-vertex cross entropy over full-inference logits (k_full_xent) lives here too: one warp per row, the logsumexp of the
+// training loss (warp_logsumexp, sage_kernels.cuh).
 #include "full_infer.cuh"
+#include "sage_kernels.cuh"
 #include <algorithm>
 
 namespace ogl {
@@ -195,7 +199,45 @@ int launch_segmax(const GraphView& gv, const void* x, int ld, int strips, const 
   return OGL_OK;
 }
 
+// loss[r] = logsumexp(logits[r, :C]) - logits[r, y], y = labels[v_r], v_r = rows[r] | row0 + r.  A v_r outside [0, n_vertices) reads
+// vertex 0's label and sets bit 0 of *err; a label outside [0, C) gives NaN and sets bit 1.
+template <typename Idx>
+__global__ void __launch_bounds__(kBlock) k_full_xent(const float* __restrict__ logits, int ld, int C, const int32_t* __restrict__ labels,
+                                                      const Idx* __restrict__ rows, int64_t row0, int64_t n, int64_t n_vertices,
+                                                      float* __restrict__ loss, uint32_t* __restrict__ err) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  for (int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < n; r += warps) {
+    int64_t v = rows ? (int64_t)rows[r] : row0 + r;
+    uint32_t bits = 0;
+    if (v < 0 || v >= n_vertices) {
+      v = 0;
+      bits |= 1u;
+    }
+    const float* l = logits + r * (int64_t)ld;
+    const float lse = warp_logsumexp(l, C, lane);
+    const int y = labels[v];
+    const bool ok = y >= 0 && y < C;
+    if (!ok) bits |= 2u;
+    if (lane == 0) {
+      loss[r] = ok ? lse - l[y] : __int_as_float(0x7fc00000);
+      if (bits) atomicOr(err, bits);
+    }
+  }
+}
+
 }  // namespace
+
+int full_xent(const float* logits, int ld, int C, const int32_t* labels, const int32_t* rows32, const int64_t* rows64, int64_t row0,
+              int64_t n, int64_t n_vertices, float* loss, uint32_t* err, cudaStream_t s) {
+  if (n <= 0) return OGL_OK;
+  const int grid = (int)std::min<int64_t>(ceil_div(n, kBlock / 32), (int64_t)sm_count() * 16);
+  if (rows64)
+    OGL_LAUNCH(k_full_xent<int64_t>, grid, kBlock, 0, s, logits, ld, C, labels, rows64, row0, n, n_vertices, loss, err);
+  else
+    OGL_LAUNCH(k_full_xent<int32_t>, grid, kBlock, 0, s, logits, ld, C, labels, rows32, row0, n, n_vertices, loss, err);
+  return OGL_OK;
+}
 
 void segmax_ws_free(SegmaxWs* ws) {
   cudaFree(ws->ctl); cudaFree(ws->hubs); cudaFree(ws->chunk_hub); cudaFree(ws->partial);

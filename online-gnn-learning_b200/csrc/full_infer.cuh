@@ -32,4 +32,10 @@ void segmax_ws_free(SegmaxWs* ws);
 int csr_segmax(int mode, const GraphView& gv, int64_t n_edges, const void* x, int ld, int cols, const int32_t* rows32,
                const int64_t* rows64, int64_t row0, int64_t n_rows, void* out, int ldo, SegmaxWs* ws, cudaStream_t s);
 
+// loss[r] = logsumexp(logits[r, :C]) - logits[r, labels[v_r]] for r < n (fp32 logits [n, ld]), v_r = rows32[r] | rows64[r] | row0 + r
+// (at most one list).  The arithmetic of the training loss (warp_logsumexp): equal logits give bit-equal losses.  A v_r outside
+// [0, n_vertices) uses vertex 0's label and ORs 1 into *err; a label outside [0, C) gives NaN and ORs 2 into *err.
+int full_xent(const float* logits, int ld, int C, const int32_t* labels, const int32_t* rows32, const int64_t* rows64, int64_t row0,
+              int64_t n, int64_t n_vertices, float* loss, uint32_t* err, cudaStream_t s);
+
 }  // namespace ogl

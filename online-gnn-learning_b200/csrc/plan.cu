@@ -1138,7 +1138,7 @@ extern "C" int ogl_plan_set_option(ogl_plan* p, const char* name, int value) {
 }
 
 // bit 0: a seed id outside [0, n_vertices) was handed to a sampling call since the last read (it was replaced by vertex 0);
-// synchronises the device, clears the flags
+// bit 1: a full-inference loss met a label outside [0, classes) (its loss is NaN); synchronises the device, clears the flags
 extern "C" int ogl_plan_error_flags(ogl_plan* p, uint32_t* out) {
   OGL_ARG(p && out, "ogl_plan_error_flags: null");
   OGL_CUDA(cudaDeviceSynchronize());
@@ -1258,22 +1258,16 @@ static int full_layer(ogl_plan* p, const GraphView& gv, int64_t E, const ogl_fea
   g2.c = last ? (void*)w.logits : out; g2.ldc = last ? lb.pout : ldo; g2.m_max = m; g2.n = lb.out;
   g2.in_bf16 = p->bf16; g2.out_bf16 = last ? 0 : p->bf16; g2.f16 = p->fp16; g2.tf32 = p->tf32; g2.out_tf32 = last ? 0 : p->tf32;
   STAGE(nm("full.l%d.out_gemm", l).c_str(), gemm_nt(p, g2, s));
-  if (last)
+  if (last && out != (void*)w.logits)
     OGL_CUDA(cudaMemcpy2DAsync(out, sizeof(float) * ldo, w.logits, sizeof(float) * lb.pout, sizeof(float) * lb.out, n,
                                cudaMemcpyDeviceToDevice, s));
   return OGL_OK;
 }
 
-extern "C" int ogl_plan_infer_full(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds_dev, int64_t n, float* logits_dev,
-                                   void* stream) {
-  int64_t V = 0;
-  OGL_TRY(full_check(p, g, f, "ogl_plan_infer_full", &V));
-  cudaStream_t s = (cudaStream_t)stream;
-  if (!seeds_dev) n = V;
-  OGL_ARG(n >= 0 && n < (1LL << 31), "ogl_plan_infer_full: n out of range");
-  if (n == 0) return OGL_OK;
-  OGL_ARG(logits_dev, "ogl_plan_infer_full: null logits");
-  OGL_ARG(V > 0, "ogl_plan_infer_full: the graph has no vertices");
+// the layer loop of ogl_plan_infer_full[_loss] (arguments checked, n > 0, V > 0): logits [n, ldo] of the seeds (w.seeds after the
+// cast) or of every vertex; logits == w.logits (ldo = the last layer's pitch) leaves them in the plan's buffer
+static int full_forward(ogl_plan* p, ogl_graph* g, const ogl_features* f, const int64_t* seeds_dev, int64_t n, int64_t V, float* logits,
+                        int ldo, cudaStream_t s) {
   OGL_TRY(full_ws_reserve(p, std::max(V, n)));
   ogl_plan::FullWs& w = p->full;
   const int L = p->L;
@@ -1284,12 +1278,61 @@ extern "C" int ogl_plan_infer_full(ogl_plan* p, ogl_graph* g, ogl_features* f, c
   const void* h = nullptr;
   for (int l = 0; l < L; ++l) {
     const bool last = l == L - 1, on_seeds = last && seeds_dev;
-    void* out = last ? (void*)logits_dev : w.h[l & 1];
+    void* out = last ? (void*)logits : w.h[l & 1];
     OGL_TRY(full_layer(p, gv, E, f, l, h, p->layer[l].pin, on_seeds ? w.seeds : nullptr, 0, on_seeds ? n : V, out,
-                       last ? p->cfg.dims[L] : p->layer[l].pout, s));
+                       last ? ldo : p->layer[l].pout, s));
     h = out;
   }
   return OGL_OK;
+}
+
+extern "C" int ogl_plan_infer_full(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds_dev, int64_t n, float* logits_dev,
+                                   void* stream) {
+  int64_t V = 0;
+  OGL_TRY(full_check(p, g, f, "ogl_plan_infer_full", &V));
+  if (!seeds_dev) n = V;
+  OGL_ARG(n >= 0 && n < (1LL << 31), "ogl_plan_infer_full: n out of range");
+  if (n == 0) return OGL_OK;
+  OGL_ARG(logits_dev, "ogl_plan_infer_full: null logits");
+  OGL_ARG(V > 0, "ogl_plan_infer_full: the graph has no vertices");
+  return full_forward(p, g, f, seeds_dev, n, V, logits_dev, p->cfg.dims[p->L], (cudaStream_t)stream);
+}
+
+extern "C" int ogl_plan_infer_full_loss(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds_dev, int64_t n, float* logits_dev,
+                                        float* per_vertex_loss_dev, void* stream) {
+  int64_t V = 0;
+  OGL_TRY(full_check(p, g, f, "ogl_plan_infer_full_loss", &V));
+  if (!seeds_dev) n = V;
+  OGL_ARG(n >= 0 && n < (1LL << 31), "ogl_plan_infer_full_loss: n out of range");
+  if (n == 0) return OGL_OK;
+  OGL_ARG(per_vertex_loss_dev, "ogl_plan_infer_full_loss: null loss");
+  OGL_ARG(V > 0, "ogl_plan_infer_full_loss: the graph has no vertices");
+  cudaStream_t s = (cudaStream_t)stream;
+  const int C = p->cfg.dims[p->L];
+  // without a logits buffer of the caller's the loss reads the plan's padded one
+  float* logits = logits_dev;
+  int ld = C;
+  if (!logits_dev) {
+    OGL_TRY(full_ws_reserve(p, std::max(V, n)));
+    logits = p->full.logits;
+    ld = p->layer[p->L - 1].pout;
+  }
+  OGL_TRY(full_forward(p, g, f, seeds_dev, n, V, logits, ld, s));
+  // (the seed ids were cast and range-checked into w.seeds by full_forward)
+  return full_xent(logits, ld, C, f->labels, seeds_dev ? p->full.seeds : nullptr, nullptr, 0, n, V, per_vertex_loss_dev, p->ctl + 2, s);
+}
+
+extern "C" int ogl_plan_full_xent(ogl_plan* p, ogl_features* f, const float* logits_dev, int ld, const int64_t* rows_dev, int64_t row0,
+                                  int64_t n, float* per_vertex_loss_dev, void* stream) {
+  OGL_ARG(p && f, "ogl_plan_full_xent: null");
+  OGL_ARG(n >= 0, "ogl_plan_full_xent: n < 0");
+  if (n == 0) return OGL_OK;
+  const int C = p->cfg.dims[p->L];
+  OGL_ARG(logits_dev && per_vertex_loss_dev && ld >= C && ((uintptr_t)logits_dev & 3) == 0 && ((uintptr_t)per_vertex_loss_dev & 3) == 0,
+          "ogl_plan_full_xent: logits must be fp32 [n, ld] with ld >= %d classes, loss fp32 [n]", C);
+  OGL_ARG(rows_dev || (row0 >= 0 && row0 + n <= f->v_cap), "ogl_plan_full_xent: rows [%lld, %lld) are not rows of the feature store (%lld)",
+          (long long)row0, (long long)(row0 + n), (long long)f->v_cap);
+  return full_xent(logits_dev, ld, C, f->labels, nullptr, rows_dev, row0, n, f->v_cap, per_vertex_loss_dev, p->ctl + 2, (cudaStream_t)stream);
 }
 
 extern "C" int ogl_plan_infer_full_layer(ogl_plan* p, ogl_graph* g, ogl_features* f, int layer, const void* h_dev, int ldh,

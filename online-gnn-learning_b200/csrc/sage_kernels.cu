@@ -340,13 +340,7 @@ __global__ void __launch_bounds__(kBlock) k_xent(const float* __restrict__ logit
   for (int r = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < max(n, nz); r += warps) {
     if (r < n) {
       const float* l = logits + (int64_t)r * ldl;
-      float mx = -INFINITY;
-      for (int c = lane; c < C; c += 32) mx = fmaxf(mx, l[c]);
-      for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-      float se = 0.f;
-      for (int c = lane; c < C; c += 32) se += expf(l[c] - mx);
-      for (int o = 16; o > 0; o >>= 1) se += __shfl_xor_sync(0xffffffffu, se, o);
-      const float lse = mx + logf(se);
+      const float lse = warp_logsumexp(l, C, lane);
       const int y = labels[nodes[r]];
       if (per_loss && lane == 0) per_loss[r] = lse - l[y];
       if (want_grad) {

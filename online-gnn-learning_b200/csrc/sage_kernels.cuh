@@ -20,6 +20,17 @@ __device__ __forceinline__ float adam_math(float gi, float& mi, float& vi, float
   vi = b2 * vi + (1.f - b2) * gi * gi;
   return pi - step * mi / (sqrtf(vi) * isq + eps);
 }
+// one warp: logsumexp of the row l[0..C), the same value on every lane; shared by the training loss (k_xent, sage_kernels.cu) and
+// the full-inference loss (k_full_xent, full_infer.cu) so that equal logits give bit-equal losses
+__device__ __forceinline__ float warp_logsumexp(const float* l, int C, int lane) {
+  float mx = -INFINITY;
+  for (int c = lane; c < C; c += 32) mx = fmaxf(mx, l[c]);
+  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  float se = 0.f;
+  for (int c = lane; c < C; c += 32) se += expf(l[c] - mx);
+  for (int o = 16; o > 0; o >>= 1) se += __shfl_xor_sync(0xffffffffu, se, o);
+  return mx + logf(se);
+}
 #endif
 
 int feat_write(int mode, const float* src, const int64_t* src_rows, int64_t n, int F, void* dst, int pitch, int64_t row0, cudaStream_t s,

@@ -168,6 +168,17 @@ class GraphSAGE(nn.Module):
             return parallel.infer_full(plan, graph.native, graph.features, vertices)
         return plan.infer_full(graph.native, graph.features, seeds=vertices)
 
+    def inference_loss(self, graph, vertices=None, distributed=False):
+        """per-vertex cross-entropy losses (fp32 [n], on the device) of `inference`'s logits against the graph's labels: what PBR
+        ranks its replay buffer by, from exact neighbourhoods.  The arithmetic of the training loss, so equal logits give bit-equal
+        losses.  Ids outside the graph raise bit 0 of inference_plan(graph).error_flags(), labels outside [0, C) give NaN and raise
+        bit 1.  distributed=True: each rank computes the losses of its share of the vertices and only the losses are exchanged
+        (parallel.infer_full_loss); a collective, as for `inference`."""
+        plan = self.inference_plan(graph)
+        if distributed:
+            return parallel.infer_full_loss(plan, graph.native, graph.features, vertices)
+        return plan.infer_full_loss(graph.native, graph.features, seeds=vertices)
+
     def inference_plan(self, graph):
         """the plan `inference` runs on for `graph` (fan-out 1, one seed: only its weights and full-inference workspace are used)"""
         return self.plan_for(graph, [1] * len(self.layers), 1)

@@ -244,8 +244,12 @@ class PrioritizedPytorchSupervisedGraphSage(PytorchSupervisedGraphSage):
     """PBR: loss-prioritised rehearsal (reference :141-257)."""
 
     def __init__(self, model, batch_per_timestep, batch_size, labels, samples, priority_strategy, full_pass=2, cuda=False,
-                 batch_full=512, n_workers=0, fanouts=None, eval_neighbourhood="sampled"):
-        # (recompute_priorities stays on sampled neighbourhoods whatever eval_neighbourhood says)
+                 batch_full=512, n_workers=0, fanouts=None, eval_neighbourhood="sampled", priority_neighbourhood="sampled"):
+        if priority_neighbourhood not in ("sampled", "full"):
+            raise ValueError("priority_neighbourhood must be 'sampled' or 'full', got %r" % (priority_neighbourhood,))
+        # neighbourhoods recompute_priorities scores the train vertices from, independent of eval_neighbourhood: "sampled" (the
+        # reference's fan-outs) or "full" (every in-edge, GraphSAGE.inference_loss)
+        self.priority_neighbourhood = priority_neighbourhood
         super().__init__(model, batch_per_timestep, batch_size, labels, samples, reduction="none", n_workers=n_workers,
                          cuda=cuda, batch_full=batch_full, fanouts=fanouts, eval_neighbourhood=eval_neighbourhood)
         self.time_step = 0
@@ -305,13 +309,26 @@ class PrioritizedPytorchSupervisedGraphSage(PytorchSupervisedGraphSage):
         self.time_step += 1
 
     def recompute_priorities(self, graph_util, train_set):
-        """eval-mode forward over `train_set` in batch_full chunks; per-vertex CE loss -> priorities (reference :210-254)"""
+        """eval-mode forward over `train_set`; per-vertex CE loss -> priorities (reference :210-254).  priority_neighbourhood="sampled":
+        batch_full chunks of sampled neighbourhoods (each chunk advances the evaluation plan's Philox step).  "full": one
+        GraphSAGE.inference_loss over the whole in-neighbourhoods, shared between the ranks under torchrun; it advances no Philox
+        step.  The losses of training steps (_run_custom_train) are training losses and stay sampled either way."""
         self.graphsage_model.eval()
         id_to_subgraph = graph_util.get_original_to_subgraph_map()
         graph = graph_util.get_graph()
         sub = np.asarray(id_to_subgraph[train_set], dtype=np.int64)
         n = len(sub)
         if n == 0:
+            return
+        if self.priority_neighbourhood == "full":
+            m = self.graphsage_model
+            losses = m.inference_loss(graph, torch.as_tensor(sub).cuda(), distributed=parallel.world() > 1)
+            flags = m.inference_plan(graph).error_flags()
+            if flags & 1:
+                raise IndexError("a vertex id outside the graph was evaluated (DGL's NodeDataLoader raises on such ids)")
+            if flags & 2:
+                raise ValueError("a train vertex has a label outside [0, %d) (torch's cross_entropy raises on such labels)" % m.dims[-1])
+            self._push_priorities(graph_util, list(train_set), losses)
             return
         seeds = self._host_seeds(sub)
         plan = self._eval_plan(graph)

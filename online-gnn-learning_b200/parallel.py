@@ -63,6 +63,41 @@ def infer_full(plan, graph, features, vertices=None, exchange=allgather_rows, r=
     one process with them and an exchange of its own)."""
     r = rank() if r is None else r
     w = world() if w is None else w
+    h, v, bounds = _hidden_layers(plan, graph, features, vertices, exchange, r, w)
+    lo, hi = bounds[r], bounds[r + 1]
+    logits = torch.empty(graph.num_vertices if v is None else v.numel(), plan.dims[-1], dtype=torch.float32, device="cuda")
+    _last_layer(plan, graph, features, h, v, lo, hi, logits[lo:hi])
+    exchange(logits, bounds)
+    return logits
+
+
+def infer_full_loss(plan, graph, features, vertices=None, exchange=allgather_rows, r=None, w=None):
+    """Plan.infer_full_loss split over the ranks: fp32 per-vertex cross-entropy losses [n] of `vertices` (None: every vertex), the full
+    vector on every rank and bit-identical to the one-rank call.  The hidden layers run and are exchanged exactly as in infer_full;
+    the last layer and the loss run on this rank's share of the vertices, and only the losses (4 bytes per vertex, not 4 C) are
+    exchanged.  A collective, like infer_full; ids outside the graph raise bit 0 of plan.error_flags(), labels outside [0, C) bit 1."""
+    r = rank() if r is None else r
+    w = world() if w is None else w
+    h, v, bounds = _hidden_layers(plan, graph, features, vertices, exchange, r, w)
+    lo, hi = bounds[r], bounds[r + 1]
+    losses = torch.empty(graph.num_vertices if v is None else v.numel(), dtype=torch.float32, device="cuda")
+    if hi > lo:
+        logits = _last_layer(plan, graph, features, h, v, lo, hi, None)
+        if v is None:
+            plan.full_xent(features, logits, row0=lo, out=losses[lo:hi])
+        else:
+            # the label of an id outside the graph is vertex 0's, as in the one-rank call (the last layer has raised bit 0)
+            rows = v[lo:hi]
+            rows = torch.where((rows < 0) | (rows >= graph.num_vertices), torch.zeros_like(rows), rows)
+            plan.full_xent(features, logits, rows=rows, out=losses[lo:hi])
+    exchange(losses, bounds)
+    return losses
+
+
+def _hidden_layers(plan, graph, features, vertices, exchange, r, w):
+    """the hidden layers of infer_full / infer_full_loss, each on this rank's edge_balanced_bounds range of rows and exchanged into a
+    [V, pitch] table -> (the last hidden table, or None for a one-layer model; the vertices as a device int64 tensor, or None; the
+    bounds of the last layer's shards: the row ranges for every vertex, shard_bounds of the list otherwise)"""
     V = graph.num_vertices
     bounds = edge_balanced_bounds(graph.degrees(), w)
     lo, hi = bounds[r], bounds[r + 1]
@@ -75,19 +110,18 @@ def infer_full(plan, graph, features, vertices=None, exchange=allgather_rows, r=
         plan.infer_full_layer(graph, features, l, h, row0=lo, n=hi - lo, out=out[lo:hi])
         exchange(out, bounds)
         h = out
-    C = plan.dims[-1]
     if vertices is None:
-        logits = torch.empty(V, C, dtype=torch.float32, device="cuda")
-        plan.infer_full_layer(graph, features, plan.L - 1, h, row0=lo, n=hi - lo, out=logits[lo:hi])
-    else:
-        v = vertices.to(device="cuda", dtype=torch.int64) if isinstance(vertices, torch.Tensor) else \
-            torch.as_tensor(vertices, dtype=torch.int64, device="cuda")
-        logits = torch.empty(v.numel(), C, dtype=torch.float32, device="cuda")
-        bounds = shard_bounds(v.numel(), w)
-        lo, hi = bounds[r], bounds[r + 1]
-        plan.infer_full_layer(graph, features, plan.L - 1, h, rows=v[lo:hi], out=logits[lo:hi])
-    exchange(logits, bounds)
-    return logits
+        return h, None, bounds
+    v = vertices.to(device="cuda", dtype=torch.int64) if isinstance(vertices, torch.Tensor) else \
+        torch.as_tensor(vertices, dtype=torch.int64, device="cuda")
+    return h, v, shard_bounds(v.numel(), w)
+
+
+def _last_layer(plan, graph, features, h, v, lo, hi, out):
+    """the last layer on rows [lo, hi) of the vertices (v None: of the graph) -> fp32 logits [hi - lo, C] (into out if given)"""
+    if v is None:
+        return plan.infer_full_layer(graph, features, plan.L - 1, h, row0=lo, n=hi - lo, out=out)
+    return plan.infer_full_layer(graph, features, plan.L - 1, h, rows=v[lo:hi], out=out)
 
 
 def allreduce_grads(flat_grad, group=None):

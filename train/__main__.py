@@ -48,6 +48,9 @@ def parse(argv=None):
     ap.add_argument("--eval_neighbourhood", choices=["sampled", "full"], default="sampled",
                     help="neighbourhoods the F1 evaluation scores vertices from: sampled (the reference's fan-outs) or full (every in-edge, "
                          "GraphSAGE.inference: exact and independent of the sampler)")
+    ap.add_argument("--priority_neighbourhood", choices=["sampled", "full"], default="sampled",
+                    help="neighbourhoods the prioritized model's priority recomputation scores the train vertices from: sampled (the "
+                         "reference's fan-outs) or full (every in-edge, GraphSAGE.inference_loss: exact, no sampling noise)")
     args = ap.parse_args(argv)
     custom = {k: v for k, v in vars(args).items() if v is not None}
     with open(os.path.join(ROOT, "settings", args.dataset + ".json")) as f:
@@ -96,7 +99,7 @@ def run(args, data):
               eval_neighbourhood=data["eval_neighbourhood"])
     t_random = RandomT(mk(), data["batch_timestep"], data["batch_size"], labels, data["samples"], **kw)
     t_priority = PrioritizedT(mk(), data["batch_timestep"], data["batch_size"], labels, data["samples"], ogl_b200.LossPriority(),
-                              full_pass=data["priority_forward"], **kw)
+                              full_pass=data["priority_forward"], priority_neighbourhood=data["priority_neighbourhood"], **kw)
     t_no_reh = NoRehT(mk(), data["batch_timestep"], data["batch_size"], labels, data["samples"], **kw)
     t_full = FullT(mk(), data["epochs_offline"], data["batch_size"], labels, data["samples"], **kw)
     trainers = [t_random, t_priority, t_no_reh, t_full]
