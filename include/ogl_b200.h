@@ -119,7 +119,9 @@ typedef struct {
   uint64_t seed;         /* Philox key */
   float lr, beta1, beta2, eps;
   float feat_drop;       /* SAGEConv(feat_drop=dropout), graphsage_dgl.py:41-46: dropout of every layer's input rows in training mode
-                            (train steps; ogl_plan_forward after ogl_plan_set_option("train_mode", 1)); 0 = off */
+                            (train steps; ogl_plan_forward after ogl_plan_set_option("train_mode", 1)); 0 = off.  The mask is keyed by
+                            the optimiser step in a train step and by the number of earlier training-mode ogl_plan_forward calls in
+                            a direct forward (each such call advances it; ogl_plan_reset_optimizer zeroes it) */
 } ogl_plan_config;
 
 /* mode OGL_FP16: the power of two the stored activation gradients of a backward pass carry for a given loss scale (1 / global batch):
@@ -147,7 +149,8 @@ int ogl_plan_error_flags(ogl_plan* p, uint32_t* out);
 
 /* sample the L-hop minibatch for `seeds` (device int64, n_seeds <= max_seeds) */
 int ogl_plan_sample(ogl_plan* p, ogl_graph* g, const int64_t* seeds_dev, int n_seeds, void* stream);
-/* forward over the sampled minibatch; logits_dev (fp32 [n_seeds, classes]) may be NULL */
+/* forward over the sampled minibatch; logits_dev (fp32 [n_seeds, classes]) may be NULL.  In training mode with feat_drop > 0 it
+ * advances the direct-forward dropout counter (see ogl_plan_config.feat_drop) */
 int ogl_plan_forward(ogl_plan* p, ogl_features* f, float* logits_dev, void* stream);
 /* loss + backward; grads land in the bound gradient buffer (overwritten).
  * loss_scale multiplies dlogits (1/global_batch for the 'mean' reduction);
@@ -159,9 +162,11 @@ int ogl_plan_loss_backward(ogl_plan* p, ogl_features* f, float loss_scale, float
 /* autograd-compat path (GraphSAGE.forward(blocks, x) + loss.backward() driven from Python):
  * supply the input rows x [n_rows, F] fp32 for the outermost level instead of gathering them
  * (then call ogl_plan_forward with f == NULL), and back-propagate a caller-computed
- * dlogits [n_seeds, classes] fp32 into the bound gradient buffer */
+ * dlogits [n_seeds, classes] fp32 into the bound gradient buffer.  dlogits_amax = max |dlogits| (read only in mode OGL_FP16: the
+ * activation gradients are stored times ogl_fp16_grad_scale(dlogits_amax), so the largest is in (32, 64] whatever the loss's
+ * reduction or scale; 0 or a non-finite value gives scale 1) */
 int ogl_plan_set_input(ogl_plan* p, const float* x_dev, int n_rows, void* stream);
-int ogl_plan_backward(ogl_plan* p, const float* dlogits_dev, void* stream);
+int ogl_plan_backward(ogl_plan* p, const float* dlogits_dev, float dlogits_amax, void* stream);
 int ogl_plan_adam_step(ogl_plan* p, void* stream);
 /* fused: sample + forward + loss + backward (+ Adam if do_step) for host or device seeds */
 int ogl_plan_train_step(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t* seeds, int n_seeds,

@@ -71,7 +71,7 @@ SIGNATURES = {
     "ogl_plan_forward": (_i, [_vp, _vp, _vp, _vp]),
     "ogl_plan_loss_backward": (_i, [_vp, _vp, _f, _vp, _vp, _vp]),
     "ogl_plan_set_input": (_i, [_vp, _vp, _i, _vp]),
-    "ogl_plan_backward": (_i, [_vp, _vp, _vp]),
+    "ogl_plan_backward": (_i, [_vp, _vp, _f, _vp]),
     "ogl_plan_adam_step": (_i, [_vp, _vp]),
     "ogl_plan_train_step": (_i, [_vp, _vp, _vp, _vp, _i, _i, _f, _i, _vp, _vp, _vp]),
     "ogl_plan_train_steps": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _f, _i, _vp, _vp, _vp]),

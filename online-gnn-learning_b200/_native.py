@@ -222,6 +222,7 @@ class Plan:
         self._params = self._grads = None
         self.n_seeds = 0
         self._stamp = 0
+        self._forwards = 0
         self._version = 0
 
     def __del__(self):
@@ -253,6 +254,7 @@ class Plan:
     def forward(self, features, want_logits=True):
         out = torch.empty(self.n_seeds, self.dims[-1], dtype=torch.float32, device="cuda") if want_logits else None
         check(lib.ogl_plan_forward(self._h, features._h if features is not None else None, _ptr(out), _stream()))
+        self._forwards += 1              # the activations a backward pass differentiates are this forward's now
         return out
 
     def set_input(self, x):
@@ -265,9 +267,13 @@ class Plan:
         check(lib.ogl_plan_loss_backward(self._h, features._h, float(loss_scale), _ptr(per), _ptr(tot), _stream()))
         return per, tot
 
-    def backward(self, dlogits):
+    def backward(self, dlogits, amax=None):
+        """back-propagate caller-computed fp32 dlogits [n_seeds, C] through the last forward.  amax = max |dlogits|, which mode
+        OGL_FP16 needs for its gradient scale: read from the device (one synchronisation) when not given; other modes ignore it"""
         d = dlogits.to(device="cuda", dtype=torch.float32).contiguous()
-        check(lib.ogl_plan_backward(self._h, _ptr(d), _stream()))
+        if amax is None:
+            amax = float(d.abs().amax()) if self.mode == OGL_FP16 and d.numel() else 0.0
+        check(lib.ogl_plan_backward(self._h, _ptr(d), float(amax), _stream()))
 
     def adam_step(self):
         check(lib.ogl_plan_adam_step(self._h, _stream()))

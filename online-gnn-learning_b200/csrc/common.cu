@@ -187,6 +187,6 @@ int exclusive_scan_i32_to_i64(const int32_t* in, int64_t* out, int64_t n, int64_
 
 extern "C" {
 const char* ogl_last_error(void) { return ogl::t_err; }
-int ogl_version(void) { return 104; }
+int ogl_version(void) { return 105; }
 int64_t ogl_kernel_launches(void) { return (int64_t)ogl::g_launches.load(); }
 }

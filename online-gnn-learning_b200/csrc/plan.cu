@@ -146,7 +146,7 @@ struct ogl_plan {
   cudaEvent_t ev_ring[kSeedRing] = {nullptr, nullptr, nullptr, nullptr};
   int ring_next = 0;
   int cur_open = 0;                      // ogl_plan_step_begin filled the current set and its finish has not been enqueued yet
-  uint32_t* ctl = nullptr;               // [0]=philox step, [1]=adam t
+  uint32_t* ctl = nullptr;               // [0]=philox step, [1]=adam t, [2]=error flags, [3]=direct training-mode forwards
   int n_seeds = 0;
   // backward scratch
   float* tn_partial = nullptr;
@@ -483,6 +483,7 @@ extern "C" int ogl_plan_reset_optimizer(ogl_plan* p, uint32_t philox_step, void*
   OGL_CUDA(cudaMemsetAsync(p->adam_v, 0, sizeof(float) * p->n_params, s));
   const uint32_t ctl[2] = {philox_step, 0u};
   OGL_CUDA(cudaMemcpyAsync(p->ctl, ctl, sizeof(ctl), cudaMemcpyHostToDevice, s));
+  OGL_CUDA(cudaMemsetAsync(p->ctl + 3, 0, sizeof(uint32_t), s));
   OGL_CUDA(cudaStreamSynchronize(s));
   return OGL_OK;
 }
@@ -522,11 +523,12 @@ extern "C" int ogl_plan_sample(ogl_plan* p, ogl_graph* g, const int64_t* seeds_d
   return OGL_OK;
 }
 
-extern "C" int ogl_plan_forward(ogl_plan* p, ogl_features* f, float* logits_dev, void* stream) {
+// drop_step: the device word that keys feat_drop's mask (the last Philox counter word).  A fused step passes its optimiser step
+// ctl[1]; a direct ogl_plan_forward passes ctl[3], see there.
+static int plan_forward(ogl_plan* p, ogl_features* f, float* logits_dev, const uint32_t* drop_step, cudaStream_t s) {
   OGL_ARG(p && p->params, "ogl_plan_forward: null / parameters not bound");
   OGL_ARG(!f || (f->mode == p->cfg.mode && f->F == p->cfg.dims[0]), "ogl_plan_forward: feature store does not match the plan (mode/F)");
   OGL_ARG(p->n_seeds > 0, "ogl_plan_forward: no minibatch sampled");
-  cudaStream_t s = (cudaStream_t)stream;
   const int L = p->L;
   // f == NULL: the input rows were supplied by ogl_plan_set_input
   if (f && !p->skip_gather)
@@ -538,7 +540,7 @@ extern "C" int ogl_plan_forward(ogl_plan* p, ogl_features* f, float* logits_dev,
     // feat_drop: the layer's input rows are dropped out once, in place (they feed fc_pool, h_self and the weight gradients alike)
     if (drop)
       STAGE(nm("l%d.feat_drop", l).c_str(), feat_drop(p->mode, p->act[sl], lb.pin, lb.in, p->counts + sl, p->nmax[sl], p->cfg.feat_drop,
-                                                      p->cfg.seed, p->ctl + 1, l, s));
+                                                      p->cfg.seed, drop_step, l, s));
     GemmNT g1;
     g1.a[0] = p->act[sl]; g1.lda[0] = lb.pin; g1.b[0] = lb.wp; g1.ldb[0] = lb.pin; g1.k[0] = lb.in; g1.n_seg = 1;
     g1.bias = p->params + lb.o_bp; g1.relu = 1;
@@ -557,6 +559,17 @@ extern "C" int ogl_plan_forward(ogl_plan* p, ogl_features* f, float* logits_dev,
   }
   if (logits_dev)
     OGL_TRY(unpad_copy((const float*)p->act[0], p->layer[L - 1].pout, p->nmax[0], p->counts, p->cfg.dims[L], logits_dev, s));
+  return OGL_OK;
+}
+
+// A direct forward in training mode keys its dropout mask by its own counter ctl[3] and advances it.  A caller that drives the
+// forward / backward itself and updates the weights with its own optimiser (the autograd bridge + torch.optim) never runs the
+// plan's Adam, so the optimiser step ctl[1] that keys the fused steps' masks would stay put and every forward would reuse one mask.
+extern "C" int ogl_plan_forward(ogl_plan* p, ogl_features* f, float* logits_dev, void* stream) {
+  OGL_ARG(p, "ogl_plan_forward: null");
+  cudaStream_t s = (cudaStream_t)stream;
+  OGL_TRY(plan_forward(p, f, logits_dev, p->ctl + 3, s));
+  if (p->train_mode && p->cfg.feat_drop > 0.f) OGL_TRY(bump(p->ctl + 3, nullptr, s));
   return OGL_OK;
 }
 
@@ -707,14 +720,15 @@ extern "C" int ogl_plan_set_input(ogl_plan* p, const float* x_dev, int n_rows, v
   return OGL_OK;
 }
 
-extern "C" int ogl_plan_backward(ogl_plan* p, const float* dlogits_dev, void* stream) {
+extern "C" int ogl_plan_backward(ogl_plan* p, const float* dlogits_dev, float dlogits_amax, void* stream) {
   OGL_ARG(p && dlogits_dev && p->params && p->n_seeds > 0, "ogl_plan_backward: plan not ready");
   cudaStream_t s = (cudaStream_t)stream;
   LayerBuf& last = p->layer[p->L - 1];
   const int n = p->n_seeds;
-  // (mode OGL_FP16: the caller's fp32 dlogits carry no scale of their own; a fixed 2^12 puts 1 / batch-sized values into fp16's
-  // normal range with the same headroom as the fused loss)
-  p->grad_scale = p->fp16 ? 4096.f : 1.f;
+  // mode OGL_FP16: the caller's dlogits may have any magnitude (reduction "sum", a scaled loss, a batch of one), so the scale is
+  // the fused loss's rule applied to their largest |element|: it is stored in (32, 64], whatever the loss.  0 or a non-finite
+  // maximum gives scale 1 (zeros stay zeros, inf / NaN propagate).
+  p->grad_scale = grad_scale_for(p, dlogits_amax);
   OGL_TRY(feat_write(p->mode, dlogits_dev, nullptr, n, last.out, last.dpre, last.pout, 0, s, p->grad_scale));
   const int np = round_up(n, 128);
   if (np > n) OGL_CUDA(cudaMemsetAsync((char*)last.dpre + p->es * (size_t)n * last.pout, 0, p->es * (size_t)(np - n) * last.pout, s));
@@ -811,7 +825,7 @@ static int step_body(ogl_plan* p, int kind, ogl_graph* g, ogl_features* f, int n
     p->skip_gather = 1;
     const int keep_mode = p->train_mode;
     p->train_mode = 1;
-    int r = ogl_plan_forward(p, f, nullptr, s);
+    int r = plan_forward(p, f, nullptr, p->ctl + 1, s);
     p->skip_gather = 0;
     // the peers must have finished reading my previous gradients before this step's backward pass overwrites them: checked HERE,
     // after the forward pass (a quarter of a millisecond after they started reading), not at the start of the step where it is a
@@ -840,7 +854,7 @@ static int step_body(ogl_plan* p, int kind, ogl_graph* g, ogl_features* f, int n
   p->skip_gather = (kind == 2 || kind == 3);
   const int keep_mode = p->train_mode;
   p->train_mode = 1;                             // a train step: feat_drop on (the reference calls model.train() first, pytorch/model.py:120)
-  const int rf = ogl_plan_forward(p, f, nullptr, s);
+  const int rf = plan_forward(p, f, nullptr, p->ctl + 1, s);
   p->skip_gather = 0;
   if (rf != OGL_OK) { p->train_mode = keep_mode; return rf; }
   p->tail_mode = (kind == 3) ? 1 : 0;

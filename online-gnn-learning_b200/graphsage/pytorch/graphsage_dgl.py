@@ -65,10 +65,15 @@ class _SageFn(torch.autograd.Function):
         plan.set_input(x)
         logits = plan.forward(None)
         ctx.model, ctx.plan = model, plan
+        ctx.saved = (plan._stamp, plan._forwards)       # the plan keeps ONE set of activations: the ones backward must see
         return logits
 
     @staticmethod
     def backward(ctx, dlogits):
+        if (ctx.plan._stamp, ctx.plan._forwards) != ctx.saved:
+            raise RuntimeError("GraphSAGE backward: the plan has run another forward pass or sampled another minibatch since this "
+                               "output was computed, and it keeps only the latest activations; call backward before the next "
+                               "model(blocks, x) or loader step")
         ctx.plan.backward(dlogits)
         grads = [g.clone() for g in ctx.model._grad_views]
         return (None, None, None) + tuple(grads)
@@ -89,6 +94,7 @@ class GraphSAGE(nn.Module):
                                         activation=None if last else activation))
         self._plans = {}
         self._version = 0
+        self._seen = ()
         self._flat = self._flat_grad = None
         self._grad_views = []
         self._flatten()
@@ -116,6 +122,7 @@ class GraphSAGE(nn.Module):
         for plan in self._plans.values():
             plan.bind_params(self._flat, self._flat_grad)
         self._version += 1
+        self._seen = self._param_versions()
 
     def _apply(self, fn, *a, **k):
         super()._apply(fn, *a, **k)
@@ -129,14 +136,28 @@ class GraphSAGE(nn.Module):
         return out
 
     def params_changed(self):
-        """call after modifying parameters outside the fused kernels (optimizer.step of a torch optimiser, ...)"""
+        """mark the parameters as modified outside the fused kernels.  In-place writes to the parameters themselves (a torch optimiser's
+        step, p.copy_ under torch.no_grad()) are detected without it (_sync_params); this is for writes that bypass their version
+        counters (through p.data or a raw pointer)"""
         self._version += 1
+
+    def _param_versions(self):
+        return tuple(p._version for p in self._ordered_params())
+
+    def _sync_params(self):
+        """an in-place write to a parameter (a torch optimiser's step, load_state_dict, ...) bumps its autograd version counter:
+        if any moved since the last look, every plan's weight shadows are stale"""
+        v = self._param_versions()
+        if v != self._seen:
+            self._seen = v
+            self._version += 1
 
     # ---- plans ------------------------------------------------------------------------------------
     def plan_for(self, graph, hop_fanouts, max_seeds, gemm_impl=0):
         """The fused sampler+model workspace for `graph` (a DeviceGraph), created on first use."""
         if not self._flat.is_cuda:
             raise RuntimeError("ogl_b200 GraphSAGE must live on the GPU: call .cuda() (there is no CPU path)")
+        self._sync_params()
         L = len(self.layers)
         hop_fanouts = list(hop_fanouts)[:L]
         if len(hop_fanouts) != L:
@@ -196,6 +217,7 @@ class GraphSAGE(nn.Module):
                                "NodeDataLoader(..., plan=model.plan_for(graph, hop_fanouts, batch_size))")
         if blocks[0]._stamp != plan._stamp:
             raise RuntimeError("stale blocks: the plan has sampled another minibatch since")
+        self._sync_params()
         if plan._version != self._version:
             plan.refresh_params()
             plan._version = self._version

@@ -195,13 +195,17 @@ def xent(logits, labels, reduction="mean", quant=None):
     return torch.nn.functional.cross_entropy(logits, labels.flatten(), reduction=reduction)
 
 
-def loss_and_grads(params, x_in, blocks, labels, quant=None, dtype=torch.float32):
-    """One fwd+bwd.  Returns (loss_mean, per_vertex_loss, logits, grads dict, intermediates)."""
+def loss_and_grads(params, x_in, blocks, labels, quant=None, dtype=torch.float32, reduction="mean", loss_mult=1.0, grad_scale=None):
+    """One fwd+bwd of loss = loss_mult * cross_entropy(reduction).  Returns (loss, per_vertex_loss, logits, grads dict, intermediates).
+    quant='fp16': grad_scale is the power of two the device's stored activation gradients carry; default: the fused step's for
+    the mean over the labels (the autograd bridge picks it from max |dlogits|: grad_scale_for(max |dlogits|))."""
     p = {k: v.detach().to(dtype).requires_grad_(True) for k, v in params.items()}
-    _GSCALE[0] = grad_scale_for(1.0 / max(1, labels.numel())) if quant == "fp16" else 1.0      # loss = per.mean()
+    if grad_scale is None:
+        grad_scale = grad_scale_for(1.0 / max(1, labels.numel()))
+    _GSCALE[0] = grad_scale if quant == "fp16" else 1.0
     logits, inter = forward(p, x_in.to(dtype), blocks, quant=quant)
     per = xent(logits, labels, "none", quant=quant)
-    loss = per.mean()
+    loss = loss_mult * (per.mean() if reduction == "mean" else per.sum())
     loss.backward()
     return loss.detach(), per.detach(), logits.detach(), {k: v.grad for k, v in p.items()}, inter
 

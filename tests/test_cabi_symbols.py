@@ -29,6 +29,15 @@ def test_binding_table_covers_header():
     assert sorted(SIGNATURES) == declared_symbols()
 
 
+def test_abi_version():
+    """105: ogl_plan_backward takes max |dlogits| (mode OGL_FP16 picks its gradient scale from it)"""
+    import ogl_b200
+    lib = ctypes.CDLL(ogl_b200.LIB_PATH)
+    assert lib.ogl_version() == 105
+    from ogl_b200._lib import SIGNATURES
+    assert SIGNATURES["ogl_plan_backward"][1][2] is ctypes.c_float
+
+
 def test_fails_loudly_without_device():
     import torch
     if torch.cuda.is_available():

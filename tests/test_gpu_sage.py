@@ -62,6 +62,31 @@ def dict_from_flat(flat, dims):
     return out
 
 
+def pin_device_argmax(plan, blocks, inter, ulp):
+    """route the oracle's max-pool gradient through the slots the device picked (sets blocks[l]["arg"]), after checking that every
+    device slot attains the free-running oracle's max (`inter`) within one ulp of the mode: in a rounded arithmetic two neighbours
+    often tie, and which of them wins is decided by the last bit of the fp32 accumulation order"""
+    L = len(blocks)
+    for l in range(L):
+        n_dst, fanout = blocks[l]["n_dst"], blocks[l]["fanout"]
+        dim = inter[l]["hp"].shape[1]
+        arg = plan.tensor(f"arg{l}", rows=n_dst)[:, :dim].long().cpu()
+        arg[arg == 255] = -1
+        assert torch.equal(arg < 0, inter[l]["arg"] < 0)
+        es = blocks[l]["edge_src"].view(n_dst, fanout)
+        src_row = torch.gather(es, 1, arg.clamp(min=0))                      # [n_dst, F] local src row of the device's slot
+        assert bool((src_row[arg >= 0] >= 0).all()), "device argmax points at an empty slot"
+        hp_o = inter[l]["hp"].detach()
+        picked = hp_o[src_row.clamp(min=0), torch.arange(dim)[None, :].expand_as(src_row)]
+        mx = inter[l]["neigh"].detach()
+        # one ulp of the value + the fp32 accumulation-order noise of a cancelling dot product (relative to the scale)
+        # (same tolerance as the comparison of the stored hp itself: layer >= 1 inherits rounding flips of its input)
+        ok = (picked >= mx - 2 * ulp * mx.abs() - ulp * hp_o.abs().max()) | (arg < 0)
+        assert bool(ok.all()), "device argmax slot is not a maximum within one ulp of the mode: %d bad" % int((~ok).sum())
+        blocks[l]["arg"] = arg
+    return blocks
+
+
 class Case:
     def __init__(self, V=1500, E=9000, dims=(50, 24, 5), fanouts=(6, 4), n_seeds=96, mode="fp32", seed=3, gemm_impl=1,
                  isolated=40):
@@ -159,20 +184,7 @@ def test_forward_backward_parity_tcgen05(dims, fanouts, n_seeds, mode):
         n_src, n_dst = c.plan.level_nodes(h + 1).numel(), c.plan.level_nodes(h).numel()
         close(c.plan.tensor(f"hp{l}", rows=n_src)[:, :dims[l]].float(), inter[l]["hp"], ulp, f"hp{l}")
         close(c.plan.tensor(f"neigh{l}", rows=n_dst)[:, :dims[l]].float(), inter[l]["neigh"], ulp, f"neigh{l}")
-        arg = c.plan.tensor(f"arg{l}", rows=n_dst)[:, :dims[l]].long().cpu()
-        arg[arg == 255] = -1
-        assert torch.equal(arg < 0, inter[l]["arg"] < 0)
-        es = blocks[l]["edge_src"].view(n_dst, fanouts[h])
-        src_row = torch.gather(es, 1, arg.clamp(min=0))                      # [n_dst, F] local src row of the device's slot
-        assert bool((src_row[arg >= 0] >= 0).all()), "device argmax points at an empty slot"
-        hp_o = inter[l]["hp"].detach()
-        picked = hp_o[src_row.clamp(min=0), torch.arange(dims[l])[None, :].expand_as(src_row)]
-        mx = inter[l]["neigh"].detach()
-        # one bf16 ulp of the value + the fp32 accumulation-order noise of a cancelling dot product (relative to the scale)
-        # (same tolerance as the comparison of the stored hp itself: layer >= 1 inherits bf16 rounding flips of its input)
-        ok = (picked >= mx - 2 * ulp * mx.abs() - ulp * hp_o.abs().max()) | (arg < 0)
-        assert bool(ok.all()), "device argmax slot is not a maximum within one ulp of the mode: %d bad" % int((~ok).sum())
-        blocks[l]["arg"] = arg
+    pin_device_argmax(c.plan, blocks, inter, ulp)
     # pass 2: gradients with the device's routing through the max-pool
     labels = c.labels[torch.as_tensor(c.seeds)]
     _, _, _, grads_ref, _ = osage.loss_and_grads(c.params, x_in, blocks, labels, quant=mode, dtype=torch.float64)

@@ -255,3 +255,25 @@ def test_fp16_loss_scale_matches_the_oracle_model():
         assert gs == osage.grad_scale_for(a), (a, gs, osage.grad_scale_for(a))
         assert 32.0 < a * gs <= 64.0 and np.log2(gs) == int(np.log2(gs)), (a, gs)
     assert float(lib.ogl_fp16_grad_scale(0.0)) == 1.0 and float(lib.ogl_fp16_grad_scale(float("inf"))) == 1.0
+
+
+def test_graphsage_notices_parameter_writes_outside_the_fused_kernels():
+    """torch.optim updates the parameters in place through their views of the flat buffer and leaves the model alone: the model
+    must see by itself that its plans' weight shadows are stale (every write bumps the parameter's autograd version)"""
+    import torch
+    import ogl_b200
+    model = ogl_b200.GraphSAGE(6, 4, 3, 1, torch.nn.functional.relu, 0, "pool")
+    v0 = model._version
+    model._sync_params()
+    assert model._version == v0, "nothing was written"
+    for p in model.parameters():
+        p.grad = torch.ones_like(p)
+    torch.optim.Adam(model.parameters()).step()
+    model._sync_params()
+    assert model._version == v0 + 1, "an optimiser step was not noticed"
+    model._sync_params()
+    assert model._version == v0 + 1, "one step was counted twice"
+    with torch.no_grad():
+        model.layers[1].fc_neigh.bias[0] = 5.0
+    model._sync_params()
+    assert model._version == v0 + 2, "a single in-place write was not noticed"
