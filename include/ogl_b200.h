@@ -256,6 +256,10 @@ int ogl_plan_eval_step(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t
  *   on first use, grown with the graph, freed with the plan): a graph whose activations do not fit in device memory fails with
  *   OGL_ERR_CAPACITY.  A seed id outside [0, n_vertices) is replaced by vertex 0 and raises bit 0 of ogl_plan_error_flags.
  *   Destination shards (ogl_graph_set_source_bound) are rejected.  It is a loop of ogl_plan_infer_full_layer over the layers.
+ *   With seeds, a hidden layer l runs on S_l only, S_{L-1} = the seeds, S_l = S_{l+1} u N_in(S_{l+1}) (ogl_graph_in_frontier),
+ *   from the top down as long as S_l costs sum(in-degree + 1) <= 0.9 (E + V); that layer and every layer below it run over all
+ *   rows otherwise.  The result is bit-identical either way.  Each expanded layer synchronises `stream` once: the size of S_l is
+ *   copied to the host to size the layer's launches.
  * ogl_plan_infer_full_layer: layer `layer` of ogl_plan_infer_full for the destination rows rows_dev[0..n) (device int64) or, with
  *   rows_dev == NULL, [row0, row0 + n) (within [0, n_vertices)): hp = relu(h Wp^T + bp) over ALL vertices of g (h = f's table for
  *   layer 0, h_dev is then unused; else h_dev [n_vertices, ldh] in the storage type, ldh = round_up(layer's input width, 8), 16-byte
@@ -268,6 +272,10 @@ int ogl_plan_eval_step(ogl_plan* p, ogl_graph* g, ogl_features* f, const int64_t
  *   every vertex of g in the storage type of `mode` (OGL_F32 / OGL_TF32: fp32, OGL_BF16: bf16, OGL_FP16: fp16); x and out 16-byte
  *   aligned, ld and ldo multiples of 16 bytes; columns are written in 16-byte strips up to round_up(cols, 16 bytes) <= ldo.  A listed
  *   id outside [0, n_vertices) gives a zero row.  Synchronises `stream` (it frees its scratch before returning).
+ * ogl_graph_in_frontier: the in-neighbourhood frontier of rows_dev[0..n) (device int64; ids outside [0, n_vertices) are ignored):
+ *   out_rows_dev (device int32, capacity n_vertices) receives the distinct vertices of S u N_in(S) in ascending order, *out_n their
+ *   number and *out_edge_cost the sum over them of (in-degree + 1), the rows and edges a segment max over them reads.  Reads the
+ *   streaming CSR in place (vertex-stream prefixes included).  Synchronises `stream` (it frees its scratch before returning).
  * ogl_plan_infer_full_loss: ogl_plan_infer_full followed by the per-vertex cross entropy on its logits (PBR priorities from exact
  *   neighbourhoods, pytorch/model.py:210-254): per_vertex_loss_dev[r] = logsumexp(logits[r, :classes]) - logits[r, y] (fp32 [n]),
  *   y = f's label of seed r (of vertex r without seeds).  logits_dev (fp32 [n, classes]) may be NULL; when given it receives the
@@ -291,6 +299,8 @@ int ogl_plan_full_xent(ogl_plan* p, ogl_features* f, const float* logits_dev, in
                        int64_t n, float* per_vertex_loss_dev, void* stream);
 int ogl_graph_segment_max(ogl_graph* g, int mode, const void* x_dev, int ld, int cols, const int64_t* rows_dev, int64_t n_rows,
                           void* out_dev, int ldo, void* stream);
+int ogl_graph_in_frontier(ogl_graph* g, const int64_t* rows_dev, int64_t n, int32_t* out_rows_dev, int64_t* out_n,
+                          int64_t* out_edge_cost, void* stream);
 
 /* stage profiling for bench.py's roofline: CUDA events recorded around every stage of the plan's calls on the
  * caller's stream (off by default).  enable=1 (re)starts a collection.  _read synchronises the device and returns,
@@ -305,7 +315,8 @@ int ogl_plan_profile_read(ogl_plan* p, char* names_buf, int names_len, float* ms
 int ogl_plan_level_nodes(ogl_plan* p, int level, const int32_t** nodes_dev, const int32_t** count_dev, int* max_count);
 int ogl_plan_block_edges(ogl_plan* p, int hop, const int32_t** edge_src_local_dev, const int32_t** edge_src_global_dev,
                          const int64_t** edge_eid_dev, int* fanout);
-/* named tensors: "hp<l>", "neigh<l>", "arg<l>", "out<l>" for layer l; returns pointer, rows(max), pitch, elem bytes */
+/* named tensors: "hp<l>", "neigh<l>", "arg<l>", "out<l>" for layer l; "full_h0", "full_h1": the two hidden tables of full inference
+ * (raw [rows, widest hidden pitch] blocks, after its first call); returns pointer, rows(max), pitch, elem bytes */
 int ogl_plan_tensor(ogl_plan* p, const char* name, const void** ptr_dev, int* rows_max, int* pitch, int* elem_bytes);
 
 /* standalone sampler (config 5 sweep + tests): picks into caller buffers.

@@ -155,6 +155,15 @@ class Graph:
                                         _stream()))
         return out[:, :cols]
 
+    def in_frontier(self, rows):
+        """the in-neighbourhood frontier of the vertex ids `rows`: (ids, cost), ids = the distinct vertices of rows and of the sources
+        of their in-edges, ascending (CUDA int64), cost = sum over them of (in-degree + 1).  Ids outside the graph are ignored."""
+        r = _dev(rows, torch.int64)
+        out = torch.empty(max(self.num_vertices, 1), dtype=torch.int32, device="cuda")
+        n, cost = C.c_int64(), C.c_int64()
+        check(lib.ogl_graph_in_frontier(self._h, _ptr(r), r.numel(), _ptr(out), C.byref(n), C.byref(cost), _stream()))
+        return out[:n.value].to(torch.int64), cost.value
+
     def stats(self):
         a = (C.c_int64 * 4)()
         check(lib.ogl_graph_stats(self._h, C.byref(a)))

@@ -11,6 +11,9 @@
 // Max is exact and order-free, so every split gives the same bits; the only races are on the work cursors.  The reduction uses the
 // float max (fmaxf / __hmax2), not an integer compare of the bit patterns: no sign or NaN assumption on x.
 //
+// The in-neighbourhood frontier S u N_in(S) of a row list (k_frontier_*) reads the same CSR: it marks a bitmap, splitting hub rows
+// into the same chunks, and compacts it to ascending ids.  Full inference of a short list runs its hidden layers on these rows only.
+//
 // The per-vertex cross entropy over full-inference logits (k_full_xent) lives here too: one warp per row, the logsumexp of the
 // training loss (warp_logsumexp, sage_kernels.cuh).
 #include "full_infer.cuh"
@@ -199,6 +202,103 @@ int launch_segmax(const GraphView& gv, const void* x, int ld, int strips, const 
   return OGL_OK;
 }
 
+// ---- in-neighbourhood frontier S u N_in(S): mark a bitmap, then compact it to ascending ids (count -> scan -> ballot fill) ----
+// seed: every listed row sets its bit; the lane that set it first owns the vertex and appends it to the distinct-row list, so a
+// vertex listed many times is expanded once
+template <typename Idx>
+__global__ void __launch_bounds__(kBlock) k_frontier_seed(const Idx* __restrict__ rows, int64_t n, int64_t n_vertices, uint32_t* __restrict__ bits,
+                                                          int32_t* __restrict__ uniq, unsigned long long* __restrict__ ctl) {
+  const int lane = threadIdx.x & 31;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i0 = (int64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31); i0 < n; i0 += stride) {
+    const int64_t i = i0 + lane;
+    int64_t v = -1;
+    bool first = false;
+    if (i < n) {
+      v = (int64_t)rows[i];
+      if (v >= 0 && v < n_vertices) {
+        const uint32_t b = 1u << (v & 31);
+        first = !(atomicOr(bits + (v >> 5), b) & b);
+      }
+    }
+    const unsigned m = __ballot_sync(0xffffffffu, first);
+    if (!m) continue;
+    unsigned long long base = 0;
+    if (lane == __ffs(m) - 1) base = atomicAdd(ctl + 0, (unsigned long long)__popc(m));
+    base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
+    if (first) uniq[base + __popc(m & ((1u << lane) - 1))] = (int32_t)v;
+  }
+}
+
+// one warp sets the bits of the sources adj[0..cnt); a bit already set costs a load, not an atomic (hub sources recur)
+__device__ __forceinline__ void warp_mark_sources(const unsigned long long* __restrict__ adj, int cnt, uint32_t* __restrict__ bits, int lane) {
+  for (int j = lane; j < cnt; j += 32) {
+    const uint32_t u = (uint32_t)__ldg(adj + j);
+    const uint32_t b = 1u << (u & 31);
+    if (!(__ldcg(bits + (u >> 5)) & b)) atomicOr(bits + (u >> 5), b);
+  }
+}
+
+// rows: persistent warps take distinct rows from a cursor and mark their sources; a row of more than kSegmaxChunk edges is a hub
+// whose chunks go to the chunk list (if the list is full the warp marks the row itself)
+__global__ void __launch_bounds__(kBlock) k_frontier_rows(GraphView gv, uint32_t* __restrict__ bits, const int32_t* __restrict__ uniq,
+                                                          unsigned long long* __restrict__ ctl, int2* __restrict__ chunks, int64_t chunk_cap) {
+  const int lane = threadIdx.x & 31;
+  const int64_t n = (int64_t)ctl[0];
+  for (;;) {
+    const int64_t i = warp_next(ctl + 1, lane);
+    if (i >= n) break;
+    const int v = uniq[i];
+    const int deg = gv.deg[v];
+    const unsigned long long* adj = gv.adj + gv.row_start[v];
+    if (deg > kSegmaxChunk) {
+      const int nch = (deg + kSegmaxChunk - 1) / kSegmaxChunk;
+      long long base = 0;
+      if (lane == 0) base = (long long)atomicAdd(ctl + 2, (unsigned long long)nch);
+      base = __shfl_sync(0xffffffffu, base, 0);
+      const bool ok = base + nch <= chunk_cap;
+      for (int c = lane; c < nch && base + c < chunk_cap; c += 32) chunks[base + c] = make_int2(ok ? v : -1, c * kSegmaxChunk);
+      if (ok) continue;
+    }
+    warp_mark_sources(adj, deg, bits, lane);
+  }
+}
+
+__global__ void __launch_bounds__(kBlock) k_frontier_chunks(GraphView gv, uint32_t* __restrict__ bits, unsigned long long* __restrict__ ctl,
+                                                            const int2* __restrict__ chunks, int64_t chunk_cap) {
+  const int lane = threadIdx.x & 31;
+  const int64_t n = min((int64_t)ctl[2], chunk_cap);
+  for (;;) {
+    const int64_t c = warp_next(ctl + 3, lane);
+    if (c >= n) break;
+    const int2 ch = chunks[c];
+    if (ch.x < 0) continue;
+    warp_mark_sources(gv.adj + gv.row_start[ch.x] + ch.y, min(kSegmaxChunk, gv.deg[ch.x] - ch.y), bits, lane);
+  }
+}
+
+__global__ void __launch_bounds__(kBlock) k_frontier_count(const uint32_t* __restrict__ bits, int64_t words, int32_t* __restrict__ counts) {
+  for (int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; w < words; w += (int64_t)gridDim.x * blockDim.x) counts[w] = __popc(bits[w]);
+}
+
+// one warp per bitmap word, lane = bit: set bits go to out[offs[word] + rank among the word's set bits]; *cost += deg + 1 of each
+__global__ void __launch_bounds__(kBlock) k_frontier_fill(const uint32_t* __restrict__ bits, const int32_t* __restrict__ offs, int64_t words,
+                                                          const int32_t* __restrict__ deg, int32_t* __restrict__ out,
+                                                          unsigned long long* __restrict__ cost) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  unsigned long long c = 0;
+  for (int64_t w = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < words; w += warps) {
+    const uint32_t word = bits[w];
+    if (!((word >> lane) & 1u)) continue;
+    const int v = (int)(w * 32 + lane);
+    out[offs[w] + __popc(word & ((1u << lane) - 1))] = v;
+    c += (unsigned long long)deg[v] + 1ull;
+  }
+  for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+  if (lane == 0 && c) atomicAdd(cost, c);
+}
+
 // loss[r] = logsumexp(logits[r, :C]) - logits[r, y], y = labels[v_r], v_r = rows[r] | row0 + r.  A v_r outside [0, n_vertices) reads
 // vertex 0's label and sets bit 0 of *err; a label outside [0, C) gives NaN and sets bit 1.
 template <typename Idx>
@@ -236,6 +336,56 @@ int full_xent(const float* logits, int ld, int C, const int32_t* labels, const i
     OGL_LAUNCH(k_full_xent<int64_t>, grid, kBlock, 0, s, logits, ld, C, labels, rows64, row0, n, n_vertices, loss, err);
   else
     OGL_LAUNCH(k_full_xent<int32_t>, grid, kBlock, 0, s, logits, ld, C, labels, rows32, row0, n, n_vertices, loss, err);
+  return OGL_OK;
+}
+
+void frontier_ws_free(FrontierWs* ws) {
+  for (void* q : {(void*)ws->bits, (void*)ws->uniq, (void*)ws->counts, (void*)ws->offs, (void*)ws->scan, (void*)ws->chunks, (void*)ws->ctl,
+                  (void*)ws->out})
+    cudaFree(q);
+  *ws = FrontierWs();
+}
+
+int frontier_ws_reserve(FrontierWs* ws, int64_t n_vertices, int64_t n_edges) {
+  const int64_t chunk_cap = 2 * (n_edges / kSegmaxChunk) + 64;
+  if (ws->ctl && ws->v_cap >= n_vertices && ws->chunk_cap >= chunk_cap) return OGL_OK;
+  const int64_t vc = std::max(n_vertices, ws->v_cap), cc = std::max(chunk_cap, ws->chunk_cap), words = ceil_div(vc, 32) + 1;
+  frontier_ws_free(ws);
+  if (cudaMalloc(&ws->bits, sizeof(uint32_t) * words) != cudaSuccess || cudaMalloc(&ws->uniq, sizeof(int32_t) * vc) != cudaSuccess ||
+      cudaMalloc(&ws->counts, sizeof(int32_t) * words) != cudaSuccess || cudaMalloc(&ws->offs, sizeof(int32_t) * words) != cudaSuccess ||
+      cudaMalloc(&ws->scan, sizeof(int32_t) * scan_scratch_elems(words)) != cudaSuccess ||
+      cudaMalloc(&ws->chunks, sizeof(int2) * cc) != cudaSuccess || cudaMalloc(&ws->ctl, 4 * sizeof(unsigned long long)) != cudaSuccess ||
+      cudaMalloc(&ws->out, sizeof(FrontierOut)) != cudaSuccess) {
+    cudaGetLastError();
+    frontier_ws_free(ws);
+    set_error("in-neighbourhood frontier: cannot allocate the workspace of %lld vertices", (long long)vc);
+    return OGL_ERR_CAPACITY;
+  }
+  ws->v_cap = vc; ws->chunk_cap = cc;
+  return OGL_OK;
+}
+
+int in_frontier(const GraphView& gv, int64_t n_edges, const int32_t* rows32, const int64_t* rows64, int64_t n, int32_t* out_rows,
+                FrontierWs* ws, cudaStream_t s) {
+  OGL_TRY(frontier_ws_reserve(ws, gv.n_vertices, n_edges));
+  const int64_t words = ceil_div(gv.n_vertices, 32);
+  OGL_CUDA(cudaMemsetAsync(ws->bits, 0, sizeof(uint32_t) * words, s));
+  OGL_CUDA(cudaMemsetAsync(ws->ctl, 0, 4 * sizeof(unsigned long long), s));
+  OGL_CUDA(cudaMemsetAsync(ws->out, 0, sizeof(FrontierOut), s));
+  if (n > 0) {
+    const int persistent = sm_count() * 8;
+    if (rows64)
+      OGL_LAUNCH(k_frontier_seed<int64_t>, grid_for(n, kBlock), kBlock, 0, s, rows64, n, gv.n_vertices, ws->bits, ws->uniq, ws->ctl);
+    else
+      OGL_LAUNCH(k_frontier_seed<int32_t>, grid_for(n, kBlock), kBlock, 0, s, rows32, n, gv.n_vertices, ws->bits, ws->uniq, ws->ctl);
+    OGL_LAUNCH(k_frontier_rows, (int)std::min<int64_t>(persistent, ceil_div(n, kBlock / 32)), kBlock, 0, s, gv, ws->bits, ws->uniq, ws->ctl,
+               ws->chunks, ws->chunk_cap);
+    OGL_LAUNCH(k_frontier_chunks, persistent, kBlock, 0, s, gv, ws->bits, ws->ctl, ws->chunks, ws->chunk_cap);
+  }
+  if (words == 0) return OGL_OK;
+  OGL_LAUNCH(k_frontier_count, grid_for(words, kBlock), kBlock, 0, s, ws->bits, words, ws->counts);
+  OGL_TRY(exclusive_scan_i32(ws->counts, ws->offs, words, ws->scan, &ws->out->n, s));
+  OGL_LAUNCH(k_frontier_fill, grid_for(words * 32, kBlock), kBlock, 0, s, ws->bits, ws->offs, words, gv.deg, out_rows, &ws->out->cost);
   return OGL_OK;
 }
 
@@ -303,5 +453,28 @@ extern "C" int ogl_graph_segment_max(ogl_graph* g, int mode, const void* x_dev, 
     r = OGL_ERR_CUDA;
   }
   segmax_ws_free(&ws);
+  return r;
+}
+
+extern "C" int ogl_graph_in_frontier(ogl_graph* g, const int64_t* rows_dev, int64_t n, int32_t* out_rows_dev, int64_t* out_n,
+                                     int64_t* out_edge_cost, void* stream) {
+  OGL_TRY(require_device());
+  OGL_ARG(g && out_n && out_edge_cost && n >= 0 && (rows_dev || n == 0), "ogl_graph_in_frontier: bad arguments");
+  OGL_ARG(graph_source_bound(g) == 0, "ogl_graph_in_frontier: the graph is a destination shard (ogl_graph_set_source_bound): its sources "
+          "are not its rows");
+  const GraphView gv = graph_view(g);
+  OGL_ARG(out_rows_dev || gv.n_vertices == 0, "ogl_graph_in_frontier: null out_rows");
+  cudaStream_t s = (cudaStream_t)stream;
+  FrontierWs ws;
+  FrontierOut h{};
+  int r = in_frontier(gv, graph_num_edges(g), nullptr, rows_dev, n, out_rows_dev, &ws, s);
+  if (r == OGL_OK && (cudaMemcpyAsync(&h, ws.out, sizeof(h), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+                      cudaStreamSynchronize(s) != cudaSuccess)) {
+    set_error("ogl_graph_in_frontier: %s", cudaGetErrorString(cudaGetLastError()));
+    r = OGL_ERR_CUDA;
+  }
+  frontier_ws_free(&ws);
+  *out_n = h.n;
+  *out_edge_cost = (int64_t)h.cost;
   return r;
 }

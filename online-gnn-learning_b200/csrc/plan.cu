@@ -210,9 +210,13 @@ struct ogl_plan {
   struct FullWs {
     int64_t rows = 0;                    // row capacity (a multiple of 128)
     void *hp = nullptr, *neigh = nullptr, *hs = nullptr, *h[2] = {nullptr, nullptr};
+    void* hc = nullptr;                  // a frontier layer's output rows, compact, before the scatter into h[]
     float* logits = nullptr;
     int32_t* seeds = nullptr;
+    int32_t* front = nullptr;            // [L - 1][rows]: the rows hidden layer l needs when it runs on a frontier
     SegmaxWs sm;
+    FrontierWs fr;
+    FrontierOut* fr_host = nullptr;      // pinned
   } full;
 };
 constexpr int kProfSteps = 4096;
@@ -436,8 +440,12 @@ extern "C" int ogl_plan_destroy(ogl_plan* p) {
   for (auto& sg : p->step_graphs) cudaGraphExecDestroy(sg.exec);
   if (p->cap_stream) cudaStreamDestroy(p->cap_stream);
   if (p->prof_counts_host) cudaFreeHost(p->prof_counts_host);
-  for (void* q : {p->full.hp, p->full.neigh, p->full.hs, p->full.h[0], p->full.h[1], (void*)p->full.logits, (void*)p->full.seeds}) cudaFree(q);
+  for (void* q : {p->full.hp, p->full.neigh, p->full.hs, p->full.h[0], p->full.h[1], p->full.hc, (void*)p->full.logits, (void*)p->full.seeds,
+                  (void*)p->full.front})
+    cudaFree(q);
   segmax_ws_free(&p->full.sm);
+  frontier_ws_free(&p->full.fr);
+  if (p->full.fr_host) cudaFreeHost(p->full.fr_host);
   delete p;
   return OGL_OK;
 }
@@ -1199,19 +1207,20 @@ static int full_ws_reserve(ogl_plan* p, int64_t rows_needed) {
     max_pin = std::max(max_pin, p->layer[l].pin);
     if (l < p->L - 1) max_hid = std::max(max_hid, p->layer[l].pout);
   }
-  for (void* q : {w.hp, w.neigh, w.hs, w.h[0], w.h[1], (void*)w.logits, (void*)w.seeds}) cudaFree(q);
-  w.hp = w.neigh = w.hs = w.h[0] = w.h[1] = nullptr;
+  for (void* q : {w.hp, w.neigh, w.hs, w.h[0], w.h[1], w.hc, (void*)w.logits, (void*)w.seeds, (void*)w.front}) cudaFree(q);
+  w.hp = w.neigh = w.hs = w.h[0] = w.h[1] = w.hc = nullptr;
   w.logits = nullptr;
-  w.seeds = nullptr;
+  w.seeds = w.front = nullptr;
   w.rows = 0;
   const size_t r = (size_t)rows;
-  const size_t bytes[7] = {p->es * r * max_pin, p->es * r * max_pin, p->es * r * max_pin, p->es * r * max_hid, p->es * r * max_hid,
-                           sizeof(float) * r * p->layer[p->L - 1].pout, sizeof(int32_t) * r};
-  void** ptrs[7] = {&w.hp, &w.neigh, &w.hs, &w.h[0], &w.h[1], (void**)&w.logits, (void**)&w.seeds};
-  for (int i = 0; i < 7; ++i)
+  const size_t bytes[9] = {p->es * r * max_pin, p->es * r * max_pin, p->es * r * max_pin, p->es * r * max_hid, p->es * r * max_hid,
+                           p->es * r * max_hid, sizeof(float) * r * p->layer[p->L - 1].pout, sizeof(int32_t) * r,
+                           sizeof(int32_t) * r * std::max(p->L - 1, 1)};
+  void** ptrs[9] = {&w.hp, &w.neigh, &w.hs, &w.h[0], &w.h[1], &w.hc, (void**)&w.logits, (void**)&w.seeds, (void**)&w.front};
+  for (int i = 0; i < 9; ++i)
     if (dmalloc0(ptrs[i], bytes[i]) != OGL_OK) {
       cudaGetLastError();
-      for (int j = 0; j < 7; ++j) { cudaFree(*ptrs[j]); *ptrs[j] = nullptr; }
+      for (int j = 0; j < 9; ++j) { cudaFree(*ptrs[j]); *ptrs[j] = nullptr; }
       set_error("ogl_plan_infer_full: cannot allocate the activations of %lld rows (full-graph inference keeps every layer's [V, pitch] "
                 "tables in device memory; graphs that do not fit are not supported)", (long long)rows);
       return OGL_ERR_CAPACITY;
@@ -1278,8 +1287,17 @@ static int full_layer(ogl_plan* p, const GraphView& gv, int64_t E, const ogl_fea
   return OGL_OK;
 }
 
+// A hidden layer runs on the frontier of the rows above it when those rows cost sum(deg + 1) <= kFrontierTheta * (E + V): the
+// segment max then reads their in-edges only.  Above that share the frontier kernels and the row scatter cost more than the edges
+// they save, and the layer (with every layer below it) runs over all rows.  DESIGN.md 3d has the measured crossover.
+constexpr double kFrontierTheta = 0.9;
+
 // the layer loop of ogl_plan_infer_full[_loss] (arguments checked, n > 0, V > 0): logits [n, ldo] of the seeds (w.seeds after the
-// cast) or of every vertex; logits == w.logits (ldo = the last layer's pitch) leaves them in the plan's buffer
+// cast) or of every vertex; logits == w.logits (ldo = the last layer's pitch) leaves them in the plan's buffer.  With seeds, the
+// hidden layers run from the top down on S_{L-1} = the seeds, S_l = S_{l+1} u N_in(S_{l+1}) while S_l is cheap enough (above); each
+// such S_l is read back to the host (one small copy and a stream synchronisation per expanded layer) to size the layer's launches.
+// A frontier layer scatters its rows into the [V, pitch] table; rows outside S_l keep stale contents, which no needed row reads:
+// layer l + 1 reads h at S_{l+1} and N_in(S_{l+1}), both inside S_l, and its pool GEMM computes every row on its own.
 static int full_forward(ogl_plan* p, ogl_graph* g, const ogl_features* f, const int64_t* seeds_dev, int64_t n, int64_t V, float* logits,
                         int ldo, cudaStream_t s) {
   OGL_TRY(full_ws_reserve(p, std::max(V, n)));
@@ -1289,12 +1307,34 @@ static int full_forward(ogl_plan* p, ogl_graph* g, const ogl_features* f, const 
   const int64_t E = graph_num_edges(g);
   // out-of-range seed ids are replaced by vertex 0 and raise error bit 0, as in ogl_plan_eval_step
   if (seeds_dev) OGL_TRY(cast_nodes(seeds_dev, w.seeds, n, V, p->ctl + 2, s));
+  int lo = L - 1;                        // hidden layers [lo, L - 1) run on their frontier rows w.front + l * w.rows
+  std::vector<int64_t> rows_of(L, 0);
+  if (seeds_dev && L > 1) {
+    if (!w.fr_host) OGL_CUDA(cudaMallocHost(&w.fr_host, sizeof(FrontierOut)));
+    const double budget = kFrontierTheta * (double)(E + V);
+    for (int l = L - 2; l >= 0; --l) {
+      const int32_t* above = l == L - 2 ? w.seeds : w.front + (size_t)(l + 1) * w.rows;
+      const int64_t n_above = l == L - 2 ? n : rows_of[l + 1];
+      STAGE(nm("full.l%d.frontier", l).c_str(), in_frontier(gv, E, above, nullptr, n_above, w.front + (size_t)l * w.rows, &w.fr, s));
+      OGL_CUDA(cudaMemcpyAsync(w.fr_host, w.fr.out, sizeof(FrontierOut), cudaMemcpyDeviceToHost, s));
+      OGL_CUDA(cudaStreamSynchronize(s));
+      if ((double)w.fr_host->cost > budget) break;
+      rows_of[l] = w.fr_host->n;
+      lo = l;
+    }
+  }
   const void* h = nullptr;
   for (int l = 0; l < L; ++l) {
     const bool last = l == L - 1, on_seeds = last && seeds_dev;
+    const LayerBuf& lb = p->layer[l];
     void* out = last ? (void*)logits : w.h[l & 1];
-    OGL_TRY(full_layer(p, gv, E, f, l, h, p->layer[l].pin, on_seeds ? w.seeds : nullptr, 0, on_seeds ? n : V, out,
-                       last ? ldo : p->layer[l].pout, s));
+    if (!last && l >= lo) {
+      const int32_t* rows = w.front + (size_t)l * w.rows;
+      OGL_TRY(full_layer(p, gv, E, f, l, h, lb.pin, rows, 0, rows_of[l], w.hc, lb.pout, s));
+      STAGE(nm("full.l%d.scatter", l).c_str(), scatter_rows(p->mode, w.hc, lb.pout, rows, (int)rows_of[l], out, s));
+    } else {
+      OGL_TRY(full_layer(p, gv, E, f, l, h, lb.pin, on_seeds ? w.seeds : nullptr, 0, on_seeds ? n : V, out, last ? ldo : lb.pout, s));
+    }
     h = out;
   }
   return OGL_OK;
@@ -1442,6 +1482,12 @@ extern "C" int ogl_plan_tensor(ogl_plan* p, const char* name, const void** ptr_d
     return OGL_OK;
   };
   if (n == "x") return ret(p->act[L], p->nmax[L], pitch_of(p->cfg.dims[0]), (int)p->es);
+  if (n == "full_h0" || n == "full_h1") {       // full inference's hidden tables (as raw [rows, widest hidden pitch] blocks)
+    OGL_ARG(p->full.h[0], "ogl_plan_tensor: '%s' is allocated by the first full-inference call", name);
+    int max_hid = 8;
+    for (int l = 0; l + 1 < L; ++l) max_hid = std::max(max_hid, p->layer[l].pout);
+    return ret(p->full.h[n.back() - '0'], (int)p->full.rows, max_hid, (int)p->es);
+  }
   if (n.size() >= 2) {
     const int l = n.back() - '0';
     const std::string base = n.substr(0, n.size() - 1);

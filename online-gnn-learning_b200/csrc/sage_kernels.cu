@@ -73,6 +73,20 @@ __global__ void __launch_bounds__(kBlock) k_gather_rows(const T* __restrict__ ta
   }
 }
 
+// table[nodes[r], :] = rows[r, :] for r < n: the inverse of k_gather_rows (distinct nodes: no two rows race)
+template <typename T>
+__global__ void __launch_bounds__(kBlock) k_scatter_rows(const T* __restrict__ rows, int pitch, const int32_t* __restrict__ nodes, int n,
+                                                         T* __restrict__ table) {
+  const int vpr = pitch / Vec<T>::N;
+  const int64_t total = (int64_t)n * vpr;
+  const uint4* rb = reinterpret_cast<const uint4*>(rows);
+  uint4* tb = reinterpret_cast<uint4*>(table);
+  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
+    const int r = (int)(t / vpr), c = (int)(t % vpr);
+    tb[(int64_t)nodes[r] * vpr + c] = __ldg(rb + t);
+  }
+}
+
 // ---- feat_drop: dropout of a layer's input rows, in place (training mode) ----------------------------------------------------
 // graphsage_dgl.py:41-46 hands `dropout` to SAGEConv(feat_drop=...): the layer input is dropped ONCE and the same dropped rows
 // feed h_self and fc_pool.  keep(r, c) = philox4x32_10(counter = (c >> 2, r, 0xD0 + layer, optimiser step), key = seed)[c & 3]
@@ -479,6 +493,12 @@ int label_write(const int64_t* src, const int64_t* src_rows, int64_t n, int32_t*
 int gather_rows(int mode, const void* table, int pitch, const int32_t* nodes, const int32_t* n_dev, int n_max, void* out, cudaStream_t s) {
   const int grid = grid_for((int64_t)n_max * pitch / 8, kBlock, 16);
   L2T(k_gather_rows, grid, s, ARGS((const T*)table, pitch, nodes, n_dev, n_max, (T*)out));
+  return OGL_OK;
+}
+int scatter_rows(int mode, const void* rows, int pitch, const int32_t* nodes, int n, void* table, cudaStream_t s) {
+  if (n <= 0) return OGL_OK;
+  const int grid = grid_for((int64_t)n * pitch / 8, kBlock, 16);
+  L2T(k_scatter_rows, grid, s, ARGS((const T*)rows, pitch, nodes, n, (T*)table));
   return OGL_OK;
 }
 int feat_drop(int mode, void* x, int pitch, int cols, const int32_t* n_dev, int n_max, float p, uint64_t seed, const uint32_t* step_dev,

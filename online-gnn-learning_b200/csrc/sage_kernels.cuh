@@ -37,6 +37,8 @@ int feat_write(int mode, const float* src, const int64_t* src_rows, int64_t n, i
                float scale = 1.f);
 int label_write(const int64_t* src, const int64_t* src_rows, int64_t n, int32_t* dst, int64_t row0, cudaStream_t s);
 int gather_rows(int mode, const void* table, int pitch, const int32_t* nodes, const int32_t* n_dev, int n_max, void* out, cudaStream_t s);
+// table[nodes[r], :] = rows[r, :] for r < n (rows [n, pitch], table [*, pitch], both in the storage type; nodes distinct)
+int scatter_rows(int mode, const void* rows, int pitch, const int32_t* nodes, int n, void* table, cudaStream_t s);
 // in-place dropout of a layer's input rows (no-op for p == 0); step_dev = the optimiser step counter
 int feat_drop(int mode, void* x, int pitch, int cols, const int32_t* n_dev, int n_max, float p, uint64_t seed, const uint32_t* step_dev,
               int layer, cudaStream_t s);
