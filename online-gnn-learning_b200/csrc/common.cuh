@@ -118,8 +118,21 @@ __device__ __forceinline__ float round_tf32(float x) {
 template <> __device__ __forceinline__ float to_f32<tf32_t>(tf32_t v) { return v.v; }
 template <> __device__ __forceinline__ tf32_t from_f32<tf32_t>(float v) { return tf32_t{round_tf32(v)}; }
 
-// element bytes / elements per 16-byte vector of a mode's storage type
+// the arithmetic modes and their storage types: element bytes / elements per 16-byte vector
+static inline int mode_valid(int mode) { return mode == OGL_F32 || mode == OGL_BF16 || mode == OGL_TF32 || mode == OGL_FP16; }
 static inline int mode_is_16bit(int mode) { return mode == OGL_BF16 || mode == OGL_FP16; }
+static inline int mode_bytes(int mode) { return mode_is_16bit(mode) ? 2 : 4; }
 static inline int mode_vec(int mode) { return mode_is_16bit(mode) ? 8 : 4; }
+
+// runs the statement(s) with T = the storage element type of mode: float (OGL_F32), __nv_bfloat16, __half, tf32_t (OGL_TF32)
+#define OGL_MODE_DISPATCH(mode, ...)                                   \
+  do {                                                                 \
+    switch (mode) {                                                    \
+      case OGL_BF16: { using T = __nv_bfloat16; __VA_ARGS__; } break;  \
+      case OGL_FP16: { using T = __half; __VA_ARGS__; } break;         \
+      case OGL_TF32: { using T = ogl::tf32_t; __VA_ARGS__; } break;    \
+      default: { using T = float; __VA_ARGS__; } break;                \
+    }                                                                  \
+  } while (0)
 
 }  // namespace ogl

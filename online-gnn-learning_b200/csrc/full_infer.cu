@@ -417,12 +417,8 @@ int csr_segmax(int mode, const GraphView& gv, int64_t n_edges, const void* x, in
   const int nv = mode_vec(mode);
   const int strips = (cols + nv - 1) / nv;
   OGL_TRY(segmax_ws_reserve(ws, n_edges, (int64_t)strips * 16));
-  switch (mode) {
-    case OGL_BF16: return launch_segmax<__nv_bfloat16>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s);
-    case OGL_FP16: return launch_segmax<__half>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s);
-    case OGL_TF32: return launch_segmax<tf32_t>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s);
-    default: return launch_segmax<float>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s);
-  }
+  OGL_MODE_DISPATCH(mode, OGL_TRY(launch_segmax<T>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s)));
+  return OGL_OK;
 }
 
 }  // namespace ogl
@@ -432,7 +428,7 @@ using namespace ogl;
 extern "C" int ogl_graph_segment_max(ogl_graph* g, int mode, const void* x_dev, int ld, int cols, const int64_t* rows_dev, int64_t n_rows,
                                      void* out_dev, int ldo, void* stream) {
   OGL_TRY(require_device());
-  OGL_ARG(g && (mode == OGL_F32 || mode == OGL_BF16 || mode == OGL_TF32 || mode == OGL_FP16), "ogl_graph_segment_max: bad arguments");
+  OGL_ARG(g && mode_valid(mode), "ogl_graph_segment_max: bad arguments");
   OGL_ARG(graph_source_bound(g) == 0, "ogl_graph_segment_max: the graph is a destination shard (ogl_graph_set_source_bound): its sources "
           "are not rows of x");
   const GraphView gv = graph_view(g);

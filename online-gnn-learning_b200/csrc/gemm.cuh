@@ -1,4 +1,6 @@
 // Dense GEMM entry points of the GraphSAGE-pool path (SIMT fp32-accumulate + tcgen05 bf16 / fp16 / tf32).
+// Operands are in the storage type of the arithmetic mode (common.cuh); in mode OGL_TF32 that is fp32 holding TF32-rounded values,
+// which tcgen05 kind::tf32 reads exactly, as the SIMT path does.
 #pragma once
 #include "common.cuh"
 
@@ -8,7 +10,7 @@ namespace ogl {
 // A, B row-major with the contraction index contiguous ("NT").  Up to two (A, B, K) segments
 // accumulate into the same output (used for [h_self | neigh] x [W_self | W_neigh]^T).
 struct GemmNT {
-  const void* a[2] = {nullptr, nullptr};   // element type = in_bf16 ? bf16 : f32
+  const void* a[2] = {nullptr, nullptr};   // element type = the mode's storage type
   int lda[2] = {0, 0};
   const void* b[2] = {nullptr, nullptr};
   int ldb[2] = {0, 0};
@@ -23,15 +25,13 @@ struct GemmNT {
   float alpha = 1.f;               // scales the accumulated product before the bias (feat_drop's 1 / (1 - p) in the backward pass)
   const void* mask = nullptr;      // same shape/type as A-typed [m, ldmask]: out = mask>0 ? out : 0
   int ldmask = 0;
-  void* c = nullptr;               // out_bf16 ? bf16 : f32
+  void* c = nullptr;               // out_f32 ? f32 : the mode's storage type
   int ldc = 0;
   int m_max = 0;                   // static row bound (grid size)
   const int32_t* m_dev = nullptr;  // dynamic row count on device (nullptr: m_max)
   int n = 0;
-  int in_bf16 = 0, out_bf16 = 0;   // 16-bit operands / output ...
-  int f16 = 0;                     // ... which are fp16 instead of bf16 (mode OGL_FP16)
-  int tf32 = 0;                    // mode OGL_TF32: operands are fp32 holding TF32-rounded values (tcgen05 kind::tf32 / exact on the SIMT path)
-  int out_tf32 = 0;                // ... and the fp32 output is rounded to TF32 too (it is a later GEMM's operand)
+  int mode = OGL_F32;              // arithmetic mode (OGL_F32 | OGL_BF16 | OGL_TF32 | OGL_FP16)
+  int out_f32 = 0;                 // 1: plain fp32 output (logits); 0: the mode's storage type (OGL_TF32: TF32-rounded, a later operand)
   int zero_tail = 1;               // write zeros to rows [m, round_up(m, 128)) (contraction padding for later TN GEMMs)
 };
 
@@ -46,18 +46,23 @@ struct GemmTN {
   int n = 0, k = 0;
   int m_max = 0;
   const int32_t* m_dev = nullptr;
-  int in_bf16 = 0;           // 16-bit operands ...
-  int f16 = 0;               // ... which are fp16 instead of bf16 (mode OGL_FP16)
-  int tf32 = 0;              // operands are fp32 holding TF32-rounded values
+  int mode = OGL_F32;        // arithmetic mode: the operands' storage type
   float alpha = 1.f;         // C = alpha * A^T B (mode OGL_FP16: undoes the loss scale carried by the activation gradients)
   float* partial = nullptr;  // split workspace [splits, n, k]
   int64_t partial_elems = 0;
 };
 
+// tcgen05 when the mode has tensor-core operands (not OGL_F32), SIMT is not forced (force_simt: ogl_plan_config.gemm_impl != 0) and
+// the driver supports it; the SIMT kernels otherwise
+int gemm_nt(const GemmNT& g, int force_simt, cudaStream_t s);
+// up to 4 weight-gradient GEMMs that contract over the same rows: one launch on the tcgen05 path
+int gemm_tn_group(const GemmTN* g, int count, int force_simt, cudaStream_t s);
+static inline int gemm_tn(const GemmTN& g, int force_simt, cudaStream_t s) { return gemm_tn_group(&g, 1, force_simt, s); }
+
 int gemm_nt_simt(const GemmNT& g, cudaStream_t s);
 int gemm_tn_simt(const GemmTN& g, cudaStream_t s);
 
-// tcgen05 / TMA / TMEM versions (bf16 or tf32 operands, fp32 accumulate); same contracts
+// tcgen05 / TMA / TMEM versions (bf16, fp16 or tf32 operands, fp32 accumulate); same contracts
 int gemm_nt_tc(const GemmNT& g, cudaStream_t s);
 int gemm_tn_tc(const GemmTN& g, cudaStream_t s);
 // up to 4 weight-gradient GEMMs contracting over the same rows (same m_dev / m_max) in one launch; g[0].partial is the workspace

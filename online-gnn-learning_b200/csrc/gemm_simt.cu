@@ -202,13 +202,8 @@ int reduce_splits(const float* partial, int splits, int n, int k, float* c, int 
 
 int gemm_nt_simt(const GemmNT& g, cudaStream_t s) {
   dim3 grid((unsigned)ceil_div(g.n, BN), (unsigned)ceil_div(g.m_max, BM));
-  if (g.in_bf16 && g.f16 && g.out_bf16) OGL_LAUNCH((k_gemm_nt<__half, __half>), grid, 256, 0, s, g);
-  else if (g.in_bf16 && g.f16) OGL_LAUNCH((k_gemm_nt<__half, float>), grid, 256, 0, s, g);
-  else if (g.in_bf16 && g.out_bf16) OGL_LAUNCH((k_gemm_nt<__nv_bfloat16, __nv_bfloat16>), grid, 256, 0, s, g);
-  else if (g.in_bf16) OGL_LAUNCH((k_gemm_nt<__nv_bfloat16, float>), grid, 256, 0, s, g);
-  else if (!g.out_bf16 && g.out_tf32) OGL_LAUNCH((k_gemm_nt<float, tf32_t>), grid, 256, 0, s, g);
-  else if (!g.out_bf16) OGL_LAUNCH((k_gemm_nt<float, float>), grid, 256, 0, s, g);
-  else { set_error("gemm_nt_simt: f32 in / bf16 out unsupported"); return OGL_ERR_ARG; }
+  OGL_MODE_DISPATCH(g.mode, if (g.out_f32) OGL_LAUNCH((k_gemm_nt<T, float>), grid, 256, 0, s, g);
+                            else OGL_LAUNCH((k_gemm_nt<T, T>), grid, 256, 0, s, g));
   return OGL_OK;
 }
 
@@ -224,9 +219,7 @@ int gemm_tn_simt(const GemmTN& g, cudaStream_t s) {
   int rows_per_split = (int)ceil_div(g.m_max, splits);
   rows_per_split = (rows_per_split + BK - 1) / BK * BK;
   dim3 grid((unsigned)ceil_div(g.k, BN), (unsigned)ceil_div(g.n, BM), (unsigned)splits);
-  if (g.in_bf16 && g.f16) OGL_LAUNCH((k_gemm_tn<__half>), grid, 256, 0, s, g, rows_per_split, g.partial, per);
-  else if (g.in_bf16) OGL_LAUNCH((k_gemm_tn<__nv_bfloat16>), grid, 256, 0, s, g, rows_per_split, g.partial, per);
-  else OGL_LAUNCH((k_gemm_tn<float>), grid, 256, 0, s, g, rows_per_split, g.partial, per);
+  OGL_MODE_DISPATCH(g.mode, OGL_LAUNCH((k_gemm_tn<T>), grid, 256, 0, s, g, rows_per_split, g.partial, per));
   return reduce_splits(g.partial, splits, g.n, g.k, g.c, g.ldc, s, g.alpha);
 }
 

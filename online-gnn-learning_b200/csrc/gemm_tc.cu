@@ -975,16 +975,31 @@ int tc_init() {
   return 1;
 }
 
-// 2-D bf16 (es = 2) or fp32 (es = 4) tensor [rows, cols] with row pitch ld (elements), box = box_cols x box_rows (box_cols * es
-// = 128 bytes), 128-byte swizzle
-int make_map(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows, int es = 2,
-             CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B, int f16 = 0) {
-  OGL_ARG(((uintptr_t)ptr & 15) == 0 && (ld * es) % 16 == 0, "gemm_tc: operand not 16-byte aligned (ptr %p, ld %lld)", ptr, (long long)ld);
+// what a mode's operands are to the tcgen05 kernels: the kernels' KIND (0 = bf16, 1 = tf32, 2 = fp16), the element bytes and the
+// tensor-map data type.  false for OGL_F32, which has no tensor-core path
+struct TcType {
+  int kind, es;
+  CUtensorMapDataType dtype;
+};
+bool tc_type(int mode, TcType* t) {
+  switch (mode) {
+    case OGL_BF16: *t = {0, 2, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16}; return true;
+    case OGL_TF32: *t = {1, 4, CU_TENSOR_MAP_DATA_TYPE_FLOAT32}; return true;
+    case OGL_FP16: *t = {2, 2, CU_TENSOR_MAP_DATA_TYPE_FLOAT16}; return true;
+    default: return false;
+  }
+}
+
+// 2-D tensor [rows, cols] of t's elements with row pitch ld (elements), box = box_cols x box_rows (box_cols * t.es = 128 bytes),
+// 128-byte swizzle
+int make_map(CUtensorMap* map, const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_cols, int box_rows, const TcType& t,
+             CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
+  OGL_ARG(((uintptr_t)ptr & 15) == 0 && (ld * t.es) % 16 == 0, "gemm_tc: operand not 16-byte aligned (ptr %p, ld %lld)", ptr, (long long)ld);
   cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)(rows > 0 ? rows : 1)};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * (cuuint64_t)es};
+  cuuint64_t strides[1] = {(cuuint64_t)ld * (cuuint64_t)t.es};
   cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = g_encode(map, es == 2 ? (f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16) : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
+  CUresult r = g_encode(map, t.dtype, 2,
                         const_cast<void*>(ptr), dims, strides, box, estr,
                         CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -1045,13 +1060,11 @@ static int launch_gemm(Kernel kernel, int grid, int block, int smem, int cluster
 
 int gemm_nt_tc(const GemmNT& g, cudaStream_t s) {
   OGL_ARG(tc_init() == 1, "gemm_nt_tc: tcgen05 path unavailable (driver lacks cuTensorMapEncodeTiled?)");
-  OGL_ARG((g.in_bf16 != 0) != (g.tf32 != 0), "gemm_nt_tc: 16-bit or tf32 operands only");
-  OGL_ARG(!(g.f16 && g.tf32), "gemm_nt_tc: f16 goes with 16-bit operands");
-  OGL_ARG(!(g.tf32 && g.out_bf16), "gemm_nt_tc: tf32 operands give fp32 output");
+  TcType t;
+  OGL_ARG(tc_type(g.mode, &t), "gemm_nt_tc: 16-bit or tf32 operands only");
   OGL_ARG(g.n > 0 && g.m_max > 0 && g.n_seg >= 1 && g.n_seg <= 2, "gemm_nt_tc: bad shape");
-  const int tf = g.tf32 ? 1 : 0;
-  const int es = tf ? 4 : 2;                 // operand element bytes
-  const int bke = 128 / es;                  // contraction elements per 128-byte swizzle row
+  const int tf = t.kind == 1;
+  const int bke = 128 / t.es;                // contraction elements per 128-byte swizzle row
   NtParams p;
   memset(&p, 0, sizeof(p));
   p.n = g.n;
@@ -1065,8 +1078,8 @@ int gemm_nt_tc(const GemmNT& g, cudaStream_t s) {
     p.k[i] = g.k[i];
     p.a_rows_dev[i] = g.a_rows_dev[i];
     const int64_t a_rows = g.a_rows_max[i] > 0 ? g.a_rows_max[i] : g.m_max;      // rows that exist in segment i's A buffer
-    OGL_TRY(make_map(&p.ta[i], g.a[i], a_rows, g.k[i], g.lda[i], bke, BM, es, CU_TENSOR_MAP_SWIZZLE_128B, g.f16));
-    OGL_TRY(make_map(&p.tb[i], g.b[i], g.n, g.k[i], g.ldb[i], bke, cg == 2 ? p.bn / 2 : p.bn, es, CU_TENSOR_MAP_SWIZZLE_128B, g.f16));
+    OGL_TRY(make_map(&p.ta[i], g.a[i], a_rows, g.k[i], g.lda[i], bke, BM, t));
+    OGL_TRY(make_map(&p.tb[i], g.b[i], g.n, g.k[i], g.ldb[i], bke, cg == 2 ? p.bn / 2 : p.bn, t));
   }
   p.m_dev = g.m_dev;
   p.m_max = g.m_max;
@@ -1078,28 +1091,28 @@ int gemm_nt_tc(const GemmNT& g, cudaStream_t s) {
   p.ldmask = g.ldmask;
   p.c = g.c;
   p.ldc = g.ldc;
-  p.out_bf16 = g.out_bf16;
+  p.out_bf16 = !g.out_f32 && mode_is_16bit(g.mode);
   // tf32 mode: activations leave through 32 x 32 fp32 TMA-store boxes (the logits GEMM -- no rounding, not a later operand -- keeps
   // the direct fp32 stores, its 41 columns are no 16-byte multiple of anything)
-  p.out_f32_tma = (tf && (g.out_tf32 || g.mask)) ? 1 : 0;
-  p.round_out = g.out_tf32;
+  p.out_f32_tma = tf && (!g.out_f32 || g.mask);
+  p.round_out = !g.out_f32 && tf;
   p.zero_tail = g.zero_tail;
-  OGL_ARG(!(g.mask && !(g.out_bf16 || p.out_f32_tma)), "gemm_nt_tc: the mask epilogue is implemented for the TMA-store outputs only");
-  if (g.out_bf16) OGL_TRY(make_map(&p.tc, g.c, g.m_max, g.ldc, g.ldc, 64, 32, 2, CU_TENSOR_MAP_SWIZZLE_128B, g.f16));
-  if (p.out_f32_tma) OGL_TRY(make_map(&p.tc, g.c, g.m_max, g.ldc, g.ldc, 32, 32, 4));
+  OGL_ARG(!(g.mask && !(p.out_bf16 || p.out_f32_tma)), "gemm_nt_tc: the mask epilogue is implemented for the TMA-store outputs only");
+  // TMA-store boxes of 32 rows x 128 bytes in the operands' type
+  if (p.out_bf16 || p.out_f32_tma) OGL_TRY(make_map(&p.tc, g.c, g.m_max, g.ldc, g.ldc, bke, 32, t));
   OGL_ARG(g.ldc % 8 == 0 && ((uintptr_t)g.c & 15) == 0, "gemm_nt_tc: output pitch must be a multiple of 8 elements");
   OGL_ARG(!g.mask || (g.ldmask % 8 == 0 && ((uintptr_t)g.mask & 15) == 0), "gemm_nt_tc: mask pitch must be a multiple of 8 elements");
   if (cg == 2) {
     const int pairs = (int)(super_tiles < sm_count() / 2 ? super_tiles : sm_count() / 2);
-    if (tf) OGL_TRY(launch_gemm(k_gemm_nt_tc<2, 1>, 2 * pairs, THREADS_NT, SMEM_NT2, 2, p, s));
-    else if (g.f16) OGL_TRY(launch_gemm(k_gemm_nt_tc<2, 2>, 2 * pairs, THREADS_NT, SMEM_NT2, 2, p, s));
+    if (t.kind == 1) OGL_TRY(launch_gemm(k_gemm_nt_tc<2, 1>, 2 * pairs, THREADS_NT, SMEM_NT2, 2, p, s));
+    else if (t.kind == 2) OGL_TRY(launch_gemm(k_gemm_nt_tc<2, 2>, 2 * pairs, THREADS_NT, SMEM_NT2, 2, p, s));
     else OGL_TRY(launch_gemm(k_gemm_nt_tc<2, 0>, 2 * pairs, THREADS_NT, SMEM_NT2, 2, p, s));
     return OGL_OK;
   }
   const int64_t tiles = ceil_div(g.m_max, BM) * p.n_tiles;
   const int grid = (int)(tiles < sm_count() ? tiles : sm_count());
-  if (tf) return launch_gemm(k_gemm_nt_tc<1, 1>, grid, THREADS_NT, SMEM_NT1, 1, p, s);
-  if (g.f16) return launch_gemm(k_gemm_nt_tc<1, 2>, grid, THREADS_NT, SMEM_NT1, 1, p, s);
+  if (t.kind == 1) return launch_gemm(k_gemm_nt_tc<1, 1>, grid, THREADS_NT, SMEM_NT1, 1, p, s);
+  if (t.kind == 2) return launch_gemm(k_gemm_nt_tc<1, 2>, grid, THREADS_NT, SMEM_NT1, 1, p, s);
   return launch_gemm(k_gemm_nt_tc<1, 0>, grid, THREADS_NT, SMEM_NT1, 1, p, s);
 }
 
@@ -1111,20 +1124,20 @@ int gemm_tn_tc_group(const GemmTN* g, int count, cudaStream_t s) {
   p.n_prob = count;
   p.m_dev = g[0].m_dev;
   p.m_max = g[0].m_max;
-  const int tf = g[0].tf32 ? 1 : 0;
-  const int es = tf ? 4 : 2;
-  const int cw = 128 / es;                   // TMA box: cw output-index elements (128 bytes) x cw contraction rows
+  TcType t;
+  OGL_ARG(tc_type(g[0].mode, &t), "gemm_tn_tc: 16-bit or tf32 operands only");
+  const int cw = 128 / t.es;                 // TMA box: cw output-index elements (128 bytes) x cw contraction rows
   int tiles = 0;
   int64_t per_total = 0;
   for (int i = 0; i < count; ++i) {
-    OGL_ARG((g[i].in_bf16 || g[i].tf32) && g[i].n > 0 && g[i].k > 0 && g[i].m_max > 0, "gemm_tn_tc: bad arguments");
-    OGL_ARG(g[i].m_dev == g[0].m_dev && g[i].m_max == g[0].m_max && g[i].tf32 == g[0].tf32 && g[i].f16 == g[0].f16,
+    OGL_ARG(g[i].n > 0 && g[i].k > 0 && g[i].m_max > 0, "gemm_tn_tc: bad arguments");
+    OGL_ARG(g[i].m_dev == g[0].m_dev && g[i].m_max == g[0].m_max && g[i].mode == g[0].mode,
             "gemm_tn_tc: grouped problems must contract over the same rows in the same arithmetic");
     TnProblem& q = p.pr[i];
     // (MN-major tf32 operands: the 32-byte-atom flavour of the 128-byte swizzle, see smem_desc)
-    const CUtensorMapSwizzle sw = tf ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B;
-    OGL_TRY(make_map(&q.ta, g[i].a, g[i].m_max, g[i].n, g[i].lda, cw, cw, es, sw, g[i].f16));
-    OGL_TRY(make_map(&q.tb, g[i].b, g[i].m_max, g[i].k, g[i].ldb, cw, cw, es, sw, g[i].f16));
+    const CUtensorMapSwizzle sw = t.kind == 1 ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B;
+    OGL_TRY(make_map(&q.ta, g[i].a, g[i].m_max, g[i].n, g[i].lda, cw, cw, t, sw));
+    OGL_TRY(make_map(&q.tb, g[i].b, g[i].m_max, g[i].k, g[i].ldb, cw, cw, t, sw));
     q.n = g[i].n;
     q.k = g[i].k;
     q.k_tiles = (g[i].k + BN_MAX - 1) / BN_MAX;
@@ -1168,8 +1181,8 @@ int gemm_tn_tc_group(const GemmTN* g, int count, cudaStream_t s) {
   }
   p.use_tma_store = staged ? 1 : 0;
   p.alpha_direct = g[0].alpha;
-  if (tf) OGL_TRY(launch_gemm(k_gemm_tn_tc<1>, tiles * splits, THREADS, SMEM_TN, 1, p, s));
-  else if (g[0].f16) OGL_TRY(launch_gemm(k_gemm_tn_tc<2>, tiles * splits, THREADS, SMEM_TN, 1, p, s));
+  if (t.kind == 1) OGL_TRY(launch_gemm(k_gemm_tn_tc<1>, tiles * splits, THREADS, SMEM_TN, 1, p, s));
+  else if (t.kind == 2) OGL_TRY(launch_gemm(k_gemm_tn_tc<2>, tiles * splits, THREADS, SMEM_TN, 1, p, s));
   else OGL_TRY(launch_gemm(k_gemm_tn_tc<0>, tiles * splits, THREADS, SMEM_TN, 1, p, s));
   if (staged) return reduce_splits_group(rg, s);
   return OGL_OK;
@@ -1177,83 +1190,81 @@ int gemm_tn_tc_group(const GemmTN* g, int count, cudaStream_t s) {
 
 int gemm_tn_tc(const GemmTN& g, cudaStream_t s) { return gemm_tn_tc_group(&g, 1, s); }
 
+static bool use_tc(int mode, int force_simt) { return mode != OGL_F32 && !force_simt && gemm_tc_available(); }
+
+int gemm_nt(const GemmNT& g, int force_simt, cudaStream_t s) {
+  return use_tc(g.mode, force_simt) ? gemm_nt_tc(g, s) : gemm_nt_simt(g, s);
+}
+
+int gemm_tn_group(const GemmTN* g, int count, int force_simt, cudaStream_t s) {
+  if (use_tc(g[0].mode, force_simt)) return gemm_tn_tc_group(g, count, s);
+  for (int i = 0; i < count; ++i) OGL_TRY(gemm_tn_simt(g[i], s));
+  return OGL_OK;
+}
+
 }  // namespace ogl
 
 using namespace ogl;
 
+// the ogl_gemm_* entry points: one contraction segment, no zero tail, always on the tcgen05 path
+static int entry_nt(const char* who, int mode, const void* a, int lda, const void* b, int ldb, void* c, int ldc, int m, int n, int k,
+                    int out_f32, const float* bias, int relu, const void* mask, int ldmask, int cg, void* stream) {
+  OGL_TRY(require_device());
+  OGL_ARG(a && b && c && m > 0 && n > 0 && k > 0, "%s: bad arguments", who);
+  GemmNT g;
+  g.a[0] = a; g.lda[0] = lda; g.b[0] = b; g.ldb[0] = ldb; g.k[0] = k; g.n_seg = 1;
+  g.c = c; g.ldc = ldc; g.m_max = m; g.n = n; g.mode = mode; g.out_f32 = out_f32; g.zero_tail = 0;
+  g.bias = bias; g.relu = relu; g.force_cg = cg; g.mask = mask; g.ldmask = ldmask;
+  return gemm_nt_tc(g, (cudaStream_t)stream);
+}
+
+static int entry_tn(const char* who, int mode, const void* a, int lda, const void* b, int ldb, float* c, int ldc, int m, int n, int k,
+                    float alpha, float* workspace, int64_t workspace_elems, void* stream) {
+  OGL_TRY(require_device());
+  OGL_ARG(a && b && c && m > 0 && n > 0 && k > 0, "%s: bad arguments", who);
+  GemmTN g;
+  g.a = a; g.lda = lda; g.b = b; g.ldb = ldb; g.c = c; g.ldc = ldc; g.n = n; g.k = k; g.m_max = m; g.mode = mode; g.alpha = alpha;
+  g.partial = workspace; g.partial_elems = workspace ? workspace_elems : 0;
+  return gemm_tn_tc(g, (cudaStream_t)stream);
+}
+
 extern "C" int ogl_gemm_bf16_nt(const void* a_dev, int lda, const void* b_dev, int ldb, float* c_dev, int ldc, int m, int n, int k,
                                 void* stream) {
-  OGL_TRY(require_device());
-  OGL_ARG(a_dev && b_dev && c_dev && m > 0 && n > 0 && k > 0, "ogl_gemm_bf16_nt: bad arguments");
-  GemmNT g;
-  g.a[0] = a_dev; g.lda[0] = lda; g.b[0] = b_dev; g.ldb[0] = ldb; g.k[0] = k; g.n_seg = 1;
-  g.c = c_dev; g.ldc = ldc; g.m_max = m; g.n = n; g.in_bf16 = 1; g.out_bf16 = 0; g.zero_tail = 0;
-  return gemm_nt_tc(g, (cudaStream_t)stream);
+  return entry_nt("ogl_gemm_bf16_nt", OGL_BF16, a_dev, lda, b_dev, ldb, c_dev, ldc, m, n, k, 1, nullptr, 0, nullptr, 0, 0, stream);
 }
 
 extern "C" int ogl_gemm_bf16_nt_ex(const void* a_dev, int lda, const void* b_dev, int ldb, void* c_dev, int ldc, int m, int n, int k,
                                    int out_bf16, const float* bias_dev, int relu, int cg, void* stream) {
-  OGL_TRY(require_device());
-  OGL_ARG(a_dev && b_dev && c_dev && m > 0 && n > 0 && k > 0, "ogl_gemm_bf16_nt_ex: bad arguments");
-  GemmNT g;
-  g.a[0] = a_dev; g.lda[0] = lda; g.b[0] = b_dev; g.ldb[0] = ldb; g.k[0] = k; g.n_seg = 1;
-  g.c = c_dev; g.ldc = ldc; g.m_max = m; g.n = n; g.in_bf16 = 1; g.out_bf16 = out_bf16; g.zero_tail = 0;
-  g.bias = bias_dev; g.relu = relu; g.force_cg = cg;
-  return gemm_nt_tc(g, (cudaStream_t)stream);
+  return entry_nt("ogl_gemm_bf16_nt_ex", OGL_BF16, a_dev, lda, b_dev, ldb, c_dev, ldc, m, n, k, !out_bf16, bias_dev, relu, nullptr, 0, cg,
+                  stream);
 }
 
 extern "C" int ogl_gemm_bf16_tn(const void* a_dev, int lda, const void* b_dev, int ldb, float* c_dev, int ldc, int m, int n, int k,
                                 float* workspace_dev, int64_t workspace_elems, void* stream) {
-  OGL_TRY(require_device());
-  OGL_ARG(a_dev && b_dev && c_dev && m > 0 && n > 0 && k > 0, "ogl_gemm_bf16_tn: bad arguments");
-  GemmTN g;
-  g.a = a_dev; g.lda = lda; g.b = b_dev; g.ldb = ldb; g.c = c_dev; g.ldc = ldc; g.n = n; g.k = k; g.m_max = m; g.in_bf16 = 1;
-  g.partial = workspace_dev; g.partial_elems = workspace_dev ? workspace_elems : 0;
-  return gemm_tn_tc(g, (cudaStream_t)stream);
+  return entry_tn("ogl_gemm_bf16_tn", OGL_BF16, a_dev, lda, b_dev, ldb, c_dev, ldc, m, n, k, 1.f, workspace_dev, workspace_elems, stream);
 }
 
 // tf32 flavour of the two entry points above (fp32 operands that hold TF32-rounded values; tests / bench)
 extern "C" int ogl_gemm_tf32_nt_ex(const float* a_dev, int lda, const float* b_dev, int ldb, float* c_dev, int ldc, int m, int n, int k,
                                    int tma_out, const float* bias_dev, int relu, const float* mask_dev, int ldmask, int cg, void* stream) {
-  OGL_TRY(require_device());
-  OGL_ARG(a_dev && b_dev && c_dev && m > 0 && n > 0 && k > 0, "ogl_gemm_tf32_nt_ex: bad arguments");
-  GemmNT g;
-  g.a[0] = a_dev; g.lda[0] = lda; g.b[0] = b_dev; g.ldb[0] = ldb; g.k[0] = k; g.n_seg = 1;
-  g.c = c_dev; g.ldc = ldc; g.m_max = m; g.n = n; g.tf32 = 1; g.out_tf32 = tma_out; g.zero_tail = 0;
-  g.bias = bias_dev; g.relu = relu; g.force_cg = cg; g.mask = mask_dev; g.ldmask = ldmask;
-  return gemm_nt_tc(g, (cudaStream_t)stream);
+  return entry_nt("ogl_gemm_tf32_nt_ex", OGL_TF32, a_dev, lda, b_dev, ldb, c_dev, ldc, m, n, k, !tma_out, bias_dev, relu, mask_dev, ldmask,
+                  cg, stream);
 }
 
 extern "C" int ogl_gemm_tf32_tn(const float* a_dev, int lda, const float* b_dev, int ldb, float* c_dev, int ldc, int m, int n, int k,
                                 float* workspace_dev, int64_t workspace_elems, void* stream) {
-  OGL_TRY(require_device());
-  OGL_ARG(a_dev && b_dev && c_dev && m > 0 && n > 0 && k > 0, "ogl_gemm_tf32_tn: bad arguments");
-  GemmTN g;
-  g.a = a_dev; g.lda = lda; g.b = b_dev; g.ldb = ldb; g.c = c_dev; g.ldc = ldc; g.n = n; g.k = k; g.m_max = m; g.tf32 = 1;
-  g.partial = workspace_dev; g.partial_elems = workspace_dev ? workspace_elems : 0;
-  return gemm_tn_tc(g, (cudaStream_t)stream);
+  return entry_tn("ogl_gemm_tf32_tn", OGL_TF32, a_dev, lda, b_dev, ldb, c_dev, ldc, m, n, k, 1.f, workspace_dev, workspace_elems, stream);
 }
 
 // fp16 flavour (mode OGL_FP16: tcgen05 kind::f16 with fp16 operands; tests / bench).  mask (fp16, [m, ldmask]): out = mask > 0 ? out : 0;
 // alpha scales the weight-gradient output (the plan passes 1 / loss scale there)
 extern "C" int ogl_gemm_f16_nt_ex(const void* a_dev, int lda, const void* b_dev, int ldb, void* c_dev, int ldc, int m, int n, int k,
                                   int out_f16, const float* bias_dev, int relu, const void* mask_dev, int ldmask, int cg, void* stream) {
-  OGL_TRY(require_device());
-  OGL_ARG(a_dev && b_dev && c_dev && m > 0 && n > 0 && k > 0, "ogl_gemm_f16_nt_ex: bad arguments");
-  GemmNT g;
-  g.a[0] = a_dev; g.lda[0] = lda; g.b[0] = b_dev; g.ldb[0] = ldb; g.k[0] = k; g.n_seg = 1;
-  g.c = c_dev; g.ldc = ldc; g.m_max = m; g.n = n; g.in_bf16 = 1; g.f16 = 1; g.out_bf16 = out_f16; g.zero_tail = 0;
-  g.bias = bias_dev; g.relu = relu; g.force_cg = cg; g.mask = mask_dev; g.ldmask = ldmask;
-  return gemm_nt_tc(g, (cudaStream_t)stream);
+  return entry_nt("ogl_gemm_f16_nt_ex", OGL_FP16, a_dev, lda, b_dev, ldb, c_dev, ldc, m, n, k, !out_f16, bias_dev, relu, mask_dev, ldmask,
+                  cg, stream);
 }
 
 extern "C" int ogl_gemm_f16_tn(const void* a_dev, int lda, const void* b_dev, int ldb, float* c_dev, int ldc, int m, int n, int k,
                                float alpha, float* workspace_dev, int64_t workspace_elems, void* stream) {
-  OGL_TRY(require_device());
-  OGL_ARG(a_dev && b_dev && c_dev && m > 0 && n > 0 && k > 0, "ogl_gemm_f16_tn: bad arguments");
-  GemmTN g;
-  g.a = a_dev; g.lda = lda; g.b = b_dev; g.ldb = ldb; g.c = c_dev; g.ldc = ldc; g.n = n; g.k = k; g.m_max = m; g.in_bf16 = 1; g.f16 = 1;
-  g.alpha = alpha;
-  g.partial = workspace_dev; g.partial_elems = workspace_dev ? workspace_elems : 0;
-  return gemm_tn_tc(g, (cudaStream_t)stream);
+  return entry_tn("ogl_gemm_f16_tn", OGL_FP16, a_dev, lda, b_dev, ldb, c_dev, ldc, m, n, k, alpha, workspace_dev, workspace_elems, stream);
 }

@@ -280,14 +280,8 @@ int peer_sum_adam(ogl_peer* p, const PeerAdamArgs& a, int64_t lo, int64_t hi, cu
   int grid = (int)ceil_div(quads, 256);
   if (grid > 2 * sm_count()) grid = 2 * sm_count();
   if (grid < 1) grid = 1;
-#define OGL_PEER_LAUNCH(T)                                                                                                          \
-  OGL_LAUNCH((k_peer_sum_adam<T>), grid, 256, 0, s, p->view, lo, hi, a.params, a.m, a.v, a.lr, a.b1, a.b2, a.eps, a.t_dev, \
-             a.segs, a.n_segs, a.reduced_out)
-  if (a.mode == OGL_BF16) OGL_PEER_LAUNCH(__nv_bfloat16);
-  else if (a.mode == OGL_FP16) OGL_PEER_LAUNCH(__half);
-  else if (a.mode == OGL_TF32) OGL_PEER_LAUNCH(tf32_t);
-  else OGL_PEER_LAUNCH(float);
-#undef OGL_PEER_LAUNCH
+  OGL_MODE_DISPATCH(a.mode, OGL_LAUNCH((k_peer_sum_adam<T>), grid, 256, 0, s, p->view, lo, hi, a.params, a.m, a.v, a.lr, a.b1, a.b2, a.eps,
+                                       a.t_dev, a.segs, a.n_segs, a.reduced_out));
   return OGL_OK;
 }
 

@@ -31,11 +31,10 @@ struct ogl_features {
 
 extern "C" int ogl_features_create(ogl_features** out, int64_t v_cap, int n_feats, int mode) {
   OGL_TRY(require_device());
-  OGL_ARG(out && v_cap > 0 && n_feats > 0 && (mode == OGL_F32 || mode == OGL_BF16 || mode == OGL_TF32 || mode == OGL_FP16),
-          "ogl_features_create: bad arguments");
+  OGL_ARG(out && v_cap > 0 && n_feats > 0 && mode_valid(mode), "ogl_features_create: bad arguments");
   ogl_features* f = new ogl_features();
   f->v_cap = v_cap; f->F = n_feats; f->pitch = pitch_of(n_feats); f->mode = mode;
-  const size_t es = mode_is_16bit(mode) ? 2 : 4;
+  const size_t es = mode_bytes(mode);
   OGL_CUDA(cudaMalloc(&f->table, es * (size_t)v_cap * f->pitch));
   OGL_CUDA(cudaMemset(f->table, 0, es * (size_t)v_cap * f->pitch));
   OGL_CUDA(cudaMalloc(&f->labels, sizeof(int32_t) * v_cap));
@@ -113,9 +112,8 @@ struct LayerBuf {
 struct ogl_plan {
   ogl_plan_config cfg;
   int L = 0;
-  int bf16 = 0, tf32 = 0, mode = 0;      // mode = cfg.mode; bf16 = 16-bit storage (OGL_BF16 or OGL_FP16), tf32 = mode == OGL_TF32
-  int fp16 = 0;                          // mode == OGL_FP16: the 16-bit storage is fp16 and activation gradients carry a loss scale
-  size_t es = 4;
+  int mode = 0;                          // = cfg.mode
+  size_t es = 4;                         // its storage type's element bytes
   std::vector<int> nmax;                 // [L+1]
   std::vector<int32_t*> nodes;           // [L+1]
   int32_t* counts = nullptr;             // [L+1] device
@@ -272,21 +270,6 @@ static std::string nm(const char* fmt, int i) {
   return b;
 }
 
-static int gemm_nt(const ogl_plan* p, const GemmNT& g, cudaStream_t s) {
-  if ((p->bf16 || p->tf32) && p->cfg.gemm_impl == 0 && gemm_tc_available()) return gemm_nt_tc(g, s);
-  return gemm_nt_simt(g, s);
-}
-static int gemm_tn(const ogl_plan* p, const GemmTN& g, cudaStream_t s) {
-  if ((p->bf16 || p->tf32) && p->cfg.gemm_impl == 0 && gemm_tc_available()) return gemm_tn_tc(g, s);
-  return gemm_tn_simt(g, s);
-}
-// weight-gradient GEMMs that contract over the same rows: one launch on the tcgen05 path
-static int gemm_tn_group(const ogl_plan* p, const GemmTN* g, int count, cudaStream_t s) {
-  if ((p->bf16 || p->tf32) && p->cfg.gemm_impl == 0 && gemm_tc_available()) return gemm_tn_tc_group(g, count, s);
-  for (int i = 0; i < count; ++i) OGL_TRY(gemm_tn_simt(g[i], s));
-  return OGL_OK;
-}
-
 static int dmalloc0(void** ptr, size_t bytes) {
   OGL_CUDA(cudaMalloc(ptr, bytes ? bytes : 16));
   OGL_CUDA(cudaMemset(*ptr, 0, bytes ? bytes : 16));
@@ -301,7 +284,7 @@ extern "C" int ogl_plan_create(ogl_plan** out, const ogl_plan_config* cfg) {
   OGL_ARG(out && cfg, "ogl_plan_create: null");
   OGL_ARG(cfg->n_layers >= 1 && cfg->n_layers <= 7, "ogl_plan_create: n_layers must be in [1,7]");
   OGL_ARG(cfg->max_seeds > 0 && cfg->v_cap > 0, "ogl_plan_create: max_seeds / v_cap must be positive");
-  OGL_ARG(cfg->mode == OGL_F32 || cfg->mode == OGL_BF16 || cfg->mode == OGL_TF32 || cfg->mode == OGL_FP16, "ogl_plan_create: bad mode");
+  OGL_ARG(mode_valid(cfg->mode), "ogl_plan_create: bad mode");
   OGL_ARG(cfg->feat_drop >= 0.f && cfg->feat_drop < 1.f, "ogl_plan_create: feat_drop must be in [0, 1)");
   for (int i = 0; i <= cfg->n_layers; ++i) OGL_ARG(cfg->dims[i] > 0, "ogl_plan_create: dims[%d] must be positive", i);
   for (int i = 0; i < cfg->n_layers; ++i) OGL_ARG(cfg->fanouts[i] > 0 && cfg->fanouts[i] < 255, "ogl_plan_create: fanouts[%d] must be in [1,254]", i);
@@ -309,10 +292,7 @@ extern "C" int ogl_plan_create(ogl_plan** out, const ogl_plan_config* cfg) {
   p->cfg = *cfg;
   const int L = p->L = cfg->n_layers;
   p->mode = cfg->mode;
-  p->bf16 = mode_is_16bit(cfg->mode);
-  p->fp16 = cfg->mode == OGL_FP16;
-  p->tf32 = cfg->mode == OGL_TF32;
-  p->es = p->bf16 ? 2 : 4;
+  p->es = mode_bytes(cfg->mode);
   p->nmax.resize(L + 1);
   p->nmax[0] = cfg->max_seeds;
   for (int h = 0; h < L; ++h) {
@@ -531,6 +511,29 @@ extern "C" int ogl_plan_sample(ogl_plan* p, ogl_graph* g, const int64_t* seeds_d
   return OGL_OK;
 }
 
+// the forward GEMMs of layer l, shared by the sampled forward and full-neighbourhood inference (m_dev: the dynamic row count, or
+// nullptr for m_max rows).  The pool GEMM: hp = relu(x Wp^T + bp)
+static int pool_gemm(const ogl_plan* p, int l, const void* x, int ldx, void* hp, int ldhp, int m_max, const int32_t* m_dev, cudaStream_t s) {
+  const LayerBuf& lb = p->layer[l];
+  GemmNT g;
+  g.a[0] = x; g.lda[0] = ldx; g.b[0] = lb.wp; g.ldb[0] = lb.pin; g.k[0] = lb.in; g.n_seg = 1;
+  g.bias = p->params + lb.o_bp; g.relu = 1;
+  g.c = hp; g.ldc = ldhp; g.m_max = m_max; g.m_dev = m_dev; g.n = lb.in; g.mode = p->mode;
+  return gemm_nt(g, p->cfg.gemm_impl, s);
+}
+// the output GEMM: [h_self | neigh] [Ws | Wn]^T + bs + bn, with ReLU and in the storage type for a hidden layer, fp32 logits for the last
+static int out_gemm(const ogl_plan* p, int l, const void* self, int ld_self, const void* neigh, int ld_neigh, void* out, int ldo, int m_max,
+                    const int32_t* m_dev, cudaStream_t s) {
+  const LayerBuf& lb = p->layer[l];
+  const bool last = l == p->L - 1;
+  GemmNT g;
+  g.a[0] = self; g.lda[0] = ld_self; g.b[0] = lb.ws; g.ldb[0] = lb.pin; g.k[0] = lb.in;
+  g.a[1] = neigh; g.lda[1] = ld_neigh; g.b[1] = lb.wn; g.ldb[1] = lb.pin; g.k[1] = lb.in; g.n_seg = 2;
+  g.bias = p->params + lb.o_bs; g.bias2 = p->params + lb.o_bn; g.relu = !last;
+  g.c = out; g.ldc = ldo; g.m_max = m_max; g.m_dev = m_dev; g.n = lb.out; g.mode = p->mode; g.out_f32 = last;
+  return gemm_nt(g, p->cfg.gemm_impl, s);
+}
+
 // drop_step: the device word that keys feat_drop's mask (the last Philox counter word).  A fused step passes its optimiser step
 // ctl[1]; a direct ogl_plan_forward passes ctl[3], see there.
 static int plan_forward(ogl_plan* p, ogl_features* f, float* logits_dev, const uint32_t* drop_step, cudaStream_t s) {
@@ -549,21 +552,12 @@ static int plan_forward(ogl_plan* p, ogl_features* f, float* logits_dev, const u
     if (drop)
       STAGE(nm("l%d.feat_drop", l).c_str(), feat_drop(p->mode, p->act[sl], lb.pin, lb.in, p->counts + sl, p->nmax[sl], p->cfg.feat_drop,
                                                       p->cfg.seed, drop_step, l, s));
-    GemmNT g1;
-    g1.a[0] = p->act[sl]; g1.lda[0] = lb.pin; g1.b[0] = lb.wp; g1.ldb[0] = lb.pin; g1.k[0] = lb.in; g1.n_seg = 1;
-    g1.bias = p->params + lb.o_bp; g1.relu = 1;
-    g1.c = lb.hp; g1.ldc = lb.pin; g1.m_max = p->nmax[sl]; g1.m_dev = p->counts + sl; g1.n = lb.in;
-    g1.in_bf16 = p->bf16; g1.out_bf16 = p->bf16; g1.f16 = p->fp16; g1.tf32 = p->tf32; g1.out_tf32 = p->tf32;
-    STAGE(nm("l%d.pool_gemm", l).c_str(), gemm_nt(p, g1, s));
+    STAGE(nm("l%d.pool_gemm", l).c_str(), pool_gemm(p, l, p->act[sl], lb.pin, lb.hp, lb.pin, p->nmax[sl], p->counts + sl, s));
     STAGE(nm("l%d.segmax", l).c_str(),
           segmax_fwd(p->mode, lb.hp, lb.pin, p->edge_lid[h], p->cfg.fanouts[h], p->counts + dl, p->nmax[dl], lb.neigh, lb.arg, s));
-    GemmNT g2;
-    g2.a[0] = p->act[sl]; g2.lda[0] = lb.pin; g2.b[0] = lb.ws; g2.ldb[0] = lb.pin; g2.k[0] = lb.in;
-    g2.a[1] = lb.neigh; g2.lda[1] = lb.pin; g2.b[1] = lb.wn; g2.ldb[1] = lb.pin; g2.k[1] = lb.in; g2.n_seg = 2;
-    g2.bias = p->params + lb.o_bs; g2.bias2 = p->params + lb.o_bn; g2.relu = (l < L - 1);
-    g2.c = p->act[dl]; g2.ldc = lb.pout; g2.m_max = p->nmax[dl]; g2.m_dev = p->counts + dl; g2.n = lb.out;
-    g2.in_bf16 = p->bf16; g2.out_bf16 = (l < L - 1) ? p->bf16 : 0; g2.f16 = p->fp16; g2.tf32 = p->tf32; g2.out_tf32 = (l < L - 1) ? p->tf32 : 0;
-    STAGE(nm("l%d.out_gemm", l).c_str(), gemm_nt(p, g2, s));
+    // (the destination rows are the first rows of the source level)
+    STAGE(nm("l%d.out_gemm", l).c_str(),
+          out_gemm(p, l, p->act[sl], lb.pin, lb.neigh, lb.pin, p->act[dl], lb.pout, p->nmax[dl], p->counts + dl, s));
   }
   if (logits_dev)
     OGL_TRY(unpad_copy((const float*)p->act[0], p->layer[L - 1].pout, p->nmax[0], p->counts, p->cfg.dims[L], logits_dev, s));
@@ -594,7 +588,7 @@ extern "C" float ogl_fp16_grad_scale(float loss_scale) {
   frexpf(64.f / a, &e);                 // 64 / a = m * 2^e, m in [0.5, 1)
   return ldexpf(1.f, e - 1);            // 2^floor(log2(64 / a)):  a * gs in (32, 64]
 }
-static float grad_scale_for(const ogl_plan* p, float loss_scale) { return p->fp16 ? ogl_fp16_grad_scale(loss_scale) : 1.f; }
+static float grad_scale_for(const ogl_plan* p, float loss_scale) { return p->mode == OGL_FP16 ? ogl_fp16_grad_scale(loss_scale) : 1.f; }
 
 static int plan_loss(ogl_plan* p, ogl_features* f, float scale, int want_grad, float* per_vertex_loss_dev, float* loss_sum_dev, cudaStream_t s) {
   const int L = p->L;
@@ -630,13 +624,13 @@ static int plan_backward_layers(ogl_plan* p, cudaStream_t s) {
     const int sl = L - l;
     GemmTN tp;
     tp.a = lb.dhp; tp.lda = lb.pin; tp.n = lb.in; tp.b = p->act[sl]; tp.ldb = lb.pin; tp.k = lb.in;
-    tp.c = p->grads + lb.o_wp; tp.ldc = lb.in; tp.m_max = p->nmax[sl]; tp.m_dev = p->counts + sl; tp.in_bf16 = p->bf16; tp.f16 = p->fp16; tp.tf32 = p->tf32;
+    tp.c = p->grads + lb.o_wp; tp.ldc = lb.in; tp.m_max = p->nmax[sl]; tp.m_dev = p->counts + sl; tp.mode = p->mode;
     tp.alpha = 1.f / p->grad_scale;
     tp.partial = p->tn_partial; tp.partial_elems = p->tn_partial_elems;
     return tp;
   };
   if (p->tail_mode == 2) {                        // only dWp of layer 0 (its dhp was left in place by the tail_mode 1 pass)
-    STAGE("l0.dW_pool", gemm_tn(p, dw_pool(0), s));
+    STAGE("l0.dW_pool", gemm_tn(dw_pool(0), p->cfg.gemm_impl, s));
     return OGL_OK;
   }
   OGL_TRY(join_side(p, s));                      // reverse edge lists built on the side stream during sampling
@@ -658,13 +652,13 @@ static int plan_backward_layers(ogl_plan* p, cudaStream_t s) {
     if (l + 1 < L) grp[ng++] = dw_pool(l + 1);
     GemmTN t;
     t.a = lb.dpre; t.lda = lb.pout; t.n = lb.out; t.b = p->act[sl]; t.ldb = lb.pin; t.k = lb.in;
-    t.c = G + lb.o_ws; t.ldc = lb.in; t.m_max = p->nmax[dl]; t.m_dev = p->counts + dl; t.in_bf16 = p->bf16; t.f16 = p->fp16; t.tf32 = p->tf32;
+    t.c = G + lb.o_ws; t.ldc = lb.in; t.m_max = p->nmax[dl]; t.m_dev = p->counts + dl; t.mode = p->mode;
     t.alpha = 1.f / p->grad_scale;
     grp[ng++] = t;
     t.b = lb.neigh; t.c = G + lb.o_wn;
     grp[ng++] = t;
     for (int i = 0; i < ng; ++i) { grp[i].partial = ov ? p->tn_partial2 : p->tn_partial; grp[i].partial_elems = p->tn_partial_elems; }
-    STAGE_ON(ss, nm("l%d.dW_group", l).c_str(), gemm_tn_group(p, grp, ng, ss));
+    STAGE_ON(ss, nm("l%d.dW_group", l).c_str(), gemm_tn_group(grp, ng, p->cfg.gemm_impl, ss));
     STAGE_ON(ss, nm("l%d.db_out", l).c_str(), colsum(p->mode, lb.dpre, lb.pout, lb.out, p->counts + dl, p->nmax[dl],
                                                      ov ? p->colsum_partial2 : p->colsum_partial, G + lb.o_bs, G + lb.o_bn, ss,
                                                      1.f / p->grad_scale));
@@ -672,9 +666,9 @@ static int plan_backward_layers(ogl_plan* p, cudaStream_t s) {
     GemmNT n1;
     n1.a[0] = lb.dpre; n1.lda[0] = lb.pout; n1.b[0] = lb.wnT; n1.ldb[0] = lb.pout; n1.k[0] = lb.out; n1.n_seg = 1;
     n1.c = lb.dng; n1.ldc = lb.pin; n1.m_max = p->nmax[dl]; n1.m_dev = p->counts + dl; n1.n = lb.in;
-    n1.in_bf16 = p->bf16; n1.out_bf16 = p->bf16; n1.f16 = p->fp16; n1.tf32 = p->tf32; n1.out_tf32 = p->tf32; n1.zero_tail = 0;
+    n1.mode = p->mode; n1.zero_tail = 0;
     n1.mask = lb.neigh; n1.ldmask = lb.pin;        // relu'(hp) at the argmax: neigh[d, f] == hp[src(arg), f]
-    STAGE(nm("l%d.dneigh_gemm", l).c_str(), gemm_nt(p, n1, s));
+    STAGE(nm("l%d.dneigh_gemm", l).c_str(), gemm_nt(n1, p->cfg.gemm_impl, s));
     // fc_pool bias gradient: every dng[d, f] lands in exactly one source row, so colsum(dhp) == colsum(dng).  Side stream too (behind the
     // weight-gradient group): only Adam reads it
     if (ov) {
@@ -689,7 +683,7 @@ static int plan_backward_layers(ogl_plan* p, cudaStream_t s) {
                                                   p->counts + sl, p->nmax[sl], lb.dhp, s));
     // dWp = dhp^T act[src]: layer 0 computes it here (the step's last and largest weight gradient; data-parallel runs peel it off
     // as the second gradient bucket); the layers above hold it back for the next grouped launch
-    if (l == 0 && p->tail_mode != 1) STAGE("l0.dW_pool", gemm_tn(p, dw_pool(0), s));
+    if (l == 0 && p->tail_mode != 1) STAGE("l0.dW_pool", gemm_tn(dw_pool(0), p->cfg.gemm_impl, s));
     if (l > 0) {
       // dpre[l-1] = relu'(act[src]) * ( dhp Wp + [dpre Ws on the first n_d rows] )
       LayerBuf& prev = p->layer[l - 1];
@@ -701,8 +695,8 @@ static int plan_backward_layers(ogl_plan* p, cudaStream_t s) {
       d.mask = p->act[sl]; d.ldmask = lb.pin;      // (after feat_drop a dropped element is 0 as well: relu' and the keep mask in one)
       if (p->train_mode && p->cfg.feat_drop > 0.f) d.alpha = 1.f / (1.f - p->cfg.feat_drop);
       d.c = prev.dpre; d.ldc = prev.pout; d.m_max = p->nmax[sl]; d.m_dev = p->counts + sl; d.n = lb.in;
-      d.in_bf16 = p->bf16; d.out_bf16 = p->bf16; d.f16 = p->fp16; d.tf32 = p->tf32; d.out_tf32 = p->tf32;
-      STAGE(nm("l%d.dx_gemm", l).c_str(), gemm_nt(p, d, s));
+      d.mode = p->mode;
+      STAGE(nm("l%d.dx_gemm", l).c_str(), gemm_nt(d, p->cfg.gemm_impl, s));
     }
   }
   if (p->use_side && !p->prof_on) {                                   // join: the side-stream gradients precede Adam / the caller
@@ -1256,12 +1250,7 @@ static int full_layer(ogl_plan* p, const GraphView& gv, int64_t E, const ogl_fea
     h = f->table;
     ldh = f->pitch;
   }
-  GemmNT g1;
-  g1.a[0] = h; g1.lda[0] = ldh; g1.b[0] = lb.wp; g1.ldb[0] = lb.pin; g1.k[0] = lb.in; g1.n_seg = 1;
-  g1.bias = p->params + lb.o_bp; g1.relu = 1;
-  g1.c = w.hp; g1.ldc = lb.pin; g1.m_max = (int)gv.n_vertices; g1.n = lb.in;
-  g1.in_bf16 = p->bf16; g1.out_bf16 = p->bf16; g1.f16 = p->fp16; g1.tf32 = p->tf32; g1.out_tf32 = p->tf32;
-  STAGE(nm("full.l%d.pool_gemm", l).c_str(), gemm_nt(p, g1, s));
+  STAGE(nm("full.l%d.pool_gemm", l).c_str(), pool_gemm(p, l, h, ldh, w.hp, lb.pin, (int)gv.n_vertices, nullptr, s));
   STAGE(nm("full.l%d.segmax", l).c_str(), csr_segmax(p->mode, gv, E, w.hp, lb.pin, lb.in, rows32, nullptr, row0, m, w.neigh, lb.pin,
                                                      &w.sm, s));
   const int mp = round_up(m, 128);
@@ -1273,14 +1262,9 @@ static int full_layer(ogl_plan* p, const GraphView& gv, int64_t E, const ogl_fea
     self = w.hs;
   }
   OGL_ARG(((uintptr_t)self & 15) == 0, "full inference: the self rows of layer %d start off the 16-byte grid", l);
-  GemmNT g2;
-  g2.a[0] = self; g2.lda[0] = ldh; g2.b[0] = lb.ws; g2.ldb[0] = lb.pin; g2.k[0] = lb.in;
-  g2.a[1] = w.neigh; g2.lda[1] = lb.pin; g2.b[1] = lb.wn; g2.ldb[1] = lb.pin; g2.k[1] = lb.in; g2.n_seg = 2;
-  g2.bias = p->params + lb.o_bs; g2.bias2 = p->params + lb.o_bn; g2.relu = !last;
   // (the logits go through the plan's padded buffer: the GEMM writes rows of a multiple of 8 columns)
-  g2.c = last ? (void*)w.logits : out; g2.ldc = last ? lb.pout : ldo; g2.m_max = m; g2.n = lb.out;
-  g2.in_bf16 = p->bf16; g2.out_bf16 = last ? 0 : p->bf16; g2.f16 = p->fp16; g2.tf32 = p->tf32; g2.out_tf32 = last ? 0 : p->tf32;
-  STAGE(nm("full.l%d.out_gemm", l).c_str(), gemm_nt(p, g2, s));
+  STAGE(nm("full.l%d.out_gemm", l).c_str(), out_gemm(p, l, self, ldh, w.neigh, lb.pin, last ? (void*)w.logits : out, last ? lb.pout : ldo, m,
+                                                    nullptr, s));
   if (last && out != (void*)w.logits)
     OGL_CUDA(cudaMemcpy2DAsync(out, sizeof(float) * ldo, w.logits, sizeof(float) * lb.pout, sizeof(float) * lb.out, n,
                                cudaMemcpyDeviceToDevice, s));

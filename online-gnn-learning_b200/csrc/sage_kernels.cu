@@ -461,28 +461,12 @@ __global__ void __launch_bounds__(kBlock) k_unpad_copy(const float* __restrict__
 
 // ================================ host wrappers ====================================================
 // mode: OGL_F32 (exact fp32), OGL_BF16, OGL_FP16, OGL_TF32 (fp32 storage, values rounded to TF32 where a GEMM operand is produced)
-#define L2(K, grid, s, ...)                                                                      \
-  do {                                                                                           \
-    if (mode == OGL_BF16) OGL_LAUNCH((K<__nv_bfloat16>), grid, kBlock, 0, s, __VA_ARGS__);       \
-    else if (mode == OGL_FP16) OGL_LAUNCH((K<__half>), grid, kBlock, 0, s, __VA_ARGS__);         \
-    else if (mode == OGL_TF32) OGL_LAUNCH((K<tf32_t>), grid, kBlock, 0, s, __VA_ARGS__);         \
-    else OGL_LAUNCH((K<float>), grid, kBlock, 0, s, __VA_ARGS__);                                \
-  } while (0)
-// the same with typed views of the void* arguments (T names the element type inside CALL)
-#define L2T(K, grid, s, CALL)                                                                    \
-  do {                                                                                           \
-    if (mode == OGL_BF16) { using T = __nv_bfloat16; OGL_LAUNCH((K<T>), grid, kBlock, 0, s, CALL); } \
-    else if (mode == OGL_FP16) { using T = __half; OGL_LAUNCH((K<T>), grid, kBlock, 0, s, CALL); }   \
-    else if (mode == OGL_TF32) { using T = tf32_t; OGL_LAUNCH((K<T>), grid, kBlock, 0, s, CALL); }   \
-    else { using T = float; OGL_LAUNCH((K<T>), grid, kBlock, 0, s, CALL); }                      \
-  } while (0)
-#define ARGS(...) __VA_ARGS__
 
 int feat_write(int mode, const float* src, const int64_t* src_rows, int64_t n, int F, void* dst, int pitch, int64_t row0, cudaStream_t s,
                float scale) {
   if (n <= 0) return OGL_OK;
   const int grid = grid_for(n * 32, kBlock);
-  L2T(k_feat_write, grid, s, ARGS(src, src_rows, n, F, (T*)dst, pitch, row0, scale));
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_feat_write<T>), grid, kBlock, 0, s, src, src_rows, n, F, (T*)dst, pitch, row0, scale));
   return OGL_OK;
 }
 int label_write(const int64_t* src, const int64_t* src_rows, int64_t n, int32_t* dst, int64_t row0, cudaStream_t s) {
@@ -492,13 +476,13 @@ int label_write(const int64_t* src, const int64_t* src_rows, int64_t n, int32_t*
 }
 int gather_rows(int mode, const void* table, int pitch, const int32_t* nodes, const int32_t* n_dev, int n_max, void* out, cudaStream_t s) {
   const int grid = grid_for((int64_t)n_max * pitch / 8, kBlock, 16);
-  L2T(k_gather_rows, grid, s, ARGS((const T*)table, pitch, nodes, n_dev, n_max, (T*)out));
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_gather_rows<T>), grid, kBlock, 0, s, (const T*)table, pitch, nodes, n_dev, n_max, (T*)out));
   return OGL_OK;
 }
 int scatter_rows(int mode, const void* rows, int pitch, const int32_t* nodes, int n, void* table, cudaStream_t s) {
   if (n <= 0) return OGL_OK;
   const int grid = grid_for((int64_t)n * pitch / 8, kBlock, 16);
-  L2T(k_scatter_rows, grid, s, ARGS((const T*)rows, pitch, nodes, n, (T*)table));
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_scatter_rows<T>), grid, kBlock, 0, s, (const T*)rows, pitch, nodes, n, (T*)table));
   return OGL_OK;
 }
 int feat_drop(int mode, void* x, int pitch, int cols, const int32_t* n_dev, int n_max, float p, uint64_t seed, const uint32_t* step_dev,
@@ -509,33 +493,37 @@ int feat_drop(int mode, void* x, int pitch, int cols, const int32_t* n_dev, int 
   const float scale = 1.f / (1.f - p);
   const uint2 key = make_uint2((uint32_t)(seed & 0xffffffffu), (uint32_t)(seed >> 32));
   const int grid = grid_for((int64_t)n_max * ((cols + 3) / 4), kBlock, 16);
-  L2T(k_feat_drop, grid, s, ARGS((T*)x, pitch, cols, n_dev, n_max, thresh, scale, key, step_dev, (uint32_t)layer));
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_feat_drop<T>), grid, kBlock, 0, s, (T*)x, pitch, cols, n_dev, n_max, thresh, scale, key, step_dev,
+                                     (uint32_t)layer));
   return OGL_OK;
 }
 int segmax_fwd(int mode, const void* hp, int pitch, const int32_t* edge_lid, int fanout, const int32_t* n_dst_dev, int n_dst_max, void* ng,
                uint8_t* arg, cudaStream_t s) {
   const int grid = grid_for((int64_t)n_dst_max * pitch / 8, kBlock, 16);
-  L2T(k_segmax_fwd, grid, s, ARGS((const T*)hp, pitch, edge_lid, fanout, n_dst_dev, n_dst_max, (T*)ng, arg));
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_segmax_fwd<T>), grid, kBlock, 0, s, (const T*)hp, pitch, edge_lid, fanout, n_dst_dev, n_dst_max,
+                                     (T*)ng, arg));
   return OGL_OK;
 }
 int pool_bwd(int mode, const void* dng, int pitch, const uint8_t* arg, const int32_t* rev_ptr, const int32_t* rev_edge, int fanout,
              const int32_t* n_src_dev, int n_src_max, void* dhp, cudaStream_t s) {
   const int grid = grid_for((int64_t)round_up(n_src_max, 128) * pitch / mode_vec(mode), kBlock, 32);
-  L2T(k_pool_bwd, grid, s, ARGS((const T*)dng, pitch, arg, rev_ptr, rev_edge, fanout, n_src_dev, n_src_max, (T*)dhp));
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_pool_bwd<T>), grid, kBlock, 0, s, (const T*)dng, pitch, arg, rev_ptr, rev_edge, fanout, n_src_dev,
+                                     n_src_max, (T*)dhp));
   return OGL_OK;
 }
 int64_t colsum_partial_elems(int n_max, int cols) { return ceil_div(n_max, kColRows) * (int64_t)cols; }
 int colsum(int mode, const void* x, int pitch, int cols, const int32_t* n_dev, int n_max, float* partial, float* out, float* out2, cudaStream_t s,
            float alpha) {
   dim3 grid((unsigned)ceil_div(pitch / mode_vec(mode), 32), (unsigned)ceil_div(n_max, kColRows));
-  L2T(k_colsum_partial, grid, s, ARGS((const T*)x, pitch, cols, n_dev, n_max, partial));
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_colsum_partial<T>), grid, kBlock, 0, s, (const T*)x, pitch, cols, n_dev, n_max, partial));
   OGL_LAUNCH(k_colsum_final, (unsigned)ceil_div(cols, 32), 1024, 0, s, partial, cols, n_dev, n_max, out, out2, alpha);
   return OGL_OK;
 }
 int xent(int mode, const float* logits, int ldl, int C, const int32_t* labels, const int32_t* nodes, const int32_t* n_dev, int n_max,
          int rows_buf, float scale, float* per_loss, void* dlogits, int ldd, int want_grad, cudaStream_t s) {
   const int grid = grid_for((int64_t)(rows_buf > n_max ? rows_buf : n_max) * 32, kBlock);
-  L2T(k_xent, grid, s, ARGS(logits, ldl, C, labels, nodes, n_dev, n_max, rows_buf, scale, per_loss, (T*)dlogits, ldd, want_grad));
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_xent<T>), grid, kBlock, 0, s, logits, ldl, C, labels, nodes, n_dev, n_max, rows_buf, scale, per_loss,
+                                     (T*)dlogits, ldd, want_grad));
   return OGL_OK;
 }
 int sum_f32(const float* x, const int32_t* n_dev, int n_max, float* out, cudaStream_t s) {
@@ -551,7 +539,8 @@ int adam_shadow(int mode, float* p, const float* g, float* m, float* v, int64_t 
   OGL_ARG(n_segs <= 48, "adam_shadow: too many weight segments");
   OGL_ARG(lo >= 0 && hi > lo, "adam_shadow: empty range");
   const int grid = grid_for(hi - lo, kBlock);
-  L2(k_adam_shadow, grid, s, p, g, m, v, lo, hi, lr, b1, b2, eps, t_dev, segs_dev, n_segs);
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_adam_shadow<T>), grid, kBlock, 0, s, p, g, m, v, lo, hi, lr, b1, b2, eps, t_dev, segs_dev,
+                                     n_segs));
   return OGL_OK;
 }
 int bump(uint32_t* a, uint32_t* b, cudaStream_t s) {
@@ -560,7 +549,7 @@ int bump(uint32_t* a, uint32_t* b, cudaStream_t s) {
 }
 int weight_shadow(int mode, const float* w, int out, int in, void* ws, int pitch_in, void* wt, int pitch_out, cudaStream_t s) {
   const int grid = grid_for((int64_t)out * pitch_in, kBlock);
-  L2T(k_weight_shadow, grid, s, ARGS(w, out, in, (T*)ws, pitch_in, (T*)wt, pitch_out));
+  OGL_MODE_DISPATCH(mode, OGL_LAUNCH((k_weight_shadow<T>), grid, kBlock, 0, s, w, out, in, (T*)ws, pitch_in, (T*)wt, pitch_out));
   return OGL_OK;
 }
 int unpad_copy(const float* src, int lds, int n_rows_max, const int32_t* n_dev, int cols, float* dst, cudaStream_t s) {
