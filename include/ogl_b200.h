@@ -381,6 +381,27 @@ int ogl_gemm_f16_nt_ex(const void* a_dev, int lda, const void* b_dev, int ldb, v
                        int out_f16, const float* bias_dev, int relu, const void* mask_dev, int ldmask, int cg, void* stream);
 int ogl_gemm_f16_tn(const void* a_dev, int lda, const void* b_dev, int ldb, float* c_dev, int ldc,
                     int m, int n, int k, float alpha, float* workspace_dev, int64_t workspace_elems, void* stream);
+/* The train step's GEMM descriptors (csrc/gemm.cuh) field for field, through the dispatcher the plan uses: tcgen05 for the
+ * tensor-core modes unless force_simt != 0, the SIMT kernels for OGL_F32 or when forced.  Operands and outputs are in the storage
+ * type of `mode` (out_f32: fp32 output).  NT: C = act(alpha * sum_s A_s B_s^T + bias + bias2) over up to two contraction segments,
+ * segment s counting only for rows m < *a_rows_dev[s]; cg: 0 auto, 1 one CTA per 128-row tile, 2 CTA pairs */
+typedef struct {
+  const void* a[2]; int lda[2]; const void* b[2]; int ldb[2]; int k[2]; int n_seg;
+  const int32_t* a_rows_dev[2]; int a_rows_max[2];
+  const float* bias; const float* bias2; int relu; float alpha;
+  const void* mask; int ldmask;
+  void* c; int ldc; int m_max; const int32_t* m_dev; int n;
+  int mode; int out_f32; int zero_tail; int cg;
+} ogl_gemm_nt_desc;
+int ogl_gemm_nt(const ogl_gemm_nt_desc* d, int force_simt, void* stream);
+/* TN: C[n, k] (fp32) = alpha * sum_{m < *m_dev} A[m, :n]^T B[m, :k]; up to 4 problems over the same rows (same m_dev, m_max and
+ * mode) share one launch and the split workspace */
+typedef struct {
+  const void* a; int lda; const void* b; int ldb; float* c; int ldc; int n, k, m_max;
+  const int32_t* m_dev; int mode; float alpha;
+} ogl_gemm_tn_desc;
+int ogl_gemm_tn_group(const ogl_gemm_tn_desc* d, int count, float* workspace_dev, int64_t workspace_elems, int force_simt,
+                      void* stream);
 
 #pragma GCC visibility pop
 #ifdef __cplusplus

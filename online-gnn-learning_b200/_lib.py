@@ -23,6 +23,22 @@ class PlanConfig(C.Structure):
                 ("lr", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float), ("eps", C.c_float), ("feat_drop", C.c_float)]
 
 
+class GemmNTDesc(C.Structure):
+    """ogl_gemm_nt_desc"""
+    _fields_ = [("a", C.c_void_p * 2), ("lda", C.c_int * 2), ("b", C.c_void_p * 2), ("ldb", C.c_int * 2), ("k", C.c_int * 2),
+                ("n_seg", C.c_int), ("a_rows_dev", C.c_void_p * 2), ("a_rows_max", C.c_int * 2),
+                ("bias", C.c_void_p), ("bias2", C.c_void_p), ("relu", C.c_int), ("alpha", C.c_float),
+                ("mask", C.c_void_p), ("ldmask", C.c_int),
+                ("c", C.c_void_p), ("ldc", C.c_int), ("m_max", C.c_int), ("m_dev", C.c_void_p), ("n", C.c_int),
+                ("mode", C.c_int), ("out_f32", C.c_int), ("zero_tail", C.c_int), ("cg", C.c_int)]
+
+
+class GemmTNDesc(C.Structure):
+    """ogl_gemm_tn_desc"""
+    _fields_ = [("a", C.c_void_p), ("lda", C.c_int), ("b", C.c_void_p), ("ldb", C.c_int), ("c", C.c_void_p), ("ldc", C.c_int),
+                ("n", C.c_int), ("k", C.c_int), ("m_max", C.c_int), ("m_dev", C.c_void_p), ("mode", C.c_int), ("alpha", C.c_float)]
+
+
 def _load():
     if not os.path.exists(LIB_PATH):
         raise ImportError(
@@ -128,6 +144,8 @@ SIGNATURES = {
     "ogl_fp16_grad_scale": (_f, [_f]),
     "ogl_gemm_f16_nt_ex": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _i, _vp, _i, _i, _vp]),
     "ogl_gemm_f16_tn": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _f, _vp, _i64, _vp]),
+    "ogl_gemm_nt": (_i, [C.POINTER(GemmNTDesc), _i, _vp]),
+    "ogl_gemm_tn_group": (_i, [C.POINTER(GemmTNDesc), _i, _vp, _i64, _i, _vp]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -4,7 +4,7 @@ import ctypes as C
 import numpy as np
 import torch
 
-from ._lib import lib, check, PlanConfig, OGL_F32, OGL_BF16, OGL_TF32, OGL_FP16, kernel_launches  # noqa: F401
+from ._lib import lib, check, PlanConfig, GemmNTDesc, GemmTNDesc, OGL_F32, OGL_BF16, OGL_TF32, OGL_FP16, kernel_launches  # noqa: F401
 
 
 def _stream():
@@ -717,6 +717,38 @@ def gemm_f16_tn(a, b, n=None, k=None, alpha=1.0, workspace_elems=1 << 24):
     check(lib.ogl_gemm_f16_tn(_ptr(a), a.shape[1], _ptr(b), b.shape[1], _ptr(c), k, a.shape[0], n, k, float(alpha),
                               _ptr(ws), int(workspace_elems), _stream()))
     return c
+
+
+def gemm_nt(c, segs, m_max, n, mode, m_dev=None, bias=None, bias2=None, relu=False, alpha=1.0, mask=None, out_f32=False,
+            zero_tail=True, cg=0, force_simt=False):
+    """the train step's NT descriptor through the GEMM dispatcher (tests): c = act(alpha * sum_s A_s B_s^T + bias + bias2) into the
+    [m_max, ldc] output c.  segs: up to two (a, b, k, a_rows_dev, a_rows_max), a_rows_dev an int32 CUDA scalar tensor or None;
+    m_dev likewise.  Row pitches are the tensors' shape[1]"""
+    d = GemmNTDesc()
+    assert 1 <= len(segs) <= 2
+    for i, (a, b, k, rows_dev, rows_max) in enumerate(segs):
+        d.a[i], d.lda[i], d.b[i], d.ldb[i], d.k[i] = a.data_ptr(), a.shape[1], b.data_ptr(), b.shape[1], int(k)
+        d.a_rows_dev[i], d.a_rows_max[i] = rows_dev.data_ptr() if rows_dev is not None else None, int(rows_max)
+        assert a.is_contiguous() and b.is_contiguous()
+    d.n_seg = len(segs)
+    d.bias, d.bias2 = _ptr(bias), _ptr(bias2)
+    d.relu, d.alpha = int(relu), float(alpha)
+    d.mask, d.ldmask = _ptr(mask), mask.shape[1] if mask is not None else 0
+    d.c, d.ldc, d.m_max, d.m_dev, d.n = _ptr(c), c.shape[1], int(m_max), _ptr(m_dev), int(n)
+    d.mode, d.out_f32, d.zero_tail, d.cg = int(mode), int(out_f32), int(zero_tail), int(cg)
+    check(lib.ogl_gemm_nt(C.byref(d), int(force_simt), _stream()))
+
+
+def gemm_tn_group(problems, m_max, mode, m_dev=None, workspace=None, force_simt=False):
+    """up to 4 weight-gradient descriptors over the same rows through the GEMM dispatcher (tests): c = alpha * A[:m, :n]^T B[:m, :k]
+    with m = min(*m_dev, m_max).  problems: (a, b, c, n, k, alpha) with fp32 outputs c [n, ldc]; workspace: fp32 CUDA tensor or None"""
+    descs = (GemmTNDesc * len(problems))()
+    for d, (a, b, c, n, k, alpha) in zip(descs, problems):
+        assert a.is_contiguous() and b.is_contiguous() and c.is_contiguous() and c.dtype == torch.float32
+        d.a, d.lda, d.b, d.ldb, d.c, d.ldc = a.data_ptr(), a.shape[1], b.data_ptr(), b.shape[1], c.data_ptr(), c.shape[1]
+        d.n, d.k, d.m_max, d.m_dev, d.mode, d.alpha = int(n), int(k), int(m_max), _ptr(m_dev), int(mode), float(alpha)
+    check(lib.ogl_gemm_tn_group(descs, len(problems), _ptr(workspace), workspace.numel() if workspace is not None else 0,
+                                int(force_simt), _stream()))
 
 
 def eval_confusion(logits, labels, n_classes=None):

@@ -9,6 +9,16 @@ namespace ogl {
 // C[m, n] = act( sum_seg sum_k A_seg[m, k] * B_seg[n, k] + bias[n] ) , optional relu / mask.
 // A, B row-major with the contraction index contiguous ("NT").  Up to two (A, B, K) segments
 // accumulate into the same output (used for [h_self | neigh] x [W_self | W_neigh]^T).
+//
+// Rows read: with m = min(*m_dev, m_max) and rv_s = min(*a_rows_dev[s], m), segment s counts for rows m' < rv_s.  Rows
+// [rv_s, round_up(rv_s, 128)) of A_s must be zero (the tile holding row rv_s multiplies them); rows at or past round_up(rv_s, 128)
+// are never read, whatever they hold (a CTA pair whose second 128-row tile lies there loads it as zeros).  Columns >= k of A and
+// B and rows >= n of B are never read either.
+// Rows written: [0, m) the result, [m, round_up(m, 128)) zeros when zero_tail (clamped to m_max).  The tcgen05 epilogues that
+// leave through TMA stores (16-bit outputs, TF32 activations) store whole 128-row tiles, 256-row tiles of a CTA pair: the rows past
+// the zero tail up to round_up(that, 256) may receive zeros as well; rows past that are never written.  Columns [n, ldc) are not
+// part of the result: the tcgen05 epilogues store zeros into those their 32- or 64-column boxes cover (all of them when
+// ldc <= round_up(n, 32)), the SIMT kernel leaves them alone.
 struct GemmNT {
   const void* a[2] = {nullptr, nullptr};   // element type = the mode's storage type
   int lda[2] = {0, 0};
@@ -36,6 +46,8 @@ struct GemmNT {
 };
 
 // C[n, k] = sum_{m < *m_dev} A[m, n] * B[m, k]   (fp32 out; weight gradients)
+// The tcgen05 kernel contracts whole 64-row blocks (32 in mode OGL_TF32): rows [m, round_up(m, 64)) of A must be zero (B may hold
+// any finite values there); rows past round_up(m, 128), columns >= n of A and >= k of B are never read.
 struct GemmTN {
   const void* a = nullptr;   // [m, lda], n contiguous
   int lda = 0;

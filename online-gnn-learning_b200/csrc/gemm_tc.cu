@@ -407,17 +407,21 @@ __global__ void __launch_bounds__(THREADS_NT, 1) k_gemm_nt_tc(const __grid_const
       const int bn_tile = (nb == p.n_tiles - 1) ? ((p.n - nb * BN_MAX + 15) / 16 * 16) : p.bn;
       for (int seg = 0; seg < p.n_seg; ++seg) {
         if (mt * CG * BM >= rows_valid[seg]) continue;          // (pair-uniform: decided on the pair's first row)
+        // pair mode: the second CTA's 128 rows may all lie at or past rows_valid[seg], where the buffer holds whatever an earlier
+        // (longer) use left there -- only [rows_valid, round_up(rows_valid, 128)) is zero.  Its A box then starts above row 0:
+        // TMA fills every element of it with zeros and still completes the full byte count, so the MMA reads zeros
+        const int a_row = mb * BM < rows_valid[seg] ? mb * BM : -BM;
         const int nkb = (p.k[seg] + BKE - 1) / BKE;
         for (int kb = 0; kb < nkb; ++kb) {
           mbar_wait(&s.empty[stage], phase ^ 1);
           if (elect_one()) {
             if (CG == 2) {
               if (rank == 0) mbar_expect_tx(&s.full[stage], tx);
-              if (a_boxes) tma_load_2d_pair(s.a(stage), &p.ta[seg], &s.full[stage], kb * BKE, mb * BM);
+              if (a_boxes) tma_load_2d_pair(s.a(stage), &p.ta[seg], &s.full[stage], kb * BKE, a_row);
               else tma_load_2d_pair(s.b(stage), &p.tb[seg], &s.full[stage], kb * BKE, nb * BN_MAX + rank * (bn_tile / 2));
             } else {
               mbar_expect_tx(&s.full[stage], tx);
-              if (a_boxes) tma_load_2d(s.a(stage), &p.ta[seg], &s.full[stage], kb * BKE, mb * BM);
+              if (a_boxes) tma_load_2d(s.a(stage), &p.ta[seg], &s.full[stage], kb * BKE, a_row);
               else tma_load_2d(s.b(stage), &p.tb[seg], &s.full[stage], kb * BKE, nb * BN_MAX);
             }
           }
@@ -1267,4 +1271,35 @@ extern "C" int ogl_gemm_f16_nt_ex(const void* a_dev, int lda, const void* b_dev,
 extern "C" int ogl_gemm_f16_tn(const void* a_dev, int lda, const void* b_dev, int ldb, float* c_dev, int ldc, int m, int n, int k,
                                float alpha, float* workspace_dev, int64_t workspace_elems, void* stream) {
   return entry_tn("ogl_gemm_f16_tn", OGL_FP16, a_dev, lda, b_dev, ldb, c_dev, ldc, m, n, k, alpha, workspace_dev, workspace_elems, stream);
+}
+
+extern "C" int ogl_gemm_nt(const ogl_gemm_nt_desc* d, int force_simt, void* stream) {
+  OGL_TRY(require_device());
+  OGL_ARG(d && d->c && d->n > 0 && d->m_max > 0 && d->n_seg >= 1 && d->n_seg <= 2, "ogl_gemm_nt: bad arguments");
+  GemmNT g;
+  for (int i = 0; i < d->n_seg; ++i) {
+    OGL_ARG(d->a[i] && d->b[i] && d->k[i] > 0, "ogl_gemm_nt: segment %d: bad operands", i);
+    g.a[i] = d->a[i]; g.lda[i] = d->lda[i]; g.b[i] = d->b[i]; g.ldb[i] = d->ldb[i]; g.k[i] = d->k[i];
+    g.a_rows_dev[i] = d->a_rows_dev[i]; g.a_rows_max[i] = d->a_rows_max[i];
+  }
+  g.n_seg = d->n_seg;
+  g.bias = d->bias; g.bias2 = d->bias2; g.relu = d->relu; g.alpha = d->alpha;
+  g.mask = d->mask; g.ldmask = d->ldmask;
+  g.c = d->c; g.ldc = d->ldc; g.m_max = d->m_max; g.m_dev = d->m_dev; g.n = d->n;
+  g.mode = d->mode; g.out_f32 = d->out_f32; g.zero_tail = d->zero_tail; g.force_cg = d->cg;
+  return gemm_nt(g, force_simt, (cudaStream_t)stream);
+}
+
+extern "C" int ogl_gemm_tn_group(const ogl_gemm_tn_desc* d, int count, float* workspace_dev, int64_t workspace_elems, int force_simt,
+                                 void* stream) {
+  OGL_TRY(require_device());
+  OGL_ARG(d && count >= 1 && count <= kTnGroup, "ogl_gemm_tn_group: 1..%d problems", kTnGroup);
+  GemmTN g[kTnGroup];
+  for (int i = 0; i < count; ++i) {
+    OGL_ARG(d[i].a && d[i].b && d[i].c && d[i].n > 0 && d[i].k > 0 && d[i].m_max > 0, "ogl_gemm_tn_group: problem %d: bad arguments", i);
+    g[i].a = d[i].a; g[i].lda = d[i].lda; g[i].b = d[i].b; g[i].ldb = d[i].ldb; g[i].c = d[i].c; g[i].ldc = d[i].ldc;
+    g[i].n = d[i].n; g[i].k = d[i].k; g[i].m_max = d[i].m_max; g[i].m_dev = d[i].m_dev; g[i].mode = d[i].mode; g[i].alpha = d[i].alpha;
+    g[i].partial = workspace_dev; g[i].partial_elems = workspace_dev ? workspace_elems : 0;
+  }
+  return gemm_tn_group(g, count, force_simt, (cudaStream_t)stream);
 }
