@@ -302,6 +302,47 @@ int ogl_graph_segment_max(ogl_graph* g, int mode, const void* x_dev, int ld, int
 int ogl_graph_in_frontier(ogl_graph* g, const int64_t* rows_dev, int64_t n, int32_t* out_rows_dev, int64_t* out_n,
                           int64_t* out_edge_cost, void* stream);
 
+/* ---- incremental full-neighbourhood inference (inference.StreamingInference): per-vertex tables of the caller's kept current as the
+ * graph grows, a row list at a time, each row with the bits of ogl_plan_infer_full's --------------------------------------------
+ * ogl_graph_out_frontier: the out-neighbourhood frontier of rows_dev[0..n) (device int64; ids outside [0, n_vertices) are ignored):
+ *   out_rows_dev (device int32, capacity n_vertices) receives the distinct vertices of S u N_out(S) -- S and every vertex with an
+ *   in-edge from S -- in ascending order, *out_n their number and *out_edge_cost the sum over them of (in-degree + 1).  The CSR holds
+ *   in-edges only, so this reads every row's adjacency once, in place (O(E) whatever n; an empty list reads nothing).  Synchronises
+ *   `stream` (it frees its scratch before returning).
+ * ogl_graph_segment_max_suffix: in place, for the distinct vertices v = rows_dev[0..n) (device int64; ids outside [0, n_vertices) are
+ *   skipped): acc[v, :cols] = max(acc[v, :cols], max over the in-edges of v at row positions [deg_prev[v], in-degree of v) of
+ *   x[source, :cols]) -- the edges appended to the row since it had deg_prev[v] of them (the edges of a row are kept in insertion
+ *   order).  deg_prev[v] == 0 (or above the in-degree) replaces the row with the max over all its edges (zeros without any).
+ *   deg_prev_dev: device int64 indexed by vertex id; x and acc [*, ld] / [*, ldacc] rows per vertex id in the storage type of `mode`,
+ *   with ogl_graph_segment_max's alignment rules.  The float max of ogl_graph_segment_max: the result has the bits of a whole-row
+ *   max.  A suffix of any length (hub rows) is cut into chunks.  Synchronises `stream`.
+ * ogl_plan_out_frontier: ogl_graph_out_frontier into a device int64 out_rows_dev on the plan's frontier scratch (no allocation after
+ *   the first call), profiled as stage "stream.l<layer>.frontier".  Synchronises `stream` once (the size is read back).
+ * ogl_plan_pool_rows: hp[v] = relu(h[v] Wp^T + bp) of layer `layer` for the vertices v = rows_dev[0..n) (device int64) or, with
+ *   rows_dev == NULL, [row0, row0 + n) (within [0, n_vertices)), written by vertex id into the caller's table hp_dev [*, ldhp] (storage
+ *   type, ldhp = round_up(layer's input width, 8)).  h = f's table for layer 0 (h_dev unused), else h_dev [n_vertices, ldh] as for
+ *   ogl_plan_infer_full_layer.  Out-of-range ids use vertex 0 and raise bit 0 of ogl_plan_error_flags.
+ * ogl_plan_stream_rows: the rest of layer `layer` for those rows: neigh_r = the max over the in-edges of v_r of hp[source], then
+ *   out[v_r] = [h_r | neigh_r] [Ws | Wn]^T + b written by vertex id into out_dev [*, ldo], ldo = round_up(output width, 8): ReLU and
+ *   the storage type for a hidden layer, fp32 logits for the last.  neigh_mode 0: the segment max over whole rows (hp_dev [n_vertices,
+ *   ldhp]); the rows are also written into neigh_dev when it is not NULL.  1: the suffix max of ogl_graph_segment_max_suffix into
+ *   neigh_dev in place (deg_prev_dev as there), then its rows are read.  2: the rows are read from neigh_dev (hp_dev unused).  neigh_dev
+ *   [*, ldn], ldn = round_up(input width, 8).  Listed ids must be distinct.
+ *   Both: ordered on `stream`, no host synchronisation; profiled as stages "stream.l<layer>.pool_rows", ".segmax", ".segmax_suffix",
+ *   ".out_gemm", ".scatter".  They read the weights and use the full-inference workspace as compact scratch only (its per-vertex
+ *   tables are not read across calls), so they leave every other plan state alone, as ogl_plan_infer_full does.  n == 0 is a no-op. */
+int ogl_graph_out_frontier(ogl_graph* g, const int64_t* rows_dev, int64_t n, int32_t* out_rows_dev, int64_t* out_n,
+                           int64_t* out_edge_cost, void* stream);
+int ogl_graph_segment_max_suffix(ogl_graph* g, int mode, const void* x_dev, int ld, int cols, const int64_t* rows_dev, int64_t n,
+                                 const int64_t* deg_prev_dev, void* acc_dev, int ldacc, void* stream);
+int ogl_plan_out_frontier(ogl_plan* p, ogl_graph* g, int layer, const int64_t* rows_dev, int64_t n, int64_t* out_rows_dev,
+                          int64_t* out_n, int64_t* out_edge_cost, void* stream);
+int ogl_plan_pool_rows(ogl_plan* p, ogl_graph* g, ogl_features* f, int layer, const void* h_dev, int ldh, const int64_t* rows_dev,
+                       int64_t row0, int64_t n, void* hp_dev, int ldhp, void* stream);
+int ogl_plan_stream_rows(ogl_plan* p, ogl_graph* g, ogl_features* f, int layer, const void* h_dev, int ldh, const void* hp_dev, int ldhp,
+                         const int64_t* rows_dev, int64_t row0, int64_t n, void* neigh_dev, int ldn, int neigh_mode,
+                         const int64_t* deg_prev_dev, void* out_dev, int ldo, void* stream);
+
 /* stage profiling for bench.py's roofline: CUDA events recorded around every stage of the plan's calls on the
  * caller's stream (off by default).  enable=1 (re)starts a collection.  _read synchronises the device and returns,
  * per stage, the summed milliseconds and kernel launches, plus the per-level node counts summed over the

@@ -120,6 +120,11 @@ SIGNATURES = {
     "ogl_plan_full_xent": (_i, [_vp, _vp, _vp, _i, _vp, _i64, _i64, _vp, _vp]),
     "ogl_graph_segment_max": (_i, [_vp, _i, _vp, _i, _i, _vp, _i64, _vp, _i, _vp]),
     "ogl_graph_in_frontier": (_i, [_vp, _vp, _i64, _vp, C.POINTER(_i64), C.POINTER(_i64), _vp]),
+    "ogl_graph_out_frontier": (_i, [_vp, _vp, _i64, _vp, C.POINTER(_i64), C.POINTER(_i64), _vp]),
+    "ogl_graph_segment_max_suffix": (_i, [_vp, _i, _vp, _i, _i, _vp, _i64, _vp, _vp, _i, _vp]),
+    "ogl_plan_out_frontier": (_i, [_vp, _vp, _i, _vp, _i64, _vp, C.POINTER(_i64), C.POINTER(_i64), _vp]),
+    "ogl_plan_pool_rows": (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, _i64, _i64, _vp, _i, _vp]),
+    "ogl_plan_stream_rows": (_i, [_vp, _vp, _vp, _i, _vp, _i, _vp, _i, _vp, _i64, _i64, _vp, _i, _i, _vp, _vp, _i, _vp]),
     "ogl_plan_profile": (_i, [_vp, _i]),
     "ogl_plan_profile_read": (_i, [_vp, C.c_char_p, _i, _vp, _vp, _i, C.POINTER(_i), _vp, C.POINTER(_i)]),
     "ogl_plan_level_nodes": (_i, [_vp, _i, _pp, _pp, C.POINTER(_i)]),

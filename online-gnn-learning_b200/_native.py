@@ -55,6 +55,9 @@ class Graph:
         self._h = C.c_void_p()
         check(lib.ogl_graph_create(C.byref(self._h), int(v_cap), int(e_cap_directed)))
         self.v_cap = int(v_cap)
+        # bumped whenever rows are rebuilt from a parent graph (load_parent, set_active_prefix): their edges are then in parent
+        # edge-id order, so what a row gained is no longer the tail of its adjacency (StreamingInference recomputes such rows whole)
+        self.rebuilds = 0
 
     def __del__(self):
         # (at interpreter shutdown the module globals may already be gone: nothing left to free then)
@@ -90,9 +93,11 @@ class Graph:
         ip, ix, ei = _dev(indptr, torch.int64), _dev(indices, torch.int64), _dev(eids, torch.int64)
         check(lib.ogl_graph_load_parent(self._h, _ptr(ip), _ptr(ix), _ptr(ei), ip.numel() - 1, _stream()))
         torch.cuda.current_stream().synchronize()
+        self.rebuilds += 1
 
     def set_active_prefix(self, n_active):
         check(lib.ogl_graph_set_active_prefix(self._h, int(n_active), _stream()))
+        self.rebuilds += 1
 
     @property
     def num_vertices(self):
@@ -163,6 +168,31 @@ class Graph:
         n, cost = C.c_int64(), C.c_int64()
         check(lib.ogl_graph_in_frontier(self._h, _ptr(r), r.numel(), _ptr(out), C.byref(n), C.byref(cost), _stream()))
         return out[:n.value].to(torch.int64), cost.value
+
+    def out_frontier(self, rows):
+        """the out-neighbourhood frontier of the vertex ids `rows`: (ids, cost), ids = the distinct vertices of rows and every vertex with
+        an in-edge from one of them, ascending (CUDA int64), cost = sum over them of (in-degree + 1).  Ids outside the graph are
+        ignored.  One pass over every row's adjacency, whatever the list's length."""
+        r = _dev(rows, torch.int64)
+        out = torch.empty(max(self.num_vertices, 1), dtype=torch.int32, device="cuda")
+        n, cost = C.c_int64(), C.c_int64()
+        check(lib.ogl_graph_out_frontier(self._h, _ptr(r), r.numel(), _ptr(out), C.byref(n), C.byref(cost), _stream()))
+        return out[:n.value].to(torch.int64), cost.value
+
+    def segment_max_suffix(self, x, acc, rows, deg_prev, cols=None):
+        """in place: acc[v] = max(acc[v], max over the in-edges of v appended since it had deg_prev[v] of them of x[source]) for the
+        distinct vertex ids `rows`; deg_prev[v] == 0 replaces the row (zeros without in-edges).  x, acc: CUDA fp32 / bf16 / fp16
+        [*, ld] tables with a row per vertex id and unit column stride; deg_prev: int64 [>= num_vertices] indexed by vertex id"""
+        mode = {torch.float32: OGL_F32, torch.bfloat16: OGL_BF16, torch.float16: OGL_FP16}[x.dtype]
+        assert x.is_cuda and acc.is_cuda and x.dtype == acc.dtype and x.dim() == 2 and acc.dim() == 2
+        assert x.stride(1) == 1 and acc.stride(1) == 1
+        cols = x.shape[1] if cols is None else int(cols)
+        r = _dev(rows, torch.int64)
+        d = _dev(deg_prev, torch.int64)
+        assert d.numel() >= self.num_vertices
+        check(lib.ogl_graph_segment_max_suffix(self._h, mode, C.c_void_p(x.data_ptr()), x.stride(0), cols, _ptr(r), r.numel(), _ptr(d),
+                                               C.c_void_p(acc.data_ptr()), acc.stride(0), _stream()))
+        return acc
 
     def stats(self):
         a = (C.c_int64 * 4)()
@@ -417,6 +447,59 @@ class Plan:
         + 1 of infer_full_layer); pitch = round_up(width, 8)"""
         assert 0 <= layer < self.L - 1, "layer %d has no hidden output (the model has %d layers)" % (layer, self.L)
         return torch.empty((int(rows) + 127) // 128 * 128, (self.dims[layer + 1] + 7) // 8 * 8, dtype=self.dtype, device="cuda")
+
+    def pool_table(self, layer, rows):
+        """a zeroed [round_up(rows, 256), pitch] table in the plan's storage dtype for layer `layer`'s pool rows relu(h Wp^T + bp)
+        (pool_rows; the hp of stream_rows), pitch = round_up(the layer's input width, 8)"""
+        assert 0 <= layer < self.L
+        return torch.zeros((int(rows) + 255) // 256 * 256, (self.dims[layer] + 7) // 8 * 8, dtype=self.dtype, device="cuda")
+
+    def _rows_arg(self, rows, row0, n, graph):
+        r = None if rows is None else _dev(rows, torch.int64)
+        if r is not None:
+            return r, 0, r.numel()
+        return None, int(row0), graph.num_vertices - int(row0) if n is None else int(n)
+
+    @staticmethod
+    def _tab(t, dtype):
+        if t is None:
+            return None, 0
+        assert t.is_cuda and t.dim() == 2 and t.stride(1) == 1 and t.dtype == dtype
+        return C.c_void_p(t.data_ptr()), t.stride(0)
+
+    def pool_rows(self, graph, features, layer, h, hp, rows=None, row0=0, n=None):
+        """hp[v] = relu(h[v] Wp^T + bp) of `layer` for the vertex ids `rows` (distinct) or [row0, row0 + n), written by vertex id into
+        the table hp (a pool_table(layer, >= V)); h as for infer_full_layer (None for layer 0, which reads `features`)"""
+        r, row0, n = self._rows_arg(rows, row0, n, graph)
+        hp_, ldh = self._tab(h, self.dtype)
+        pp, ldp = self._tab(hp, self.dtype)
+        check(lib.ogl_plan_pool_rows(self._h, graph._h, features._h, int(layer), hp_, ldh, _ptr(r), row0, n, pp, ldp, _stream()))
+
+    NEIGH_SEGMAX, NEIGH_SUFFIX, NEIGH_TABLE = 0, 1, 2
+
+    def stream_rows(self, graph, features, layer, h, hp, out, rows=None, row0=0, n=None, neigh=None, neigh_mode=0, deg_prev=None):
+        """the segment max of hp over the in-edges of the vertex ids `rows` (distinct) or [row0, row0 + n) and layer `layer`'s output
+        GEMM, written by vertex id into `out` (a hidden_table, or fp32 logits [*, round_up(C, 8)] for the last layer).  neigh_mode
+        NEIGH_SEGMAX: whole rows, also written into the table `neigh` when given; NEIGH_SUFFIX: the suffix max into `neigh` in place
+        (deg_prev: int64 [>= V] by vertex id, see Graph.segment_max_suffix); NEIGH_TABLE: the rows of `neigh` as they are"""
+        r, row0, n = self._rows_arg(rows, row0, n, graph)
+        last = layer == self.L - 1
+        hh, ldh = self._tab(h, self.dtype)
+        pp, ldp = self._tab(hp, self.dtype)
+        nn_, ldn = self._tab(neigh, self.dtype)
+        oo, ldo = self._tab(out, torch.float32 if last else self.dtype)
+        d = None if deg_prev is None else _dev(deg_prev, torch.int64)
+        check(lib.ogl_plan_stream_rows(self._h, graph._h, features._h, int(layer), hh, ldh, pp, ldp, _ptr(r), row0, n, nn_, ldn,
+                                       int(neigh_mode), _ptr(d), oo, ldo, _stream()))
+
+    def out_frontier(self, graph, rows, layer=0):
+        """Graph.out_frontier on the plan's scratch (no allocation after the first call), profiled as stage stream.l<layer>.frontier:
+        (ids CUDA int64 ascending, cost)"""
+        r = _dev(rows, torch.int64)
+        out = torch.empty(max(graph.num_vertices, 1), dtype=torch.int64, device="cuda")
+        n, cost = C.c_int64(), C.c_int64()
+        check(lib.ogl_plan_out_frontier(self._h, graph._h, int(layer), _ptr(r), r.numel(), _ptr(out), C.byref(n), C.byref(cost), _stream()))
+        return out[:n.value], cost.value
 
     def infer_full_layer(self, graph, features, layer, h, rows=None, row0=0, n=None, out=None):
         """layer `layer` of infer_full for the destination rows `rows` (int64 ids) or [row0, row0 + n) (n None: to the last vertex):

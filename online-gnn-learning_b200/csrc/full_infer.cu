@@ -14,6 +14,9 @@
 // The in-neighbourhood frontier S u N_in(S) of a row list (k_frontier_*) reads the same CSR: it marks a bitmap, splitting hub rows
 // into the same chunks, and compacts it to ascending ids.  Full inference of a short list runs its hidden layers on these rows only.
 //
+// The out-neighbourhood frontier S u N_out(S) (k_out_frontier_*) and the suffix max (k_suffix_rows: the max over the edges appended
+// to a row since a refresh, folded into the row's stored max) serve incremental inference (StreamingInference, plan.cu).
+//
 // The per-vertex cross entropy over full-inference logits (k_full_xent) lives here too: one warp per row, the logsumexp of the
 // training loss (warp_logsumexp, sage_kernels.cuh).
 #include "full_infer.cuh"
@@ -56,10 +59,11 @@ __device__ __forceinline__ uint4 vmax(uint4 a, uint4 b) {
   return make_uint4(Strip<T>::max2(a.x, b.x), Strip<T>::max2(a.y, b.y), Strip<T>::max2(a.z, b.z), Strip<T>::max2(a.w, b.w));
 }
 
-// one warp: o[strips] = max over the cnt adjacency entries adj[0..cnt) of x[src], 0 if cnt == 0
-template <typename T>
+// one warp: o[strips] = max over the cnt adjacency entries adj[0..cnt) of x[src], 0 if cnt == 0.  Merge (the suffix max): unless
+// `replace`, o = max(o, that max) instead, and o is left alone when cnt == 0
+template <typename T, bool Merge = false>
 __device__ __forceinline__ void warp_row_max(const T* __restrict__ x, int ld, int strips, const unsigned long long* __restrict__ adj,
-                                             int cnt, T* __restrict__ o, int lane) {
+                                             int cnt, T* __restrict__ o, int lane, bool replace = true) {
   constexpr int NV = Strip<T>::N;
   for (int s0 = 0; s0 < strips; s0 += 32) {
     const int st = s0 + lane;
@@ -85,7 +89,11 @@ __device__ __forceinline__ void warp_row_max(const T* __restrict__ x, int ld, in
         if (act) acc = vmax<T>(acc, __ldg(reinterpret_cast<const uint4*>(x + (int64_t)src * ld) + st));
       }
     }
-    if (act) *reinterpret_cast<uint4*>(o + (int64_t)st * NV) = cnt > 0 ? acc : make_uint4(0u, 0u, 0u, 0u);
+    if (act) {
+      uint4* po = reinterpret_cast<uint4*>(o + (int64_t)st * NV);
+      if (!Merge || replace) *po = cnt > 0 ? acc : make_uint4(0u, 0u, 0u, 0u);
+      else if (cnt > 0) *po = vmax<T>(*po, acc);
+    }
   }
 }
 
@@ -142,7 +150,8 @@ __global__ void __launch_bounds__(kBlock) k_csr_segmax_rows(GraphView gv, const 
   }
 }
 
-template <typename T>
+// Suffix: the records are those of k_suffix_rows (r = the first edge of the suffix, the output row is the vertex)
+template <typename T, bool Suffix = false>
 __global__ void __launch_bounds__(kBlock) k_csr_segmax_chunks(GraphView gv, const T* __restrict__ x, int ld, int strips,
                                                               unsigned long long* __restrict__ ctl, const SegmaxHub* __restrict__ hubs,
                                                               const int32_t* __restrict__ chunk_hub, int64_t chunk_cap, T* __restrict__ partial,
@@ -157,29 +166,97 @@ __global__ void __launch_bounds__(kBlock) k_csr_segmax_chunks(GraphView gv, cons
     const SegmaxHub hb = hubs[h];
     const int64_t i = c - hb.base;
     const int deg = gv.deg[hb.v];
-    const int e0 = (int)(i * kSegmaxChunk);
+    const int e0 = (Suffix ? (int)hb.r : 0) + (int)(i * kSegmaxChunk);
     warp_row_max(x, ld, strips, gv.adj + gv.row_start[hb.v] + e0, min(kSegmaxChunk, deg - e0), partial + c * (int64_t)ldp, lane);
   }
 }
 
-template <typename T>
+// Suffix: the partial rows are combined into out[v] (kept unless the record's pad flag says the row is replaced)
+template <typename T, bool Suffix = false>
 __global__ void __launch_bounds__(kBlock) k_csr_segmax_combine(const unsigned long long* __restrict__ ctl, const SegmaxHub* __restrict__ hubs,
                                                                int64_t hub_cap, const T* __restrict__ partial, int ldp, int strips,
                                                                T* __restrict__ out, int ldo) {
-  constexpr int NV = Strip<T>::N;
   const int lane = threadIdx.x & 31;
   const int64_t n = min((int64_t)ctl[1], hub_cap);
   const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   for (int64_t h = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; h < n; h += warps) {
     const SegmaxHub hb = hubs[h];
     if (hb.n == 0) continue;
+    uint4* o = reinterpret_cast<uint4*>(out + (Suffix ? (int64_t)hb.v : hb.r) * (int64_t)ldo);
     for (int st = lane; st < strips; st += 32) {
       uint4 acc = Strip<T>::neg_inf();
       for (int i = 0; i < hb.n; ++i)
         acc = vmax<T>(acc, __ldg(reinterpret_cast<const uint4*>(partial + (int64_t)(hb.base + i) * ldp) + st));
-      *reinterpret_cast<uint4*>(out + hb.r * (int64_t)ldo + (int64_t)st * NV) = acc;
+      if (Suffix && !hb.pad) acc = vmax<T>(acc, o[st]);
+      o[st] = acc;
     }
   }
+}
+
+// ---- suffix segment max (csr_segmax_suffix): the rows pass of k_csr_segmax_rows over the edges [e0, deg) of each listed row, e0 =
+// deg_prev[v] (0 and a replaced row when deg_prev[v] is 0 or past the degree).  A suffix of more than kSegmaxChunk edges goes to the
+// chunk list as a hub record {r = e0, v, base, n, pad = replace}; the chunk and combine passes above then finish it.
+template <typename T, typename Idx>
+__global__ void __launch_bounds__(kBlock) k_suffix_rows(GraphView gv, const T* __restrict__ x, int ld, int strips, const Idx* __restrict__ rows,
+                                                        int64_t row0, int64_t n_rows, const int64_t* __restrict__ deg_prev, T* __restrict__ acc,
+                                                        int ldacc, unsigned long long* __restrict__ ctl, SegmaxHub* __restrict__ hubs,
+                                                        int64_t hub_cap, int32_t* __restrict__ chunk_hub, int64_t chunk_cap) {
+  const int lane = threadIdx.x & 31;
+  for (;;) {
+    const int64_t r = warp_next(ctl + 0, lane);
+    if (r >= n_rows) break;
+    const int64_t v = rows ? (int64_t)rows[r] : row0 + r;
+    if (v < 0 || v >= gv.n_vertices) continue;
+    const int deg = gv.deg[v];
+    const int64_t prev = deg_prev[v];
+    const bool replace = prev <= 0 || prev > deg;
+    const int e0 = replace ? 0 : (int)prev, cnt = deg - e0;
+    const unsigned long long* adj = gv.adj + gv.row_start[v] + e0;
+    T* o = acc + v * (int64_t)ldacc;
+    if (cnt > kSegmaxChunk) {
+      const int nch = (cnt + kSegmaxChunk - 1) / kSegmaxChunk;
+      long long h = -1, base = -1;
+      if (lane == 0) {
+        h = (long long)atomicAdd(ctl + 1, 1ull);
+        if (h < hub_cap) {
+          base = (long long)atomicAdd(ctl + 2, (unsigned long long)nch);
+          const bool ok = base + nch <= chunk_cap;
+          hubs[h] = SegmaxHub{e0, (int32_t)v, (int32_t)(ok ? base : 0), ok ? nch : 0, replace ? 1 : 0};
+          if (!ok) {
+            for (long long c = base; c < chunk_cap && c < base + nch; ++c) chunk_hub[c] = -1;
+            base = -1;
+          }
+        }
+      }
+      base = __shfl_sync(0xffffffffu, base, 0);
+      h = __shfl_sync(0xffffffffu, h, 0);
+      if (base >= 0) {
+        for (int c = lane; c < nch; c += 32) chunk_hub[base + c] = (int32_t)h;
+        continue;
+      }
+    }
+    warp_row_max<T, true>(x, ld, strips, adj, cnt, o, lane, replace);
+  }
+}
+
+template <typename T>
+int launch_suffix(const GraphView& gv, const void* x, int ld, int strips, const int32_t* rows32, const int64_t* rows64, int64_t row0,
+                  int64_t n_rows, const int64_t* deg_prev, void* acc, int ldacc, SegmaxWs* ws, cudaStream_t s) {
+  const int ldp = strips * Strip<T>::N;
+  const int persistent = sm_count() * 8;
+  const int rgrid = (int)std::min<int64_t>(persistent, ceil_div(n_rows, kBlock / 32));
+  OGL_CUDA(cudaMemsetAsync(ws->ctl, 0, 4 * sizeof(unsigned long long), s));
+  if (rows64)
+    OGL_LAUNCH((k_suffix_rows<T, int64_t>), rgrid, kBlock, 0, s, gv, (const T*)x, ld, strips, rows64, row0, n_rows, deg_prev, (T*)acc, ldacc,
+               ws->ctl, ws->hubs, ws->hub_cap, ws->chunk_hub, ws->chunk_cap);
+  else
+    OGL_LAUNCH((k_suffix_rows<T, int32_t>), rgrid, kBlock, 0, s, gv, (const T*)x, ld, strips, rows32, row0, n_rows, deg_prev, (T*)acc, ldacc,
+               ws->ctl, ws->hubs, ws->hub_cap, ws->chunk_hub, ws->chunk_cap);
+  OGL_LAUNCH((k_csr_segmax_chunks<T, true>), persistent, kBlock, 0, s, gv, (const T*)x, ld, strips, ws->ctl, ws->hubs, ws->chunk_hub,
+             ws->chunk_cap, (T*)ws->partial, ldp);
+  OGL_LAUNCH((k_csr_segmax_combine<T, true>), (int)std::min<int64_t>(persistent, ceil_div(ws->hub_cap, kBlock / 32)), kBlock, 0, s, ws->ctl,
+             ws->hubs, ws->hub_cap, (const T*)ws->partial, ldp, strips, (T*)acc, ldacc);
+  return OGL_OK;
 }
 
 template <typename T>
@@ -282,8 +359,9 @@ __global__ void __launch_bounds__(kBlock) k_frontier_count(const uint32_t* __res
 }
 
 // one warp per bitmap word, lane = bit: set bits go to out[offs[word] + rank among the word's set bits]; *cost += deg + 1 of each
+template <typename OutIdx>
 __global__ void __launch_bounds__(kBlock) k_frontier_fill(const uint32_t* __restrict__ bits, const int32_t* __restrict__ offs, int64_t words,
-                                                          const int32_t* __restrict__ deg, int32_t* __restrict__ out,
+                                                          const int32_t* __restrict__ deg, OutIdx* __restrict__ out,
                                                           unsigned long long* __restrict__ cost) {
   const int lane = threadIdx.x & 31;
   const int64_t warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
@@ -292,11 +370,73 @@ __global__ void __launch_bounds__(kBlock) k_frontier_fill(const uint32_t* __rest
     const uint32_t word = bits[w];
     if (!((word >> lane) & 1u)) continue;
     const int v = (int)(w * 32 + lane);
-    out[offs[w] + __popc(word & ((1u << lane) - 1))] = v;
+    out[offs[w] + __popc(word & ((1u << lane) - 1))] = (OutIdx)v;
     c += (unsigned long long)deg[v] + 1ull;
   }
   for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
   if (lane == 0 && c) atomicAdd(cost, c);
+}
+
+// ---- out-neighbourhood frontier S u N_out(S) (out_frontier): the CSR holds in-edges only, so every row outside S scans its own
+// sources against the bitmap of S and joins the result bitmap (seeded with S) at the first hit.  Four 32-entry groups of the
+// adjacency are loaded before the vote, then the warp stops if any lane hit.
+__device__ __forceinline__ bool warp_any_source(const unsigned long long* __restrict__ adj, int cnt, const uint32_t* __restrict__ in, int lane) {
+  constexpr int kGroups = 4;
+  for (int j0 = 0; j0 < cnt; j0 += 32 * kGroups) {
+    uint32_t u[kGroups];
+#pragma unroll
+    for (int k = 0; k < kGroups; ++k) {
+      const int j = j0 + 32 * k + lane;
+      u[k] = j < cnt ? (uint32_t)__ldg(adj + j) : 0xffffffffu;
+    }
+    bool hit = false;
+#pragma unroll
+    for (int k = 0; k < kGroups; ++k)
+      if (u[k] != 0xffffffffu) hit |= (__ldg(in + (u[k] >> 5)) >> (u[k] & 31)) & 1u;
+    if (__any_sync(0xffffffffu, hit)) return true;
+  }
+  return false;
+}
+
+// rows: persistent warps take every vertex from a cursor; a row of more than kSegmaxChunk edges is a hub whose chunks go to the chunk
+// list (if the list is full the warp scans the row itself)
+__global__ void __launch_bounds__(kBlock) k_out_frontier_rows(GraphView gv, const uint32_t* __restrict__ in, uint32_t* __restrict__ out,
+                                                              unsigned long long* __restrict__ ctl, int2* __restrict__ chunks, int64_t chunk_cap) {
+  const int lane = threadIdx.x & 31;
+  for (;;) {
+    const int64_t v = warp_next(ctl + 1, lane);
+    if (v >= gv.n_vertices) break;
+    if ((__ldg(in + (v >> 5)) >> (v & 31)) & 1u) continue;       // in S: already in the result
+    const int deg = gv.deg[v];
+    const unsigned long long* adj = gv.adj + gv.row_start[v];
+    if (deg > kSegmaxChunk) {
+      const int nch = (deg + kSegmaxChunk - 1) / kSegmaxChunk;
+      long long base = 0;
+      if (lane == 0) base = (long long)atomicAdd(ctl + 2, (unsigned long long)nch);
+      base = __shfl_sync(0xffffffffu, base, 0);
+      const bool ok = base + nch <= chunk_cap;
+      for (int c = lane; c < nch && base + c < chunk_cap; c += 32) chunks[base + c] = make_int2(ok ? (int)v : -1, c * kSegmaxChunk);
+      if (ok) continue;
+    }
+    if (warp_any_source(adj, deg, in, lane) && lane == 0) atomicOr(out + (v >> 5), 1u << (v & 31));
+  }
+}
+
+__global__ void __launch_bounds__(kBlock) k_out_frontier_chunks(GraphView gv, const uint32_t* __restrict__ in, uint32_t* __restrict__ out,
+                                                                unsigned long long* __restrict__ ctl, const int2* __restrict__ chunks,
+                                                                int64_t chunk_cap) {
+  const int lane = threadIdx.x & 31;
+  const int64_t n = min((int64_t)ctl[2], chunk_cap);
+  for (;;) {
+    const int64_t c = warp_next(ctl + 3, lane);
+    if (c >= n) break;
+    const int2 ch = chunks[c];
+    if (ch.x < 0) continue;
+    const uint32_t b = 1u << (ch.x & 31);
+    if (__ldcg(out + (ch.x >> 5)) & b) continue;                 // another chunk of the row already hit
+    if (warp_any_source(gv.adj + gv.row_start[ch.x] + ch.y, min(kSegmaxChunk, gv.deg[ch.x] - ch.y), in, lane) && lane == 0)
+      atomicOr(out + (ch.x >> 5), b);
+  }
 }
 
 // loss[r] = logsumexp(logits[r, :C]) - logits[r, y], y = labels[v_r], v_r = rows[r] | row0 + r.  A v_r outside [0, n_vertices) reads
@@ -340,7 +480,7 @@ int full_xent(const float* logits, int ld, int C, const int32_t* labels, const i
 }
 
 void frontier_ws_free(FrontierWs* ws) {
-  for (void* q : {(void*)ws->bits, (void*)ws->uniq, (void*)ws->counts, (void*)ws->offs, (void*)ws->scan, (void*)ws->chunks, (void*)ws->ctl,
+  for (void* q : {(void*)ws->bits, (void*)ws->bits_in, (void*)ws->uniq, (void*)ws->counts, (void*)ws->offs, (void*)ws->scan, (void*)ws->chunks, (void*)ws->ctl,
                   (void*)ws->out})
     cudaFree(q);
   *ws = FrontierWs();
@@ -351,7 +491,8 @@ int frontier_ws_reserve(FrontierWs* ws, int64_t n_vertices, int64_t n_edges) {
   if (ws->ctl && ws->v_cap >= n_vertices && ws->chunk_cap >= chunk_cap) return OGL_OK;
   const int64_t vc = std::max(n_vertices, ws->v_cap), cc = std::max(chunk_cap, ws->chunk_cap), words = ceil_div(vc, 32) + 1;
   frontier_ws_free(ws);
-  if (cudaMalloc(&ws->bits, sizeof(uint32_t) * words) != cudaSuccess || cudaMalloc(&ws->uniq, sizeof(int32_t) * vc) != cudaSuccess ||
+  if (cudaMalloc(&ws->bits, sizeof(uint32_t) * words) != cudaSuccess || cudaMalloc(&ws->bits_in, sizeof(uint32_t) * words) != cudaSuccess ||
+      cudaMalloc(&ws->uniq, sizeof(int32_t) * vc) != cudaSuccess ||
       cudaMalloc(&ws->counts, sizeof(int32_t) * words) != cudaSuccess || cudaMalloc(&ws->offs, sizeof(int32_t) * words) != cudaSuccess ||
       cudaMalloc(&ws->scan, sizeof(int32_t) * scan_scratch_elems(words)) != cudaSuccess ||
       cudaMalloc(&ws->chunks, sizeof(int2) * cc) != cudaSuccess || cudaMalloc(&ws->ctl, 4 * sizeof(unsigned long long)) != cudaSuccess ||
@@ -385,7 +526,34 @@ int in_frontier(const GraphView& gv, int64_t n_edges, const int32_t* rows32, con
   if (words == 0) return OGL_OK;
   OGL_LAUNCH(k_frontier_count, grid_for(words, kBlock), kBlock, 0, s, ws->bits, words, ws->counts);
   OGL_TRY(exclusive_scan_i32(ws->counts, ws->offs, words, ws->scan, &ws->out->n, s));
-  OGL_LAUNCH(k_frontier_fill, grid_for(words * 32, kBlock), kBlock, 0, s, ws->bits, ws->offs, words, gv.deg, out_rows, &ws->out->cost);
+  OGL_LAUNCH(k_frontier_fill<int32_t>, grid_for(words * 32, kBlock), kBlock, 0, s, ws->bits, ws->offs, words, gv.deg, out_rows, &ws->out->cost);
+  return OGL_OK;
+}
+
+int out_frontier(const GraphView& gv, int64_t n_edges, const int64_t* rows64, int64_t n, int32_t* out_rows32, int64_t* out_rows64,
+                 FrontierWs* ws, cudaStream_t s) {
+  OGL_TRY(frontier_ws_reserve(ws, gv.n_vertices, n_edges));
+  const int64_t words = ceil_div(gv.n_vertices, 32);
+  OGL_CUDA(cudaMemsetAsync(ws->bits_in, 0, sizeof(uint32_t) * words, s));
+  OGL_CUDA(cudaMemsetAsync(ws->ctl, 0, 4 * sizeof(unsigned long long), s));
+  OGL_CUDA(cudaMemsetAsync(ws->out, 0, sizeof(FrontierOut), s));
+  if (words == 0) return OGL_OK;
+  if (n > 0)
+    OGL_LAUNCH(k_frontier_seed<int64_t>, grid_for(n, kBlock), kBlock, 0, s, rows64, n, gv.n_vertices, ws->bits_in, ws->uniq, ws->ctl);
+  OGL_CUDA(cudaMemcpyAsync(ws->bits, ws->bits_in, sizeof(uint32_t) * words, cudaMemcpyDeviceToDevice, s));
+  if (n > 0) {
+    const int persistent = sm_count() * 8;
+    OGL_LAUNCH(k_out_frontier_rows, persistent, kBlock, 0, s, gv, ws->bits_in, ws->bits, ws->ctl, ws->chunks, ws->chunk_cap);
+    OGL_LAUNCH(k_out_frontier_chunks, persistent, kBlock, 0, s, gv, ws->bits_in, ws->bits, ws->ctl, ws->chunks, ws->chunk_cap);
+  }
+  OGL_LAUNCH(k_frontier_count, grid_for(words, kBlock), kBlock, 0, s, ws->bits, words, ws->counts);
+  OGL_TRY(exclusive_scan_i32(ws->counts, ws->offs, words, ws->scan, &ws->out->n, s));
+  if (out_rows64)
+    OGL_LAUNCH(k_frontier_fill<int64_t>, grid_for(words * 32, kBlock), kBlock, 0, s, ws->bits, ws->offs, words, gv.deg, out_rows64,
+               &ws->out->cost);
+  else
+    OGL_LAUNCH(k_frontier_fill<int32_t>, grid_for(words * 32, kBlock), kBlock, 0, s, ws->bits, ws->offs, words, gv.deg, out_rows32,
+               &ws->out->cost);
   return OGL_OK;
 }
 
@@ -418,6 +586,16 @@ int csr_segmax(int mode, const GraphView& gv, int64_t n_edges, const void* x, in
   const int strips = (cols + nv - 1) / nv;
   OGL_TRY(segmax_ws_reserve(ws, n_edges, (int64_t)strips * 16));
   OGL_MODE_DISPATCH(mode, OGL_TRY(launch_segmax<T>(gv, x, ld, strips, rows32, rows64, row0, n_rows, out, ldo, ws, s)));
+  return OGL_OK;
+}
+
+int csr_segmax_suffix(int mode, const GraphView& gv, int64_t n_edges, const void* x, int ld, int cols, const int32_t* rows32,
+                      const int64_t* rows64, int64_t row0, int64_t n, const int64_t* deg_prev, void* acc, int ldacc, SegmaxWs* ws, cudaStream_t s) {
+  if (n <= 0) return OGL_OK;
+  const int nv = mode_vec(mode);
+  const int strips = (cols + nv - 1) / nv;
+  OGL_TRY(segmax_ws_reserve(ws, n_edges, (int64_t)strips * 16));
+  OGL_MODE_DISPATCH(mode, OGL_TRY(launch_suffix<T>(gv, x, ld, strips, rows32, rows64, row0, n, deg_prev, acc, ldacc, ws, s)));
   return OGL_OK;
 }
 
@@ -472,5 +650,52 @@ extern "C" int ogl_graph_in_frontier(ogl_graph* g, const int64_t* rows_dev, int6
   frontier_ws_free(&ws);
   *out_n = h.n;
   *out_edge_cost = (int64_t)h.cost;
+  return r;
+}
+
+extern "C" int ogl_graph_out_frontier(ogl_graph* g, const int64_t* rows_dev, int64_t n, int32_t* out_rows_dev, int64_t* out_n,
+                                      int64_t* out_edge_cost, void* stream) {
+  OGL_TRY(require_device());
+  OGL_ARG(g && out_n && out_edge_cost && n >= 0 && (rows_dev || n == 0), "ogl_graph_out_frontier: bad arguments");
+  OGL_ARG(graph_source_bound(g) == 0, "ogl_graph_out_frontier: the graph is a destination shard (ogl_graph_set_source_bound): its sources "
+          "are not its rows");
+  const GraphView gv = graph_view(g);
+  OGL_ARG(out_rows_dev || gv.n_vertices == 0, "ogl_graph_out_frontier: null out_rows");
+  cudaStream_t s = (cudaStream_t)stream;
+  FrontierWs ws;
+  FrontierOut h{};
+  int r = out_frontier(gv, graph_num_edges(g), rows_dev, n, out_rows_dev, nullptr, &ws, s);
+  if (r == OGL_OK && (cudaMemcpyAsync(&h, ws.out, sizeof(h), cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+                      cudaStreamSynchronize(s) != cudaSuccess)) {
+    set_error("ogl_graph_out_frontier: %s", cudaGetErrorString(cudaGetLastError()));
+    r = OGL_ERR_CUDA;
+  }
+  frontier_ws_free(&ws);
+  *out_n = h.n;
+  *out_edge_cost = (int64_t)h.cost;
+  return r;
+}
+
+extern "C" int ogl_graph_segment_max_suffix(ogl_graph* g, int mode, const void* x_dev, int ld, int cols, const int64_t* rows_dev, int64_t n,
+                                            const int64_t* deg_prev_dev, void* acc_dev, int ldacc, void* stream) {
+  OGL_TRY(require_device());
+  OGL_ARG(g && mode_valid(mode) && n >= 0 && (rows_dev || n == 0) && (deg_prev_dev || n == 0), "ogl_graph_segment_max_suffix: bad arguments");
+  OGL_ARG(graph_source_bound(g) == 0, "ogl_graph_segment_max_suffix: the graph is a destination shard (ogl_graph_set_source_bound): its "
+          "sources are not rows of x");
+  if (n == 0) return OGL_OK;
+  const int nv = mode_vec(mode);
+  OGL_ARG(x_dev && acc_dev && cols > 0 && cols <= ld && ld % nv == 0 && ldacc % nv == 0 && (cols + nv - 1) / nv * nv <= ldacc &&
+              ((uintptr_t)x_dev & 15) == 0 && ((uintptr_t)acc_dev & 15) == 0,
+          "ogl_graph_segment_max_suffix: x / acc must be 16-byte aligned with pitches ld, ldacc multiples of %d elements and ldacc >= cols "
+          "rounded up to %d", nv, nv);
+  cudaStream_t s = (cudaStream_t)stream;
+  SegmaxWs ws;
+  int r = csr_segmax_suffix(mode, graph_view(g), graph_num_edges(g), x_dev, ld, cols, nullptr, rows_dev, 0, n, deg_prev_dev, acc_dev, ldacc,
+                            &ws, s);
+  if (r == OGL_OK && cudaStreamSynchronize(s) != cudaSuccess) {          // (the workspace is freed below)
+    set_error("ogl_graph_segment_max_suffix: %s", cudaGetErrorString(cudaGetLastError()));
+    r = OGL_ERR_CUDA;
+  }
+  segmax_ws_free(&ws);
   return r;
 }

@@ -41,6 +41,7 @@ struct FrontierOut {
 };
 struct FrontierWs {
   uint32_t* bits = nullptr;            // [words] membership bitmap
+  uint32_t* bits_in = nullptr;         // [words] out_frontier: the input set S (bits is the result)
   int32_t *uniq = nullptr, *counts = nullptr, *offs = nullptr, *scan = nullptr;
   int2* chunks = nullptr;              // (vertex, first edge) of a hub's chunk
   unsigned long long* ctl = nullptr;   // [0] distinct input rows, [1] row cursor, [2] chunk slots, [3] chunk cursor
@@ -55,6 +56,21 @@ void frontier_ws_free(FrontierWs* ws);
 // id outside [0, n_vertices) is ignored.  Reads the streaming CSR in place; ordered on s, no host synchronisation.
 int in_frontier(const GraphView& gv, int64_t n_edges, const int32_t* rows32, const int64_t* rows64, int64_t n, int32_t* out_rows,
                 FrontierWs* ws, cudaStream_t s);
+
+// the out-neighbourhood frontier S u N_out(S) of S = {v_r} (the same lists and result as in_frontier, out_rows32 | out_rows64 exactly
+// one): a vertex joins when a source of one of its in-edges is in S.  The CSR stores in-edges only, so this is one pass over every
+// row's adjacency, read in place (hub rows cut into kSegmaxChunk chunks), against a bitmap of S; the result is a second bitmap
+// seeded with S, so one call expands by one hop.  O(E) work whatever |S|.  Ordered on s, no host synchronisation.
+int out_frontier(const GraphView& gv, int64_t n_edges, const int64_t* rows64, int64_t n, int32_t* out_rows32, int64_t* out_rows64,
+                 FrontierWs* ws, cudaStream_t s);
+
+// suffix segment max, in place: for v_r = rows32[r] | rows64[r] | row0 + r (r < n; a listed id outside [0, n_vertices) is skipped), acc[v_r, :cols] = max(acc[v_r],
+// max over the in-edges of v_r at row positions [deg_prev[v_r], deg[v_r]) of x[src]) -- the edges appended since a refresh at which
+// the row had deg_prev[v_r] edges.  deg_prev[v_r] == 0 (or larger than the degree) replaces the row instead (zeros for a row without
+// in-edges).  The arithmetic of csr_segmax, so the result is the bits of a whole-row max.  A suffix longer than kSegmaxChunk is cut
+// into chunks like a hub row.  acc [*, ldacc] in the storage type, indexed by vertex id; listed ids must be distinct.
+int csr_segmax_suffix(int mode, const GraphView& gv, int64_t n_edges, const void* x, int ld, int cols, const int32_t* rows32,
+                      const int64_t* rows64, int64_t row0, int64_t n, const int64_t* deg_prev, void* acc, int ldacc, SegmaxWs* ws, cudaStream_t s);
 
 // loss[r] = logsumexp(logits[r, :C]) - logits[r, labels[v_r]] for r < n (fp32 logits [n, ld]), v_r = rows32[r] | rows64[r] | row0 + r
 // (at most one list).  The arithmetic of the training loss (warp_logsumexp): equal logits give bit-equal losses.  A v_r outside

@@ -1399,6 +1399,150 @@ extern "C" int ogl_plan_infer_full_layer(ogl_plan* p, ogl_graph* g, ogl_features
                     out_dev, ldo, s);
 }
 
+// ------------------------------------------------------------------ incremental inference ----------
+// The pieces StreamingInference (inference.py) keeps its own per-vertex tables current with, for a row list or a row range at a time:
+// the pool GEMM of listed rows scattered into the caller's hp table, and a layer's segment max (whole rows, or the suffix of edges
+// appended since the last refresh, or rows already in the caller's neigh table) + output GEMM scattered into its hidden or logits
+// table.  p->full's tables only serve as compact scratch within one call, so full-inference calls between refreshes do no harm.
+// The GEMMs compute every row on its own and the segment max is exact: a row computed here has the bits of full_forward's.
+
+// a row list: its ids cast into w.seeds (out-of-range ids become vertex 0 and raise error bit 0); a range: nullptr
+static int stream_list(ogl_plan* p, const int64_t* rows_dev, int64_t n, int64_t V, const int32_t** rows32, cudaStream_t s) {
+  *rows32 = nullptr;
+  if (!rows_dev) return OGL_OK;
+  OGL_TRY(cast_nodes(rows_dev, p->full.seeds, n, V, p->ctl + 2, s));
+  *rows32 = p->full.seeds;
+  return OGL_OK;
+}
+
+// compact rows [n, pitch] into the caller's table [*, pitch]: by vertex id, or [row0, row0 + n) in one copy
+static int put_rows(int mode, size_t es, const void* rows, int pitch, const int32_t* rows32, int64_t row0, int64_t n, void* table,
+                    cudaStream_t s) {
+  if (rows32) return scatter_rows(mode, rows, pitch, rows32, (int)n, table, s);
+  OGL_CUDA(cudaMemcpyAsync((char*)table + es * (size_t)row0 * pitch, rows, es * (size_t)n * pitch, cudaMemcpyDeviceToDevice, s));
+  return OGL_OK;
+}
+
+// the listed rows of a table gathered into compact scratch (zero rows up to the next multiple of 128), or the range read in place
+static int rows_of(const ogl_plan* p, const void* table, int pitch, const int32_t* rows32, int64_t row0, int64_t n, void* scratch,
+                   const void** out, cudaStream_t s) {
+  if (!rows32) {
+    *out = (const char*)table + p->es * (size_t)row0 * pitch;
+    return OGL_OK;
+  }
+  OGL_TRY(gather_rows(p->mode, table, pitch, rows32, nullptr, (int)n, scratch, s));
+  const int64_t np = round_up((int)n, 128);
+  if (np > n) OGL_CUDA(cudaMemsetAsync((char*)scratch + p->es * (size_t)n * pitch, 0, p->es * (size_t)(np - n) * pitch, s));
+  *out = scratch;
+  return OGL_OK;
+}
+
+static int stream_check(const ogl_plan* p, ogl_graph* g, const ogl_features* f, int layer, const void* h_dev, int ldh, const int64_t* rows_dev,
+                        int64_t row0, int64_t n, const char* who, int64_t* V) {
+  OGL_TRY(full_check(p, g, f, who, V));
+  OGL_ARG(layer >= 0 && layer < p->L, "%s: layer %d out of range [0, %d)", who, layer, p->L);
+  OGL_ARG(n >= 0 && n < (1LL << 31), "%s: n out of range", who);
+  OGL_ARG(rows_dev || (row0 >= 0 && row0 + n <= *V), "%s: rows [%lld, %lld) are not vertices of the graph (%lld)", who, (long long)row0,
+          (long long)(row0 + n), (long long)*V);
+  const LayerBuf& lb = p->layer[layer];
+  OGL_ARG(layer == 0 || (h_dev && ldh == lb.pin && ((uintptr_t)h_dev & 15) == 0),
+          "%s: h must be a 16-byte aligned [n_vertices, %d] table of layer %d's input", who, lb.pin, layer);
+  return OGL_OK;
+}
+
+extern "C" int ogl_plan_pool_rows(ogl_plan* p, ogl_graph* g, ogl_features* f, int layer, const void* h_dev, int ldh, const int64_t* rows_dev,
+                                  int64_t row0, int64_t n, void* hp_dev, int ldhp, void* stream) {
+  int64_t V = 0;
+  OGL_TRY(stream_check(p, g, f, layer, h_dev, ldh, rows_dev, row0, n, "ogl_plan_pool_rows", &V));
+  if (n == 0) return OGL_OK;
+  const LayerBuf& lb = p->layer[layer];
+  OGL_ARG(hp_dev && ldhp == lb.pin && ((uintptr_t)hp_dev & 15) == 0, "ogl_plan_pool_rows: hp must be a 16-byte aligned [*, %d] table", lb.pin);
+  cudaStream_t s = (cudaStream_t)stream;
+  OGL_TRY(full_ws_reserve(p, std::max(V, n)));
+  ogl_plan::FullWs& w = p->full;
+  const int32_t* rows32 = nullptr;
+  OGL_TRY(stream_list(p, rows_dev, n, V, &rows32, s));
+  if (layer == 0) {
+    h_dev = f->table;
+    ldh = f->pitch;
+  }
+  const void* a = nullptr;
+  prof_begin(p, nm("stream.l%d.pool_rows", layer).c_str(), s);
+  int r = rows_of(p, h_dev, ldh, rows32, row0, n, w.hs, &a, s);
+  if (r == OGL_OK) r = pool_gemm(p, layer, a, ldh, w.hp, lb.pin, (int)n, nullptr, s);
+  prof_end(p, s);
+  OGL_TRY(r);
+  STAGE(nm("stream.l%d.scatter", layer).c_str(), put_rows(p->mode, p->es, w.hp, lb.pin, rows32, row0, n, hp_dev, s));
+  return OGL_OK;
+}
+
+extern "C" int ogl_plan_stream_rows(ogl_plan* p, ogl_graph* g, ogl_features* f, int layer, const void* h_dev, int ldh, const void* hp_dev,
+                                    int ldhp, const int64_t* rows_dev, int64_t row0, int64_t n, void* neigh_dev, int ldn, int neigh_mode,
+                                    const int64_t* deg_prev_dev, void* out_dev, int ldo, void* stream) {
+  int64_t V = 0;
+  OGL_TRY(stream_check(p, g, f, layer, h_dev, ldh, rows_dev, row0, n, "ogl_plan_stream_rows", &V));
+  if (n == 0) return OGL_OK;
+  const LayerBuf& lb = p->layer[layer];
+  const bool last = layer == p->L - 1;
+  OGL_ARG(neigh_mode >= 0 && neigh_mode <= 2, "ogl_plan_stream_rows: neigh_mode %d is not 0 (segment max), 1 (suffix) or 2 (table)", neigh_mode);
+  OGL_ARG(neigh_mode == 2 || (hp_dev && ldhp == lb.pin && ((uintptr_t)hp_dev & 15) == 0),
+          "ogl_plan_stream_rows: hp must be a 16-byte aligned [n_vertices, %d] table", lb.pin);
+  OGL_ARG((neigh_mode == 0 && !neigh_dev) || (neigh_dev && ldn == lb.pin && ((uintptr_t)neigh_dev & 15) == 0),
+          "ogl_plan_stream_rows: neigh must be a 16-byte aligned [*, %d] table%s", lb.pin, neigh_mode ? "" : " (or NULL)");
+  OGL_ARG(neigh_mode != 1 || deg_prev_dev, "ogl_plan_stream_rows: the suffix max needs deg_prev");
+  OGL_ARG(out_dev && ldo == lb.pout && ((uintptr_t)out_dev & 15) == 0,
+          "ogl_plan_stream_rows: out must be a 16-byte aligned [*, %d] table (%s)", lb.pout, last ? "fp32 logits" : "the storage type");
+  cudaStream_t s = (cudaStream_t)stream;
+  OGL_TRY(full_ws_reserve(p, std::max(V, n)));
+  ogl_plan::FullWs& w = p->full;
+  const GraphView gv = graph_view(g);
+  const int64_t E = graph_num_edges(g);
+  const int32_t* rows32 = nullptr;
+  OGL_TRY(stream_list(p, rows_dev, n, V, &rows32, s));
+  if (layer == 0) {
+    h_dev = f->table;
+    ldh = f->pitch;
+  }
+  const void* neigh = w.neigh;
+  if (neigh_mode == 0) {
+    STAGE(nm("stream.l%d.segmax", layer).c_str(), csr_segmax(p->mode, gv, E, hp_dev, ldhp, lb.in, rows32, nullptr, row0, n, w.neigh, lb.pin,
+                                                             &w.sm, s));
+    const int64_t np = round_up((int)n, 128);
+    if (np > n) OGL_CUDA(cudaMemsetAsync((char*)w.neigh + p->es * (size_t)n * lb.pin, 0, p->es * (size_t)(np - n) * lb.pin, s));
+    if (neigh_dev)
+      STAGE(nm("stream.l%d.scatter", layer).c_str(), put_rows(p->mode, p->es, w.neigh, lb.pin, rows32, row0, n, neigh_dev, s));
+  } else {
+    if (neigh_mode == 1)
+      STAGE(nm("stream.l%d.segmax_suffix", layer).c_str(), csr_segmax_suffix(p->mode, gv, E, hp_dev, ldhp, lb.in, rows32, nullptr, row0, n,
+                                                                             deg_prev_dev, neigh_dev, ldn, &w.sm, s));
+    OGL_TRY(rows_of(p, neigh_dev, ldn, rows32, row0, n, w.neigh, &neigh, s));
+  }
+  const void* self = nullptr;
+  OGL_TRY(rows_of(p, h_dev, ldh, rows32, row0, n, w.hs, &self, s));
+  void* res = last ? (void*)w.logits : w.hc;
+  STAGE(nm("stream.l%d.out_gemm", layer).c_str(), out_gemm(p, layer, self, ldh, neigh, lb.pin, res, lb.pout, (int)n, nullptr, s));
+  STAGE(nm("stream.l%d.scatter", layer).c_str(), put_rows(last ? OGL_F32 : p->mode, last ? sizeof(float) : p->es, res, lb.pout, rows32, row0, n,
+                                                          out_dev, s));
+  return OGL_OK;
+}
+
+extern "C" int ogl_plan_out_frontier(ogl_plan* p, ogl_graph* g, int layer, const int64_t* rows_dev, int64_t n, int64_t* out_rows_dev,
+                                     int64_t* out_n, int64_t* out_edge_cost, void* stream) {
+  OGL_ARG(p && g && out_n && out_edge_cost && n >= 0 && (rows_dev || n == 0), "ogl_plan_out_frontier: bad arguments");
+  OGL_ARG(graph_source_bound(g) == 0, "ogl_plan_out_frontier: the graph is a destination shard (ogl_graph_set_source_bound)");
+  const GraphView gv = graph_view(g);
+  OGL_ARG(out_rows_dev || gv.n_vertices == 0, "ogl_plan_out_frontier: null out_rows");
+  cudaStream_t s = (cudaStream_t)stream;
+  ogl_plan::FullWs& w = p->full;
+  if (!w.fr_host) OGL_CUDA(cudaMallocHost(&w.fr_host, sizeof(FrontierOut)));
+  STAGE(nm("stream.l%d.frontier", layer).c_str(), out_frontier(gv, graph_num_edges(g), rows_dev, n, nullptr, out_rows_dev, &w.fr, s));
+  OGL_CUDA(cudaMemcpyAsync(w.fr_host, w.fr.out, sizeof(FrontierOut), cudaMemcpyDeviceToHost, s));
+  OGL_CUDA(cudaStreamSynchronize(s));
+  *out_n = w.fr_host->n;
+  *out_edge_cost = (int64_t)w.fr_host->cost;
+  return OGL_OK;
+}
+
 // ------------------------------------------------------------------ stage profiling -----------------
 extern "C" int ogl_plan_profile(ogl_plan* p, int enable) {
   OGL_ARG(p, "ogl_plan_profile: null");

@@ -1,5 +1,11 @@
-"""Streaming inference with cached per-vertex intermediates on the GPU: the drop-in for the per-request method of the reference's
-TorchServe handler (`MNISTDigitClassifier.inference`, /root/reference/inference_optimized.py:144-301; SURVEY 8(f)-3).
+"""Streaming inference on the GPU, in two forms.
+
+`StreamingInference` keeps the exact full-neighbourhood logits of every vertex (what `GraphSAGE.inference` computes, bit for bit)
+current as edges and vertices arrive: a refresh recomputes only the rows whose inputs changed since the last one (DESIGN.md 3e).
+
+`CachedInference` is the drop-in for the per-request method of the reference's
+TorchServe handler (`MNISTDigitClassifier.inference`, /root/reference/inference_optimized.py:144-301; SURVEY 8(f)-3), with its
+approximations.
 
 The serving graph lives in one streaming CSR of the C library that stores every edge in both directions (rows [0, V): in-edge
 sources, rows [V, 2V): out-edge targets, whose degrees are the out-degrees); the
@@ -119,3 +125,134 @@ class CachedInference:
         value = json.loads(str(data[0].get("body")))
         _, classes = self.request(value)
         return [str(classes)]
+
+
+# A layer's changed rows are recomputed on their own while they cost sum(in-degree + 1) <= _THETA * (E + V), the threshold of the
+# plan's frontier inference (kFrontierTheta, csrc/plan.cu); above it that layer and every layer above it run over all rows.
+_THETA = 0.9
+
+
+class StreamingInference:
+    """Exact full-neighbourhood logits of every vertex of `graph` (a DeviceGraph) under `model` (a GraphSAGE), kept current as the
+    graph grows: after any edge / vertex insertions, `logits(T)` is torch.equal to `model.inference(graph, T)`.
+
+    The engine owns per-vertex tables ([v_cap, pitch] each): every layer's pool rows hp_l = relu(h_l Wp + bp), the hidden outputs
+    h_l, layer 0's neighbour max neigh0, the fp32 logits and the in-degree of every row at the last refresh.  A refresh finds the rows
+    whose in-degree changed plus the new vertices (C_1), and, with frozen weights, recomputes only what depends on them:
+
+    - layer 0: hp0 of the new vertices (an existing vertex's features and hence its hp0 never change); neigh0 of C_1 as the max of
+      the stored row and the edges appended since (rows rebuilt by `set_active_prefix` / `load_parent` are recomputed whole), then the
+      output rows of C_1;
+    - layer l >= 1: hp_l of C_l, then C_{l+1} = C_l u N_out(C_l) (a row changes when its own input or an in-neighbour's did), whose
+      segment max and output rows are recomputed.
+
+    Max-pooling is exact and every GEMM row is computed on its own, so the tables hold the bits of the whole-graph call.  A layer
+    whose set is too large (_THETA) runs over all rows instead; a weight change (detected through the model's version, as the
+    model's plans detect it), a shrinking graph or `refresh(full=True)` recompute everything.
+
+    Edges are assumed append-only and feature rows of existing vertices unchanged: after rewriting an existing vertex's features, call
+    `refresh(full=True)`.  Evaluation semantics (no feat_drop).  The engine runs on the model's inference plan for `graph` and uses
+    its full-inference workspace as scratch only: `model.inference` calls in between are harmless, and training state is untouched."""
+
+    def __init__(self, model, graph):
+        self.model, self.graph = model, graph
+        self._n = 0                 # vertices at the last refresh
+        self._version = None        # model._version at the last refresh
+        self._rebuilds = 0          # graph.native.rebuilds at the last refresh
+        self._tabs = False
+
+    def _alloc(self, plan):
+        cap, dims = self.graph.v_cap, plan.dims
+        rows = (cap + 255) // 256 * 256
+        pitch = lambda d: (d + 7) // 8 * 8
+        self.hp = [plan.pool_table(l, cap) for l in range(plan.L)]
+        self.h = [None] + [torch.zeros(rows, pitch(dims[l]), dtype=plan.dtype, device="cuda") for l in range(1, plan.L)]
+        self.neigh0 = plan.pool_table(0, cap)
+        self.table = torch.zeros(rows, pitch(dims[-1]), dtype=torch.float32, device="cuda")
+        self.deg = torch.zeros(cap, dtype=torch.int64, device="cuda")
+        self._tabs = True
+
+    def _out(self, plan, l):
+        return self.table if l == plan.L - 1 else self.h[l + 1]
+
+    def _all_rows(self, plan, g, f, l, V, pool=True):
+        h = self.h[l]
+        if pool:
+            plan.pool_rows(g, f, l, h, self.hp[l], row0=0, n=V)
+        plan.stream_rows(g, f, l, h, self.hp[l], self._out(plan, l), row0=0, n=V, neigh=self.neigh0 if l == 0 else None)
+
+    def refresh(self, full=False):
+        """bring the logits of every vertex up to date with the graph and the weights.  -> dict(path = "none" | "incremental" |
+        "full", layers = [dict(rows, edges, path) per layer]): the output rows each layer recomputed, their sum of (in-degree + 1),
+        and how ("suffix" / "rebuild": layer 0 over its changed rows, "frontier": a higher layer over C_{l+1}, "all": every row after
+        the set grew too large, "full": a full recompute)"""
+        plan = self.model.inference_plan(self.graph)           # (brings the plan's weight shadows up to date)
+        g, f = self.graph.native, self.graph.features
+        if not self._tabs:
+            self._alloc(plan)
+        V, E, L = g.num_vertices, g.num_edges, plan.L
+        deg = g.degrees()
+        full = full or self._version != self.model._version or V < self._n or self._n == 0
+        layers = []
+        if V == 0:
+            path = "none"
+        elif full:
+            if V < self._n:                  # rows past the graph stay zero, as the GEMMs' row tiles expect
+                for t in self.hp + self.h[1:] + [self.neigh0, self.table]:
+                    t[V:self._n].zero_()
+            for l in range(L):
+                self._all_rows(plan, g, f, l, V)
+                layers.append(dict(rows=V, edges=E + V, path="full"))
+            path = "full"
+        else:
+            Vp = self._n
+            C = torch.cat([torch.nonzero(deg[:Vp] != self.deg[:Vp]).squeeze(1), torch.arange(Vp, V, device="cuda")])
+            if C.numel() == 0:
+                path = "none"
+            else:
+                path = "incremental"
+                budget = _THETA * (E + V)
+                if V > Vp:
+                    plan.pool_rows(g, f, 0, None, self.hp[0], row0=Vp, n=V - Vp)
+                cost = int((deg[C] + 1).sum())
+                wide = cost > budget
+                if wide:
+                    self._all_rows(plan, g, f, 0, V, pool=False)
+                    layers.append(dict(rows=V, edges=E + V, path="all"))
+                else:
+                    suffix = g.rebuilds == self._rebuilds
+                    plan.stream_rows(g, f, 0, None, self.hp[0], self._out(plan, 0), rows=C, neigh=self.neigh0,
+                                     neigh_mode=plan.NEIGH_SUFFIX if suffix else plan.NEIGH_SEGMAX, deg_prev=self.deg if suffix else None)
+                    layers.append(dict(rows=C.numel(), edges=cost, path="suffix" if suffix else "rebuild"))
+                for l in range(1, L):
+                    if not wide:
+                        C2, cost = plan.out_frontier(g, C, layer=l)
+                        wide = cost > budget
+                    if wide:
+                        self._all_rows(plan, g, f, l, V)
+                        layers.append(dict(rows=V, edges=E + V, path="all"))
+                        continue
+                    plan.pool_rows(g, f, l, self.h[l], self.hp[l], rows=C)
+                    plan.stream_rows(g, f, l, self.h[l], self.hp[l], self._out(plan, l), rows=C2)
+                    layers.append(dict(rows=C2.numel(), edges=cost, path="frontier"))
+                    C = C2
+        if path != "none" or V != self._n:
+            self.deg[:V].copy_(deg)
+            self.deg[V:].zero_()
+        self._n, self._version, self._rebuilds = V, self.model._version, g.rebuilds
+        return dict(path=path, layers=layers)
+
+    def logits(self, vertices=None):
+        """refresh, then a new fp32 [n, C] tensor of the logits of `vertices` (int64 ids; None: every vertex in id order)"""
+        self.refresh()
+        C = self.model.dims[-1]
+        if vertices is None:
+            return self.table[:self._n, :C].clone()
+        v = torch.as_tensor(vertices, dtype=torch.int64).to("cuda").reshape(-1)
+        if v.numel() and bool(((v < 0) | (v >= self._n)).any()):
+            raise IndexError("StreamingInference.logits: vertex ids outside [0, %d)" % self._n)
+        return self.table[v, :C]
+
+    def predict(self, vertices=None):
+        """the argmax class of each vertex's logits (int64, on the device)"""
+        return self.logits(vertices).argmax(dim=1)
