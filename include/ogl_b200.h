@@ -356,8 +356,10 @@ int ogl_plan_profile_read(ogl_plan* p, char* names_buf, int names_len, float* ms
 int ogl_plan_level_nodes(ogl_plan* p, int level, const int32_t** nodes_dev, const int32_t** count_dev, int* max_count);
 int ogl_plan_block_edges(ogl_plan* p, int hop, const int32_t** edge_src_local_dev, const int32_t** edge_src_global_dev,
                          const int64_t** edge_eid_dev, int* fanout);
-/* named tensors: "hp<l>", "neigh<l>", "arg<l>", "out<l>" for layer l; "full_h0", "full_h1": the two hidden tables of full inference
- * (raw [rows, widest hidden pitch] blocks, after its first call); returns pointer, rows(max), pitch, elem bytes */
+/* named tensors: "hp<l>", "neigh<l>", "arg<l>", "out<l>", "dpre<l>", "dng<l>", "dhp<l>" for layer l; "rev_ptr<h>" (int32, nmax[h+1] + 1
+ * offsets) and "rev_edge<h>" (int32 entries (dst row << 8) | slot, nmax[h] * fanout of them) for hop h, as [rows, 1], from the current
+ * buffer set; "full_h0", "full_h1": the two hidden tables of full inference (raw [rows, widest hidden pitch] blocks, after its first
+ * call); returns pointer, rows(max), pitch, elem bytes */
 int ogl_plan_tensor(ogl_plan* p, const char* name, const void** ptr_dev, int* rows_max, int* pitch, int* elem_bytes);
 
 /* standalone sampler (config 5 sweep + tests): picks into caller buffers.

@@ -577,9 +577,10 @@ class Plan:
                 wrap_device(e.value, (ne,), torch.int64), f.value)
 
     def tensor(self, name, rows=None):
+        """a view of the plan's named device buffer (ogl_plan_tensor); the reverse edge lists rev_ptr<h> / rev_edge<h> are int32"""
         p, r, pt, eb = C.c_void_p(), C.c_int(), C.c_int(), C.c_int()
         check(lib.ogl_plan_tensor(self._h, name.encode(), C.byref(p), C.byref(r), C.byref(pt), C.byref(eb)))
-        dt = {1: torch.uint8, 2: self.dtype, 4: torch.float32}[eb.value]
+        dt = torch.int32 if name.startswith("rev_") else {1: torch.uint8, 2: self.dtype, 4: torch.float32}[eb.value]
         return wrap_device(p.value, (rows if rows is not None else r.value, pt.value), dt)
 
 

@@ -1627,7 +1627,12 @@ extern "C" int ogl_plan_tensor(ogl_plan* p, const char* name, const void** ptr_d
       if (base == "arg") return ret(lb.arg, p->nmax[h], lb.pin, 1);
       if (base == "out") return ret(p->act[h], p->nmax[h], lb.pout, l == L - 1 ? 4 : (int)p->es);
       if (base == "dpre") return ret(lb.dpre, p->nmax[h], lb.pout, (int)p->es);
+      if (base == "dng") return ret(lb.dng, p->nmax[h], lb.pin, (int)p->es);
+      if (base == "dhp") return ret(lb.dhp, p->nmax[h + 1], lb.pin, (int)p->es);
     }
+    // reverse edge lists of hop h (the current buffer set): offsets [nmax[h+1] + 1], entries (dst << 8) | slot [nmax[h] * fanout]
+    if (l >= 0 && l < L && base == "rev_ptr") return ret(p->rev_ptr[l], p->nmax[l + 1] + 1, 1, 4);
+    if (l >= 0 && l < L && base == "rev_edge") return ret(p->rev_edge[l], p->nmax[l] * p->cfg.fanouts[l], 1, 4);
   }
   set_error("ogl_plan_tensor: unknown tensor '%s'", name);
   return OGL_ERR_ARG;
